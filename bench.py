@@ -1,6 +1,7 @@
 """bench.py -- the metric of BASELINE.json: swimmer env-steps/s and ARS iterations/s on 1/2/4/8 B200, % FP64 peak.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--no-ars] [--no-cpu]
+                  [--dump-outputs DIR]
 
 The driver-parsed headline (`metric`, `value`, `e2e`, `roofline`) is BASELINE config[1] (isolated batched
 physics: 3-segment swimmer, 65,536 envs per GPU, fixed random actions, 1,000 explicit-Euler steps; a "step"
@@ -46,7 +47,15 @@ def parse():
     ap.add_argument("--no-ars", action="store_true", help="skip the ARS-iteration measurements")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
     ap.add_argument("--no-sustained", action="store_true", help="skip the >= 2 s sustained run")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (returns, final_state) as "
+                         "DIR/<name>.npy, float64, to compare two builds output for output (the inputs are seeded)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------
@@ -382,6 +391,9 @@ def run_b200(args):
         evs.append((e0, e1))
     barrier()
     wall = time.perf_counter() - t_wall0
+    if args.dump_outputs:
+        # out_def holds the last timed step's results; the supplementary runs below overwrite it
+        dump_outputs(args.dump_outputs, out_def, rank, world)
     t_dev_s = max_over_ranks(sum(a.elapsed_time(b) for a, b in evs)) * 1e-3
     # ---- supplementary: one plain swm_rollout launch per step (no chunking), and the default call enqueued
     # eagerly (no graph), same timing method ----
@@ -773,6 +785,17 @@ def measure_ars(S, D, dist, device, rank, world, barrier, max_over_ranks, fp64_p
             **describe(eng, ", per-step screening as a second right-hand side on the same solution rows"))
         del eng
     return res
+
+
+def dump_outputs(path, outputs, rank, world):
+    """Writes the arrays a caller of the timed step receives (SwimmerEnv.rollout_batched: returns [B], final_state
+    [B, 2n+2]) as <path>/<name>.npy in float64, 4.7 MB per rank.  The actions are drawn from a generator seeded
+    with the rank, so the same arguments give the same inputs on every run.  With several ranks each writes its
+    own batch as <name>_rank<r>.npy."""
+    os.makedirs(path, exist_ok=True)
+    suffix = "_rank%d" % rank if world > 1 else ""
+    for name, t in outputs.items():
+        np.save(os.path.join(path, name + suffix + ".npy"), t.cpu().numpy().astype(np.float64, copy=False))
 
 
 _REAL_STDOUT = None
