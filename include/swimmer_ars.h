@@ -359,6 +359,70 @@ typedef struct {
 SWM_API int64_t swm_rlglue_protocol_state_doubles(int n);
 SWM_API int swm_rlglue_protocol(const swm_params_t* params, const swm_rlglue_protocol_t* cfg, void* stream);
 
+/* ---- Simulator-model estimation: prediction-error objective and CMA-ES on the device ---------------------
+ * Replaces Estimator.I / estimate_real_env_param (ars/estimator.py:36-62, :89-110).  The objective of a
+ * candidate x (d = 1..3 physical parameters) over K recorded trajectories of H observations is
+ *   err(x) = sum_k sum_{t < H-1} || step_x(s_{k,t}, W_k s_{k,t}) - s_{k,t+1} ||_2
+ * with the gym dynamics and the V1 policy product W_k s (as the reference, also for V2-recorded data).
+ * A candidate is the base model with fields[i] replaced by x[i]; a candidate with m_i <= 0 or l_i <= 0 is
+ * not stepped and gets +inf, and every non-finite sum becomes +inf.  Each err[c] is summed in a fixed order
+ * (transitions within a CTA, then CTAs in index order) that depends on neither M nor the candidate's index:
+ * results are bit-identical from run to run and permute with the candidates. */
+#define SWM_MAX_CANDIDATES 1024
+typedef enum { SWM_FIELD_M_I = 0, SWM_FIELD_L_I = 1, SWM_FIELD_K = 2 } swm_field;
+typedef struct {
+  const double* trajectories; /* [K, H, 2n+2] recorded observations */
+  const double* policies;     /* [K, (n-1)(2n+2)] the policy that recorded each trajectory */
+  int32_t K, H;               /* K >= 1, H >= 2 */
+  int32_t d;                  /* unknowns, 1..3 */
+  int32_t fields[3];          /* swm_field replaced by coordinate i < d; each field at most once */
+  double* workspace;          /* [swm_prediction_error_workspace_doubles(K, H, M)] scratch of the two-pass sum */
+} swm_estimate_data_t;
+SWM_API int64_t swm_prediction_error_workspace_doubles(int K, int H, int M);
+/* err[M] = err(candidates[c, 0..d)) for M (1..SWM_MAX_CANDIDATES) candidates, base->n in 2..10 */
+SWM_API int swm_prediction_error(const swm_params_t* base, const swm_estimate_data_t* data,
+                                 const double* candidates, int M, double* err, void* stream);
+
+/* CMA-ES (Hansen, "The CMA Evolution Strategy: A Tutorial", 2016) with the tutorial's default strategy
+ * parameters: mu = floor(lambda/2) positive log weights, c_sigma, d_sigma, c_c, c_1, c_mu, the h_sigma stall,
+ * rank-one + rank-mu covariance update, cumulative step-size adaptation; no active (negative-weight) update.
+ * All of its state is one device buffer of swm_cmaes_state_doubles(d, lambda) doubles, so that a CUDA graph of
+ * several generations can be replayed.  Layout (offsets in doubles; L = 10 + ceil(30 d / lambda)):
+ *   0 generation   1 status (swm_cmaes_status)   2 sigma   3 best f   4 max generations   5 tolfun   6 tolx
+ *   7 mean[d]  7+d best x[d]  7+2d p_sigma[d]  7+3d p_c[d]  7+4d D[d] (sqrt of the eigenvalues of C)
+ *   7+5d C[d*d]  7+5d+d^2 B[d*d] (eigenvectors in columns)  7+5d+2d^2 best-f history[L] (generation g at g % L)
+ *   7+5d+2d^2+L z[lambda, d] (the last generation's standard normal draws)
+ * Sampling: z ~ N(0, I) by Box-Muller (r = sqrt(-2 ln(1 - u0)), angle 2 pi u1) from Philox4x32-10, key = seed,
+ * counter = (pair j, candidate c, generation, 2), u = the 53-bit uniforms of swm_philox_t; candidate
+ * x_c = mean + sigma * B * (D .* z_c).  Update: rank by fitness ascending (+inf and NaN last, ties by lower
+ * index), recombination, evolution paths, C and sigma, then C = B diag(D^2) B^T by cyclic Jacobi with a fixed
+ * sweep count, best-ever tracking, and the stop tests (in this order): tolfun (range of the full best-f history
+ * and this generation's fitness < tolfun), tolx (sigma sqrt(C_ii) < tolx and sigma |p_c,i| < tolx for all i),
+ * condition (max D^2 / min D^2 > 1e14 or C not positive definite), max generations.  Once status != RUNNING
+ * every kernel below is a no-op, so replaying past the stop point changes nothing. */
+#define SWM_CMAES_MIN_POPSIZE 2
+typedef enum {
+  SWM_CMAES_RUNNING = 0,
+  SWM_CMAES_STOP_MAXITER = 1,
+  SWM_CMAES_STOP_TOLFUN = 2,
+  SWM_CMAES_STOP_TOLX = 3,
+  SWM_CMAES_STOP_CONDITIONCOV = 4
+} swm_cmaes_status;
+SWM_API int64_t swm_cmaes_state_doubles(int d, int lambda); /* 0 for d or lambda out of range */
+/* mean = x0 (host [d]), sigma = sigma0, C = B = I, paths 0, generation 0; max_generations <= 0 picks
+ * 100 + 150 (d+3)^2 / sqrt(lambda) (the cma package's default) */
+SWM_API int swm_cmaes_init(double* state, int d, int lambda, const double* x0, double sigma0, double tolfun,
+                           double tolx, int64_t max_generations, void* stream);
+/* candidates[lambda, d] (and z in the state) of the current generation */
+SWM_API int swm_cmaes_sample(double* state, int d, int lambda, uint64_t seed, double* candidates, void* stream);
+/* one update from the candidates of swm_cmaes_sample and their fitness[lambda]; advances the generation */
+SWM_API int swm_cmaes_update(double* state, int d, int lambda, const double* candidates, const double* fitness,
+                             void* stream);
+/* sample + prediction-error objective (data->d == d) + update: one generation, no host round trip */
+SWM_API int swm_cmaes_generation(double* state, int d, int lambda, uint64_t seed, const swm_params_t* base,
+                                 const swm_estimate_data_t* data, double* candidates, double* fitness,
+                                 void* stream);
+
 /* FP64 pipe probe: every thread runs `iters` x 8 independent DFMA chains; returns through
  * *flops_out (host) the number of floating-point operations executed (2 per DFMA).  Used by
  * bench.py to measure the FP64 roofline denominator on the box (MEASURED_PEAKS.json has none). */

@@ -21,6 +21,10 @@ KERNEL_AUTO, KERNEL_THREAD, KERNEL_LANES, KERNEL_LANES2, KERNEL_LANES3 = 0, 1, 2
 MIN_SEGMENTS, MAX_SEGMENTS = 2, 10
 ABI_VERSION = 3  # include/swimmer_ars.h SWM_ABI_VERSION
 MAX_MODELS_PER_STEP = 24  # SWM_MAX_MODELS_PER_STEP
+MAX_CANDIDATES = 1024  # SWM_MAX_CANDIDATES
+CMAES_MIN_POPSIZE = 2  # SWM_CMAES_MIN_POPSIZE
+FIELDS = {"m_i": 0, "l_i": 1, "k": 2}  # swm_field
+CMAES_STOP = {0: "running", 1: "maxiter", 2: "tolfun", 3: "tolx", 4: "conditioncov"}  # swm_cmaes_status
 
 _dp = ctypes.c_void_p
 
@@ -70,6 +74,12 @@ class SwmRlglueProtocol(ctypes.Structure):
                 ("alpha", ctypes.c_double), ("nu", ctypes.c_double), ("deltas", _dp), ("seed", ctypes.c_uint64),
                 ("iteration0", ctypes.c_uint32), ("_pad", ctypes.c_int32), ("state", _dp), ("results", _dp),
                 ("table", _dp), ("replicas", ctypes.c_int64)]
+
+
+class SwmEstimateData(ctypes.Structure):
+    """swm_estimate_data_t (include/swimmer_ars.h): recorded data and field map of the estimation objective."""
+    _fields_ = [("trajectories", _dp), ("policies", _dp), ("K", ctypes.c_int32), ("H", ctypes.c_int32),
+                ("d", ctypes.c_int32), ("fields", ctypes.c_int32 * 3), ("workspace", _dp)]
 
 
 IPC_HANDLE_BYTES = 64  # SWM_IPC_HANDLE_BYTES
@@ -142,6 +152,16 @@ def lib():
     L.swm_exchange_status.argtypes = [_dp, ctypes.POINTER(ctypes.c_uint64), ctypes.POINTER(ctypes.c_uint64)]
     L.swm_exchange_destroy.argtypes = [_dp]
     L.swm_ars_pack_exchange.argtypes = [_dp, ctypes.POINTER(SwmPack), _dp]
+    ed, u64 = ctypes.POINTER(SwmEstimateData), ctypes.c_uint64
+    L.swm_prediction_error_workspace_doubles.argtypes = [c_int, c_int, c_int]
+    L.swm_prediction_error_workspace_doubles.restype = i64
+    L.swm_prediction_error.argtypes = [pp, ed, _dp, c_int, _dp, _dp]
+    L.swm_cmaes_state_doubles.argtypes = [c_int, c_int]
+    L.swm_cmaes_state_doubles.restype = i64
+    L.swm_cmaes_init.argtypes = [_dp, c_int, c_int, ctypes.POINTER(dbl), dbl, dbl, dbl, i64, _dp]
+    L.swm_cmaes_sample.argtypes = [_dp, c_int, c_int, u64, _dp, _dp]
+    L.swm_cmaes_update.argtypes = [_dp, c_int, c_int, _dp, _dp, _dp]
+    L.swm_cmaes_generation.argtypes = [_dp, c_int, c_int, u64, pp, ed, _dp, _dp, _dp]
     if L.swm_abi_version() != ABI_VERSION:
         raise SwimmerLibError("ABI version mismatch")
     _lib = L

@@ -58,7 +58,7 @@ class ARSAgent:
                 from .estimator import Estimator
                 print("Using computed estimation...")
                 self.estimator = Estimator(self.database, guess_param, capacity=1)
-                self.estimated_param = self.estimator.estimate_real_env_param()
+                self.estimated_param = self.estimator.estimate_real_env_param(seed=0 if seed is None else seed)
             elif approx_error is not None:
                 print("Using approximated estimation...")
                 # drawn BEFORE np.random.seed, like ars_agent.py:52 vs :95

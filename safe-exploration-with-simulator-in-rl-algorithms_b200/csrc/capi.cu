@@ -1,5 +1,5 @@
 // extern "C" entry points of libswimmer_ars.so (see include/swimmer_ars.h): argument checks,
-// host-side precomputation of the physical constants and dispatch on the segment count.
+// precomputation of the physical constants (swm::make_phys) and dispatch on the segment count.
 #include <cuda_runtime.h>
 #include <stdio.h>
 #include <string.h>
@@ -10,10 +10,6 @@
 #include "lane_launch.cuh"
 
 using namespace swm;
-
-namespace swm {
-Phys make_phys_public(const swm_params_t* p);
-}
 
 namespace {
 
@@ -47,32 +43,6 @@ bool params_ok(const swm_params_t* p) {
   return p && p->n >= SWM_MIN_SEGMENTS && p->n <= SWM_MAX_SEGMENTS && p->l_i > 0.0 && p->m_i > 0.0;
 }
 
-Phys make_phys(const swm_params_t* p) {
-  Phys P;
-  const double l = p->l_i, m = p->m_i, k = p->k, n = (double)p->n;
-  P.l = l; P.m = m; P.k = k; P.h = p->h; P.max_u = p->max_u;
-  P.dirx = p->direction[0]; P.diry = p->direction[1];
-  P.inv_l = 1.0 / l;
-  P.kappa = k * l / m;
-  P.m2kappa = -2.0 * (k * l / m);
-  P.u_scale = 12.0 / (m * l * l);
-  P.gdd_c = P.m2kappa * (l / (2.0 * n));
-  P.h_gdd_c = p->h * P.gdd_c;
-  P.inv_n = 1.0 / n;
-  P.kl = k * l;
-  P.tau_c = k * (l * l * l) / 12.0;
-  P.half_l = l / 2.0;
-  P.I = m * (l * l) / 12.0;
-  return P;
-}
-
-}  // namespace
-
-// shared with rlglue_protocol.cu
-Phys swm::make_phys_public(const swm_params_t* p) { return make_phys(p); }
-
-namespace {
-
 #define SWM_DISPATCH_N(n, CALL)                 \
   switch (n) {                                  \
     case 2: return note_launch(CALL(2));        \
@@ -93,7 +63,7 @@ int step_common(const swm_params_t* params, int variant, bool acc_only, const do
   if (variant != SWM_DYN_GYM && variant != SWM_DYN_RLGLUE) return SWM_ERR_BAD_ARG;
   if (B == 0) return SWM_OK;  // empty batch: nothing to do, pointers may be NULL
   if (!state_in || !action || !out) return SWM_ERR_BAD_ARG;
-  const Phys P = make_phys(params);
+  const Phys P = make_phys(*params);
   cudaStream_t st = (cudaStream_t)stream;
 #define CALL(K) launch_step_n<K>(P, variant, acc_only, state_in, action, out, reward, (long long)B, st)
   SWM_DISPATCH_N(params->n, CALL)
@@ -143,7 +113,7 @@ extern "C" int swm_step_batched_models(const swm_params_t* params, int n_models,
   PhysSet set;
   for (int i = 0; i < n_models; ++i) {
     if (!params_ok(&params[i]) || params[i].n != params[0].n) return SWM_ERR_BAD_ARG;
-    set.p[i] = make_phys(&params[i]);
+    set.p[i] = make_phys(params[i]);
   }
   for (int i = n_models; i < SWM_MAX_MODELS_PER_STEP; ++i) set.p[i] = set.p[0];
   const long long B = (long long)n_models * envs_per_model;
@@ -208,9 +178,9 @@ int build_rollout_args(const swm_params_t* params, const swm_rollout_t* cfg, Rol
   if (cfg->init_state && cfg->init_state_count < 1) return SWM_ERR_BAD_ARG;
   if (f.screen) {
     if (!params_ok(&cfg->screen.sim) || cfg->screen.sim.n != params->n) return SWM_ERR_BAD_ARG;
-    a.sim = make_phys(&cfg->screen.sim);
+    a.sim = make_phys(cfg->screen.sim);
   }
-  a.real = make_phys(params);
+  a.real = make_phys(*params);
   a.H = cfg->H;
   a.R = cfg->rollouts_per_policy;
   a.policy_mode = cfg->policy_mode;

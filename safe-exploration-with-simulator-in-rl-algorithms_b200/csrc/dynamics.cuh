@@ -23,9 +23,12 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include "../../include/swimmer_ars.h"
+
 namespace swm {
 
-// Physical constants of one model, precomputed on the host (kernel argument -> constant bank).
+// Physical constants of one model, precomputed once per model (kernel argument -> constant bank, or shared
+// memory for the per-candidate models of the estimation objective).
 struct Phys {
   double l, m, k, h, max_u, dirx, diry;
   // gym variant, non-dimensional form (lengths in units of l, forces in units of m*l/2)
@@ -42,6 +45,27 @@ struct Phys {
   double half_l;     // l/2
   double I;          // m*l^2/12
 };
+
+// Host and device build the same constants bit for bit: only correctly rounded products and quotients, no
+// sum that the device compiler could contract into an FMA.
+__host__ __device__ inline Phys make_phys(const swm_params_t& p) {
+  Phys P;
+  const double l = p.l_i, m = p.m_i, k = p.k, n = (double)p.n;
+  P.l = l; P.m = m; P.k = k; P.h = p.h; P.max_u = p.max_u;
+  P.dirx = p.direction[0]; P.diry = p.direction[1];
+  P.inv_l = 1.0 / l;
+  P.kappa = k * l / m;
+  P.m2kappa = -2.0 * (k * l / m);
+  P.u_scale = 12.0 / (m * l * l);
+  P.gdd_c = P.m2kappa * (l / (2.0 * n));
+  P.h_gdd_c = p.h * P.gdd_c;
+  P.inv_n = 1.0 / n;
+  P.kl = k * l;
+  P.tau_c = k * (l * l * l) / 12.0;
+  P.half_l = l / 2.0;
+  P.I = m * (l * l) / 12.0;
+  return P;
+}
 
 // ~1-ulp reciprocal for well-scaled positive arguments (the 2x2 block determinants are >= 4):
 // hardware seed (>= 20 bits) + one cubically convergent step x(1 + e + e^2), e = 1 - d x

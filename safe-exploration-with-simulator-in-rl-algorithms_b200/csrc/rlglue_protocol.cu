@@ -151,8 +151,6 @@ static int launch_protocol(const Phys& P, const ProtoArgs& a, cudaStream_t st) {
   return swm::check_launch();
 }
 
-Phys make_phys_public(const swm_params_t* p);  // capi.cu
-
 }  // namespace swm
 
 using namespace swm;
@@ -176,7 +174,7 @@ extern "C" int swm_rlglue_protocol(const swm_params_t* params, const swm_rlglue_
   a.seed = cfg->seed; a.iteration0 = cfg->iteration0;
   a.state = cfg->state; a.results = cfg->results; a.table = cfg->table;
   a.replicas = cfg->replicas;
-  const Phys P = make_phys_public(params);
+  const Phys P = make_phys(*params);
   cudaStream_t st = (cudaStream_t)stream;
   switch (params->n) {
     case 2: return launch_protocol<2>(P, a, st);

@@ -6,6 +6,7 @@ not synchronise.  These are the batched entry points the reference lacks
 swimmer_env.py / environment.py / ars_agent.py / safe_ars.py are thin layers over them.
 """
 import ctypes
+import math
 
 import torch
 
@@ -15,6 +16,8 @@ from ._lib import (ARS_AGENT, ARS_RLGLUE, ARS_TOPB, DELTA_01, DELTA_PM1, GYM, PO
 
 __all__ = ["step_batched", "step_batched_models", "accelerations_batched", "rollout", "RolloutResult", "ChunkedRollout", "plan_chunks", "philox_deltas",
            "ars_topb", "ars_update", "pack_exchange", "counter_add", "record_nanmean", "stats_finalize", "stats_merge", "reduce_returns", "screen_mask", "policy_actions", "update_args",
+           "EstimateData", "prediction_error", "cmaes_default_popsize", "cmaes_state_doubles", "cmaes_view", "cmaes_init",
+           "cmaes_sample", "cmaes_update", "cmaes_generation",
            "fp64_probe", "obs_dim", "act_dim", "policy_size", "reset_state", "lane_split_envs_per_warp", "rollout_kernel_choice"]
 
 
@@ -533,6 +536,115 @@ def reduce_returns(returns, R, out=None):
         _lib.check(_lib.lib().swm_reduce_returns(_lib.ptr(returns), G, R, _lib.ptr(o),
                                                  _lib.stream_ptr()))
     return o
+
+
+class EstimateData:
+    """Recorded data of the simulator-model estimation objective, resident on the device: trajectories[K, H, 2n+2]
+    recorded under policies[K, n-1, 2n+2], the unknowns (names of the EnvParam fields x replaces, any subset of
+    m_i, l_i, k in any order) and the scratch of the objective's fixed-order sum for up to `max_candidates`
+    candidates (swm_estimate_data_t)."""
+
+    def __init__(self, trajectories, policies, unknowns=("m_i", "l_i", "k"), max_candidates=_lib.MAX_CANDIDATES):
+        self.trajectories = _lib.f64(trajectories).contiguous()
+        K, H, no = self.trajectories.shape
+        self.n = (no - 2) // 2
+        self.policies = _lib.f64(policies).contiguous().reshape(K, policy_size(self.n))
+        if not 1 <= len(unknowns) <= 3 or len(set(unknowns)) != len(unknowns):
+            raise ValueError("unknowns must be 1 to 3 distinct names of m_i, l_i, k, got %r" % (unknowns,))
+        self.unknowns = tuple(unknowns)
+        self.max_candidates = int(max_candidates)
+        nws = _lib.lib().swm_prediction_error_workspace_doubles(K, H, self.max_candidates)
+        if nws <= 0:
+            raise ValueError("need K >= 1 trajectories of H >= 2 observations and max_candidates >= 1")
+        self.workspace = torch.empty(nws, dtype=torch.float64, device=self.trajectories.device)
+        c = _lib.SwmEstimateData()
+        c.trajectories, c.policies = self.trajectories.data_ptr(), self.policies.data_ptr()
+        c.K, c.H, c.d = K, H, len(self.unknowns)
+        for i, name in enumerate(self.unknowns):
+            c.fields[i] = _lib.FIELDS[name]
+        c.workspace = self.workspace.data_ptr()
+        self.c = c
+
+    @property
+    def d(self):
+        return len(self.unknowns)
+
+
+def prediction_error(base_params, data, candidates, out=None):
+    """err[M] = sum_k sum_t || step_x(s_kt, W_k s_kt) - s_k,t+1 || for candidates[M, d] (Estimator.I of a whole
+    population in one launch; +inf for m_i <= 0 or l_i <= 0 and for non-finite sums).  `data`: EstimateData."""
+    _lib.require_cuda()
+    candidates = _lib.f64(candidates).contiguous()
+    M = candidates.shape[0]
+    if tuple(candidates.shape) != (M, data.d) or M > data.max_candidates:
+        raise ValueError("candidates must be [M <= %d, %d]" % (data.max_candidates, data.d))
+    err = torch.empty(M, dtype=torch.float64, device=candidates.device) if out is None else out
+    with torch.cuda.device(candidates.device):
+        _lib.check(_lib.lib().swm_prediction_error(ctypes.byref(base_params), ctypes.byref(data.c),
+                                                   _lib.ptr(candidates), M, _lib.ptr(err), _lib.stream_ptr()))
+    return err
+
+
+def cmaes_default_popsize(d):
+    """lambda = 4 + floor(3 ln d) (Hansen's tutorial, the cma package's default)."""
+    return 4 + int(math.floor(3.0 * math.log(d)))
+
+
+def cmaes_state_doubles(d, popsize):
+    n = _lib.lib().swm_cmaes_state_doubles(int(d), int(popsize))
+    if n <= 0:
+        raise ValueError("CMA-ES needs 1 <= d <= 3 and %d <= popsize <= %d" % (_lib.CMAES_MIN_POPSIZE,
+                                                                             _lib.MAX_CANDIDATES))
+    return n
+
+
+def cmaes_view(state, d, popsize):
+    """Named views into a CMA-ES state buffer (layout of include/swimmer_ars.h)."""
+    L = 10 + -(-30 * d // popsize)
+    o = 7
+    v = {"generation": state[0], "status": state[1], "sigma": state[2], "best_f": state[3],
+         "max_generations": state[4], "tolfun": state[5], "tolx": state[6]}
+    for name, size, shape in (("mean", d, (d,)), ("best_x", d, (d,)), ("p_sigma", d, (d,)), ("p_c", d, (d,)),
+                              ("D", d, (d,)), ("C", d * d, (d, d)), ("B", d * d, (d, d)), ("history", L, (L,)),
+                              ("z", popsize * d, (popsize, d))):
+        v[name] = state[o:o + size].view(shape)
+        o += size
+    return v
+
+
+def cmaes_init(state, x0, popsize, sigma0=1.0, tolfun=1e-11, tolx=1e-11, max_generations=0):
+    """Fresh CMA-ES state around x0 (host sequence of d floats); max_generations <= 0: the cma default."""
+    d = len(x0)
+    x = (ctypes.c_double * d)(*[float(v) for v in x0])
+    with torch.cuda.device(state.device):
+        _lib.check(_lib.lib().swm_cmaes_init(_lib.ptr(state), d, int(popsize), x, float(sigma0), float(tolfun),
+                                             float(tolx), int(max_generations), _lib.stream_ptr()))
+    return state
+
+
+def cmaes_sample(state, d, popsize, seed, candidates):
+    """candidates[popsize, d] = mean + sigma B D z of the current generation (z is kept in the state)."""
+    with torch.cuda.device(state.device):
+        _lib.check(_lib.lib().swm_cmaes_sample(_lib.ptr(state), int(d), int(popsize), int(seed) & (2 ** 64 - 1),
+                                               _lib.ptr(candidates), _lib.stream_ptr()))
+    return candidates
+
+
+def cmaes_update(state, d, popsize, candidates, fitness):
+    """One CMA-ES update from the sampled candidates and their fitness[popsize]."""
+    with torch.cuda.device(state.device):
+        _lib.check(_lib.lib().swm_cmaes_update(_lib.ptr(state), int(d), int(popsize), _lib.ptr(candidates),
+                                               _lib.ptr(fitness), _lib.stream_ptr()))
+    return state
+
+
+def cmaes_generation(state, popsize, seed, base_params, data, candidates, fitness):
+    """sample + prediction_error + update of one generation, enqueued without a host round trip (capturable)."""
+    with torch.cuda.device(state.device):
+        _lib.check(_lib.lib().swm_cmaes_generation(_lib.ptr(state), data.d, int(popsize), int(seed) & (2 ** 64 - 1),
+                                                   ctypes.byref(base_params), ctypes.byref(data.c),
+                                                   _lib.ptr(candidates), _lib.ptr(fitness), _lib.stream_ptr()))
+    return state
 
 
 def fp64_probe(blocks, threads, iters, sink):
