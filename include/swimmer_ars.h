@@ -118,6 +118,7 @@ typedef struct {
   double real_thresh;     /* real steps with cost > real_thresh are counted in violations[] */
   int32_t* violations;    /* [B] or NULL */
   int32_t* frozen_at;     /* [B] or NULL: first step index judged unsafe, H if never */
+                          /* directions skipped by dir_mask: frozen_at = H, violations = 0 */
 } swm_screen_t;
 
 /* One fused H-step rollout of B environments.  Replaces Environment.rollout

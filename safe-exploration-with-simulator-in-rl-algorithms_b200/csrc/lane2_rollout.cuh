@@ -443,6 +443,10 @@ lane2_rollout_kernel(const RolloutArgs a) {
     }
   } else if (active && seg == 0) {
     a.returns[e] = __longlong_as_double(0x7ff8000000000000LL);
+    if (SCREEN) {  // masked out: never judged unsafe, no real step taken (as rollout_kernel)
+      if (a.violations) a.violations[e] = 0;
+      if (a.frozen_at) a.frozen_at[e] = a.H;
+    }
   }
   if (STATS) {
     if (!live) { s1a = s1b = s2a = s2b = 0.0; }

@@ -311,7 +311,7 @@ def test_seed_fanout_equals_sequential_agents(S, tmp_path):
     assert len(saved) == 1 and np.array_equal(np.load(saved[0]), r_graphs)
 
 
-@pytest.mark.parametrize("mode", ["v1", "v2", "safe", "grouped"])
+@pytest.mark.parametrize("mode", ["v1", "v2", "safe", "grouped", "step_screen"])
 def test_graph_replay_equals_eager_iterations(S, mode):
     """The captured CUDA graph of one iteration (device-side Philox iteration counter) replays to
     exactly the eager sequence: returns, policy, statistics and curve bit for bit, including a
@@ -325,11 +325,19 @@ def test_graph_replay_equals_eager_iterations(S, mode):
         kw.update(v2=True, rollouts_per_direction=32, init_perturb=1e-2)
     if mode == "safe":
         kw.update(sim_params=S.make_params(n=n, l_i=.81, m_i=1.21, k=10.25), sim_threshold=-0.002)
+    if mode == "step_screen":  # per-step screening: thresholds inside the spread of the directions' peak |thd|
+        kw.update(step_screen=dict(sim_params=S.make_params(n=n, l_i=.81, m_i=1.21, k=10.25, h=0.0012),
+                                   sim_thresh=0.1, real_thresh=0.08))
     eager, graph = S.ArsEngine(p, **kw), S.ArsEngine(p, use_graph=True, **kw)
+    frozen = []
     for it in range(6):
         a, b = eager.run_iteration().clone(), graph.run_iteration().clone()
         assert torch.equal(torch.nan_to_num(a, nan=-7.0), torch.nan_to_num(b, nan=-7.0)), it
         assert torch.equal(eager.W, graph.W) and torch.equal(eager.stats, graph.stats)
+        if mode == "step_screen":
+            assert torch.equal(eager.last.frozen_at, graph.last.frozen_at), it
+            assert torch.equal(eager.last.violations, graph.last.violations), it
+            frozen.append(eager.last.frozen_at.cpu().numpy())
         if it == 3:  # resume both from the eager engine's checkpoint
             sd = eager.state_dict()
             eager.load_state_dict(sd)
@@ -339,6 +347,9 @@ def test_graph_replay_equals_eager_iterations(S, mode):
     ce, cg = eager.curve.cpu().numpy(), graph.curve.cpu().numpy()
     np.testing.assert_array_equal(np.nan_to_num(ce, nan=-7.0), np.nan_to_num(cg, nan=-7.0))
     assert np.isfinite(cg[:6]).any()
+    if mode == "step_screen":
+        frozen = np.concatenate(frozen)
+        assert (frozen < kw["H"]).any() and (frozen == kw["H"]).any()
 
 
 def test_rlglue_agent_experiment_matches_oracle_loop(S, O, tmp_path):
