@@ -231,19 +231,26 @@ def test_lane_rollout_deterministic_batch_order_invariant_and_nan_isolated(S, ke
 @pytest.mark.parametrize("kern", LANE_KERNELS)
 def test_lane_chunk_chaining_is_bit_identical(S, kern):
     """final_state -> init_state chaining in chunks that are multiples of 64 steps (the exact re-evaluation
-    of the tracked sines/cosines) reproduces the single launch bit for bit; returns accumulate."""
-    n, B, H = 5, 50, 192
-    p = S.make_params(n=n)
+    of the tracked sines/cosines) reproduces the single launch bit for bit; returns accumulate.  Inputs: explicit
+    policies from the reset state, and fixed actions on calm and spun environments sharing warps (one segment at
+    20-300 rad/s, test_trig_tiers population (b)), whose steps run in the tail and exact tiers."""
+    from test_trig_tiers import _spun
+    n, H = 5, 192
     rng = np.random.default_rng(8)
-    Ws = _cuda(rng.uniform(-1, 1, (B, n - 1, 2 * n + 2)) * 0.1)
-    one = S.ops.rollout(p, H, policies=Ws, want_final=True, kernel=_k(S, kern))
-    out = {"returns": torch.zeros(B, dtype=torch.float64, device="cuda"),
-           "final_state": torch.empty(B, 2 * n + 2, dtype=torch.float64, device="cuda")}
-    for c in range(3):
-        S.ops.rollout(p, 64, policies=Ws, want_final=True, kernel=_k(S, kern), out=out,
-                      init_state=None if c == 0 else out["final_state"], accumulate_returns=c > 0)
-    assert torch.equal(out["final_state"], one.final_state)
-    np.testing.assert_allclose(out["returns"].cpu().numpy(), one.returns.cpu().numpy(), rtol=1e-12, atol=1e-14)
+    Ws = _cuda(rng.uniform(-1, 1, (50, n - 1, 2 * n + 2)) * 0.1)
+    init, ac, _ = _spun(n)
+    for p, src, start in ((S.make_params(n=n), dict(policies=Ws), None),
+                          (S.make_params(n=n, l_i=.9, m_i=1.1, k=9.5, direction=(.6, .8)), dict(actions=_cuda(ac)),
+                           _cuda(init))):
+        B = len(next(iter(src.values())))
+        one = S.ops.rollout(p, H, want_final=True, kernel=_k(S, kern), init_state=start, **src)
+        out = {"returns": torch.zeros(B, dtype=torch.float64, device="cuda"),
+               "final_state": torch.empty(B, 2 * n + 2, dtype=torch.float64, device="cuda")}
+        for c in range(3):
+            S.ops.rollout(p, 64, want_final=True, kernel=_k(S, kern), out=out,
+                          init_state=start if c == 0 else out["final_state"], accumulate_returns=c > 0, **src)
+        assert np.array_equal(out["final_state"].cpu().numpy().view(np.int64), one.final_state.cpu().numpy().view(np.int64))
+        np.testing.assert_allclose(out["returns"].cpu().numpy(), one.returns.cpu().numpy(), rtol=1e-12, atol=1e-14)
 
 
 def test_kernel_choice(S):

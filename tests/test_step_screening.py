@@ -141,10 +141,11 @@ def _spread(fz, viol, H, zero=3, mid=5, mid_steps=5, never=5, violated=3):
             and (fz == H).sum() >= never and (viol > 0).sum() >= violated)
 
 
-def _thresholds(sim_cost, real_cost, **need):
-    """Thresholds for which the oracle's decisions give the required spread, with their margins asserted."""
+def _thresholds(sim_cost, real_cost, quantiles=np.linspace(0.05, 0.995, 200), **need):
+    """Thresholds for which the oracle's decisions give the required spread, with their margins asserted; the
+    simulator threshold is the first of the given cost quantiles that does."""
     H = sim_cost.shape[1]
-    for q in np.linspace(0.05, 0.995, 200):
+    for q in quantiles:
         s = _midpoint(sim_cost, q)
         fz = _freeze_steps(sim_cost, s)
         taken = np.concatenate([real_cost[e, :fz[e]] for e in range(len(fz))])
