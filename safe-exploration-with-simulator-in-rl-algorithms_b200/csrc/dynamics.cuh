@@ -67,7 +67,7 @@ __host__ __device__ inline Phys make_phys(const swm_params_t& p) {
   return P;
 }
 
-// ~1-ulp reciprocal for well-scaled positive arguments (the 2x2 block determinants are >= 4):
+// ~1-ulp reciprocal for well-scaled positive arguments (2x2 block determinants >= 4, joint-form pivots >= 1):
 // hardware seed (>= 20 bits) + one cubically convergent step x(1 + e + e^2), e = 1 - d x
 // (3 FMAs, residual e^3 < 2^-60), no special-case path.
 __device__ __forceinline__ double fast_rcp(double d) {
@@ -246,6 +246,141 @@ __device__ __forceinline__ void gym_accelerations(const Phys& P, const double (&
     gny = gjy;
   }
   if (J >= 1) thdd[0] = fma(3.0, fma(c[0], gny, -s[0] * gnx), thdd[0]);  // free head: g_0 = 0
+}
+
+// ---------------------------------------------------------------------------------------------
+// gym variant, joint-angle form for short chains (DESIGN.md §3.1).  With G at the origin the segment
+// centres are x_i - G = l sum_q A_iq p_q, A_iq = [q < i] + 1/2 [q = i] - (N - q - 1/2)/N, whose columns sum
+// to zero, so Gdd drops out of the angle equations.  Projecting Newton's equations on dx_i/dth_r gives,
+// divided by I = m l^2/12 and with C_rq = cos(th_q - th_r), S_rq = sin(th_q - th_r), K = A^T A:
+//   (1 + 12 K o C) thdd = tau~ + m2kappa F + 12 (K o S) thd^2,       F_r = sum_i 6 A_ir C_ir vn_i
+//   vn_i = v.n_i + sum_q A_iq thd_q C_qi   (v = Gdot / l: the centre velocity along n_i, units of l)
+// K o C is a Schur product of two PSD matrices, so the matrix is >= I: every LDL^T pivot is >= 1 and the
+// unpivoted elimination with fast_rcp is safe.  The first pivot is a compile-time constant.
+// Same interface and outputs as gym_accelerations; O(N^2) operations, fewer than the block-tridiagonal
+// sweep up to kJointFormMaxN segments.
+// ---------------------------------------------------------------------------------------------
+#ifndef SWM_JOINT_FORM_MAX_N
+#define SWM_JOINT_FORM_MAX_N 5
+#endif
+constexpr int kJointFormMaxN = SWM_JOINT_FORM_MAX_N;
+
+template <int N>
+struct JointForm {
+  double A[N][N];    // A[i][q]
+  double A6[N][N];   // 6 A
+  double K12[N][N];  // 12 K
+  __host__ __device__ constexpr JointForm() : A(), A6(), K12() {
+    for (int i = 0; i < N; ++i)
+      for (int q = 0; q < N; ++q) {
+        A[i][q] = (q < i ? 1.0 : 0.0) + (q == i ? 0.5 : 0.0) - (N - q - 0.5) / N;
+        A6[i][q] = 6.0 * A[i][q];
+      }
+    for (int r = 0; r < N; ++r)
+      for (int q = 0; q < N; ++q) {
+        double k = 0.0;
+        for (int i = 0; i < N; ++i) k += A[i][r] * A[i][q];
+        K12[r][q] = 12.0 * k;
+      }
+  }
+};
+
+template <int N>
+__device__ __forceinline__ void gym_accelerations_joint(const Phys& P, const double (&s)[N],
+                                                        const double (&c)[N], double gdx, double gdy,
+                                                        const double (&thd)[N], const double* ut,
+                                                        double& psx, double& psy, double (&thdd)[N]) {
+  constexpr JointForm<N> T{};
+  // pair terms r < q: C[r][q] = cos(th_q - th_r), S[r][q] = sin(th_q - th_r) (C symmetric, S antisymmetric)
+  double C[N][N], S[N][N];
+#pragma unroll
+  for (int r = 0; r < N; ++r)
+#pragma unroll
+    for (int q = r + 1; q < N; ++q) {
+      C[r][q] = fma(c[r], c[q], s[r] * s[q]);
+      S[r][q] = fma(s[q], c[r], -c[q] * s[r]);
+    }
+  const double vx = gdx * P.inv_l, vy = gdy * P.inv_l;
+  double vn[N];
+  psx = 0.0;
+  psy = 0.0;
+#pragma unroll
+  for (int i = 0; i < N; ++i) {
+    double a = fma(vy, c[i], -vx * s[i]);
+#pragma unroll
+    for (int q = 0; q < N; ++q) {
+      if (T.A[i][q] == 0.0) continue;
+      const double t = (q == i) ? thd[i] : thd[q] * (q < i ? C[q][i] : C[i][q]);
+      a = fma(T.A[i][q], t, a);
+    }
+    vn[i] = a;
+    psx = fma(-a, s[i], psx);
+    psy = fma(a, c[i], psy);
+  }
+  double th2[N];
+#pragma unroll
+  for (int q = 0; q < N; ++q) th2[q] = thd[q] * thd[q];
+  // right-hand side b and the symmetric matrix M (upper triangle, diagonal constant)
+  double b[N], M[N][N];
+#pragma unroll
+  for (int r = 0; r < N; ++r) {
+    double du = 0.0;
+    if (r >= 1 && r <= N - 2) du = ut[r - 1] - ut[r];
+    else if (r >= 1) du = ut[r - 1];
+    else if (r <= N - 2) du = -ut[r];
+    double f = T.A6[r][r] * vn[r];
+#pragma unroll
+    for (int i = 0; i < N; ++i) {
+      if (i == r || T.A6[i][r] == 0.0) continue;
+      f = fma(T.A6[i][r], (i < r ? C[i][r] : C[r][i]) * vn[i], f);
+    }
+    double br = fma(P.m2kappa, f, fma(P.kappa, thd[r], du));
+#pragma unroll
+    for (int q = 0; q < N; ++q) {
+      if (q == r || T.K12[r][q] == 0.0) continue;
+      br = fma(T.K12[r][q], (r < q ? S[r][q] : -S[q][r]) * th2[q], br);
+    }
+    b[r] = br;
+#pragma unroll
+    for (int q = r + 1; q < N; ++q) M[r][q] = T.K12[r][q] * C[r][q];
+  }
+  // unpivoted LDL^T, right-looking: after step k, M[i][j] (k < i <= j) holds the Schur complement and
+  // L[k][i] = M[k][i] / d_k
+  double inv_d[N], L[N][N];
+#pragma unroll
+  for (int k = 0; k < N; ++k) {
+    double dk = 1.0 + T.K12[k][k];
+#pragma unroll
+    for (int j = 0; j < k; ++j) dk = fma(-L[j][k], M[j][k], dk);
+    inv_d[k] = (k == 0) ? 1.0 / (1.0 + T.K12[0][0]) : fast_rcp(dk);
+#pragma unroll
+    for (int i = k + 1; i < N; ++i) {
+      double mki = M[k][i];
+#pragma unroll
+      for (int j = 0; j < k; ++j) mki = fma(-L[j][k], M[j][i], mki);
+      M[k][i] = mki;
+      L[k][i] = mki * inv_d[k];
+      b[i] = fma(-L[k][i], b[k], b[i]);
+    }
+  }
+#pragma unroll
+  for (int k = N - 1; k >= 0; --k) {
+    double x = b[k] * inv_d[k];
+#pragma unroll
+    for (int i = k + 1; i < N; ++i) x = fma(-L[k][i], thdd[i], x);
+    thdd[k] = x;
+  }
+}
+
+// The gym accelerations in the cheaper of the two forms for N segments (same outputs either way).
+template <int N, int FS = 0>
+__device__ __forceinline__ void gym_accel(const Phys& P, const double (&s)[N], const double (&c)[N],
+                                          double gdx, double gdy, const double (&thd)[N], const double* ut,
+                                          double& psx, double& psy, double (&thdd)[N], double* fs = nullptr) {
+  if constexpr (N <= kJointFormMaxN)
+    gym_accelerations_joint<N>(P, s, c, gdx, gdy, thd, ut, psx, psy, thdd);
+  else
+    gym_accelerations<N, FS>(P, s, c, gdx, gdy, thd, ut, psx, psy, thdd, fs);
 }
 
 // (sin, cos) of th + d from (sin, cos) of th for a small increment d: Taylor polynomials of sin d
@@ -516,7 +651,7 @@ __device__ __forceinline__ double swimmer_step(const Phys& P, double& gdx, doubl
     double ut[N > 1 ? N - 1 : 1];
 #pragma unroll
     for (int k = 0; k < N - 1; ++k) ut[k] = u[k] * P.u_scale;
-    gym_accelerations<N>(P, s, c, gdx, gdy, thd, ut, gddx, gddy, thdd);
+    gym_accel<N>(P, s, c, gdx, gdy, thd, ut, gddx, gddy, thdd);
     gddx *= P.gdd_c;
     gddy *= P.gdd_c;
   } else {
@@ -547,7 +682,7 @@ __device__ __forceinline__ void gym_step_tracked(const Phys& P, double& gdx, dou
                                                  double (&s)[N], double (&c)[N],
                                                  const double* ut, bool resync, double* fs = nullptr) {
   double psx, psy, thdd[N];
-  gym_accelerations<N, FS>(P, s, c, gdx, gdy, thd, ut, psx, psy, thdd, fs);
+  gym_accel<N, FS>(P, s, c, gdx, gdy, thd, ut, psx, psy, thdd, fs);
   gdx = fma(P.h_gdd_c, psx, gdx);
   gdy = fma(P.h_gdd_c, psy, gdy);
   double d[N];

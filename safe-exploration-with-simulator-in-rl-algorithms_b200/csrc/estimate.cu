@@ -99,7 +99,7 @@ __global__ void __launch_bounds__(kEstBlock) prediction_kernel(const EstArgs a) 
       double ut[NA > 0 ? NA : 1], gddx, gddy, thdd[N];
 #pragma unroll
       for (int r = 0; r < NA; ++r) ut[r] = u[r] * P.u_scale;
-      gym_accelerations<N, FS>(P, sn, cs, gdx, gdy, thd, ut, gddx, gddy, thdd, fs);
+      gym_accel<N, FS>(P, sn, cs, gdx, gdy, thd, ut, gddx, gddy, thdd, fs);
       gddx *= P.gdd_c;
       gddy *= P.gdd_c;
       const double ex = fma(P.h, gddx, gdx) - s1[0], ey = fma(P.h, gddy, gdy) - s1[1];

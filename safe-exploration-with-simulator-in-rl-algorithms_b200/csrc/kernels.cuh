@@ -99,7 +99,7 @@ step_kernel(Phys P, const double* state_in, const double* __restrict__ action,
     if (VARIANT == 0) {
 #pragma unroll
       for (int a = 0; a < NA; ++a) u[a] *= P.u_scale;
-      gym_accelerations<N>(P, s, c, gdx, gdy, thd, u, gddx, gddy, thdd);
+      gym_accel<N>(P, s, c, gdx, gdy, thd, u, gddx, gddy, thdd);
       gddx *= P.gdd_c;
       gddy *= P.gdd_c;
     } else {
@@ -378,7 +378,7 @@ rollout_kernel(const RolloutArgs a) {
       double sut[NA > 0 ? NA : 1], sgddx, sgddy, sthdd[N], sthd[N];
 #pragma unroll
       for (int k = 0; k < NA; ++k) sut[k] = u[k] * a.sim.u_scale;
-      gym_accelerations<N, FS>(a.sim, sn, cs, gdx, gdy, thd, sut, sgddx, sgddy, sthdd, sF);
+      gym_accel<N, FS>(a.sim, sn, cs, gdx, gdy, thd, sut, sgddx, sgddy, sthdd, sF);
 #pragma unroll
       for (int i = 0; i < N; ++i) sthd[i] = fma(a.sim.h, sthdd[i], thd[i]);
       if (!(cost_max_abs_thd<N>(sthd) <= a.sim_thresh)) {
