@@ -109,7 +109,8 @@ typedef struct {
 } swm_philox_t;
 
 /* Per-step state-constraint screening (safe_ars/ars.py:111-153, Safe_ARS.isSafe/rollout) with the
- * built-in cost of safe_ars/experiment.py:44, cost(obs) = max_i |thd_i|. */
+ * built-in cost of safe_ars/experiment.py:44, cost(obs) = max_i |thd_i| (swm_rollout), or with a
+ * max-of-affine cost of the whole observation (swm_rollout_costed). */
 typedef struct {
   int32_t enabled;
   int32_t _pad;
@@ -202,6 +203,20 @@ SWM_API int swm_accelerations_batched(const swm_params_t* params, int variant, c
                               const double* action, double* acc, int64_t B, void* stream);
 
 SWM_API int swm_rollout(const swm_params_t* params, const swm_rollout_t* cfg, void* stream);
+/* swm_rollout with per-step screening by a user-defined state cost
+ *     cost(obs) = max_j ( sum_k A[j,k] obs_k + b[j] ),   NaN if any form is NaN (like np.max),
+ * obs = [Gdot_x, Gdot_y, th_1, thd_1, ..., th_n, thd_n].  `forms` is a HOST array [n_forms, 2n+3]: row j is
+ * A[j, 0..2n+1] followed by b[j]; it is copied into the launch's arguments, so it may be freed or changed as soon
+ * as the call returns (a captured CUDA graph keeps the values of the call).  cfg->screen carries the simulator,
+ * the thresholds and the outputs as for swm_rollout; the semantics are those of the built-in cost with cost()
+ * evaluated on the simulator's whole next observation (explicit Euler) and on the real post-step observation.
+ * SWM_ERR_BAD_ARG: screening not enabled, n_forms outside 1..SWM_MAX_COST_FORMS, forms NULL, a non-finite
+ * coefficient, or whatever swm_rollout rejects.  SWM_ERR_UNSUPPORTED: kernel LANES / LANES2 / LANES3, the rlglue
+ * variant, normalize, stats_partial, fixed actions, schedule_sub > 0.  AUTO runs THREAD as one plain launch. */
+#define SWM_MAX_COST_FORMS 32
+SWM_API int swm_rollout_costed(const swm_params_t* params, const swm_rollout_t* cfg,
+                               const double* forms /* HOST [n_forms, 2n+3]: A row, then b */,
+                               int n_forms, void* stream);
 /* number of per-block rows swm_rollout writes into stats_partial for this cfg when launched on `stream` of the
  * current device (depends on the kernel and the schedule it will choose; the schedule may differ while `stream`
  * is capturing a CUDA graph) */

@@ -20,7 +20,7 @@ from .estimator import Estimator  # noqa: F401
 from .experiment import Experiment, SeedFanout  # noqa: F401
 from .parameters import ARSParam, EnvParam, Threshold  # noqa: F401
 from .rlglue_agent import RlglueArsExperiment, read_parameters  # noqa: F401
-from .safe_ars import Basic_ARS, Safe_ARS, builtin_cost  # noqa: F401
+from .safe_ars import Basic_ARS, MaxAffineCost, Safe_ARS, builtin_cost  # noqa: F401
 from .swimmer_env import SwimmerEnv  # noqa: F401
 
 __version__ = "0.1.0"

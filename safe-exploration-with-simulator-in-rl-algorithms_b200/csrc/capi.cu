@@ -1,6 +1,7 @@
 // extern "C" entry points of libswimmer_ars.so (see include/swimmer_ars.h): argument checks,
 // precomputation of the physical constants (swm::make_phys) and dispatch on the segment count.
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -443,20 +444,31 @@ extern "C" int64_t swm_rollout_stats_blocks(const swm_params_t* params, const sw
   return (cfg->B + kRolloutBlock - 1) / kRolloutBlock;
 }
 
-extern "C" int swm_rollout(const swm_params_t* params, const swm_rollout_t* cfg, void* stream) {
-  RolloutArgs a;
-  RolloutFlags f;
-  if (params_ok(params) && cfg && cfg->B == 0 && cfg->H >= 0 && cfg->rollouts_per_policy >= 1 &&
-      (cfg->variant == SWM_DYN_GYM || cfg->variant == SWM_DYN_RLGLUE))
-    return SWM_OK;  // empty batch: nothing to do, pointers may be NULL
-  const int rc = build_rollout_args(params, cfg, a, f);
-  if (rc != SWM_OK) return rc;
+namespace {
+
+// The input buffers a non-empty rollout of this cfg reads and the returns it writes.
+int check_rollout_buffers(const swm_rollout_t* cfg, const RolloutFlags& f) {
   if (!cfg->returns) return SWM_ERR_BAD_ARG;
   if (!f.linear && !cfg->actions) return SWM_ERR_BAD_ARG;
   if (f.linear && !cfg->policies) return SWM_ERR_BAD_ARG;
   if (cfg->policy_mode == SWM_POLICY_DELTAS && !cfg->deltas) return SWM_ERR_BAD_ARG;
   if (f.norm && (!cfg->mean || !cfg->inv_sigma)) return SWM_ERR_BAD_ARG;
   if (f.stats && !cfg->stats_pivot) return SWM_ERR_BAD_ARG;
+  return SWM_OK;
+}
+
+}  // namespace
+
+extern "C" int swm_rollout(const swm_params_t* params, const swm_rollout_t* cfg, void* stream) {
+  RolloutArgs a;
+  RolloutFlags f;
+  if (params_ok(params) && cfg && cfg->B == 0 && cfg->H >= 0 && cfg->rollouts_per_policy >= 1 &&
+      (cfg->variant == SWM_DYN_GYM || cfg->variant == SWM_DYN_RLGLUE))
+    return SWM_OK;  // empty batch: nothing to do, pointers may be NULL
+  int rc = build_rollout_args(params, cfg, a, f);
+  if (rc != SWM_OK) return rc;
+  rc = check_rollout_buffers(cfg, f);
+  if (rc != SWM_OK) return rc;
   const int kernel = choose_kernel(params->n, cfg, a, f);
   if (kernel < 0) return kernel;
   cudaStream_t st = (cudaStream_t)stream;
@@ -469,6 +481,36 @@ extern "C" int swm_rollout(const swm_params_t* params, const swm_rollout_t* cfg,
   if (cfg->schedule_sub > 0 && p.n_sub == 0) return SWM_ERR_UNSUPPORTED;  // a forced schedule that cannot run
   if (p.n_sub > 0) return note_launch(launch_planned(params->n, cfg, a, f, p, st));
   return launch_thread_kernel(params->n, a, f, st);
+}
+
+extern "C" int swm_rollout_costed(const swm_params_t* params, const swm_rollout_t* cfg, const double* forms,
+                                  int n_forms, void* stream) {
+  if (!params_ok(params) || !cfg || !cfg->screen.enabled || !forms) return SWM_ERR_BAD_ARG;
+  if (n_forms < 1 || n_forms > SWM_MAX_COST_FORMS) return SWM_ERR_BAD_ARG;
+  const int cols = 2 * params->n + 3;  // A row (2n+2), then b
+  CostForms cf;
+  memset(&cf, 0, sizeof(cf));
+  cf.J = n_forms;
+  for (int j = 0; j < n_forms; ++j)
+    for (int k = 0; k < cols; ++k) {
+      const double v = forms[(size_t)j * cols + k];
+      if (!isfinite(v)) return SWM_ERR_BAD_ARG;
+      cf.row[j][k] = v;
+    }
+  RolloutArgs a;
+  RolloutFlags f;
+  int rc = build_rollout_args(params, cfg, a, f);
+  if (rc != SWM_OK) return rc;
+  // the costed cost runs on the one-thread-per-environment kernel only, always as one plain launch
+  if (is_lane_kernel(cfg->kernel) || cfg->schedule_sub > 0) return SWM_ERR_UNSUPPORTED;
+  if (cfg->variant != SWM_DYN_GYM || !f.linear || f.norm || f.stats) return SWM_ERR_UNSUPPORTED;
+  if (cfg->B == 0) return SWM_OK;  // empty batch: nothing to do, pointers may be NULL
+  rc = check_rollout_buffers(cfg, f);
+  if (rc != SWM_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+#define CALL(K) launch_rollout_costed_n<K>(a, cf, f, st)
+  SWM_DISPATCH_N(params->n, CALL)
+#undef CALL
 }
 
 // Layout self-check for language bindings: sizes of the ABI structs as this build sees them.

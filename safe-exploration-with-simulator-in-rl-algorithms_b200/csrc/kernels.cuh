@@ -167,11 +167,46 @@ __device__ __forceinline__ double cost_max_abs_thd(const double (&thd)[N]) {
   return __longlong_as_double(m);
 }
 
+// User-defined state cost of per-step screening: cost(obs) = max_j (A_j . obs + b_j) over J forms.  Row j holds
+// A_j (2n+2 entries) followed by b_j; the rows have the stride of the longest chain so that one type serves every n.
+constexpr int kFormStride = 2 * SWM_MAX_SEGMENTS + 3;
+struct CostForms {
+  double row[SWM_MAX_COST_FORMS][kFormStride];
+  int J;  // 1..SWM_MAX_COST_FORMS
+};
+
+// x(k) yields observation entry k.
+template <int NO, typename Obs>
+__device__ __forceinline__ double cost_max_affine(const CostForms& f, const Obs& x) {
+  // NaN if any form is NaN, like np.max (fmax would drop it).  The forms are a warp-uniform kernel argument: the
+  // coefficients are read from the constant bank, one form at a time.
+  double m = __longlong_as_double(0xfff0000000000000LL);  // -inf
+#pragma unroll 1
+  for (int j = 0; j < f.J; ++j) {
+    const double* r = f.row[j];
+    double v = r[NO];
+#pragma unroll
+    for (int k = 0; k < NO; ++k) v = fma(r[k], x(k), v);
+    m = (m == m && !(v <= m)) ? v : m;
+  }
+  return m;
+}
+
+// Screening modes of the rollout kernel: none, the built-in cost max_i |thd_i|, or max-of-affine forms.
+enum ScreenMode { SCREEN_NONE = 0, SCREEN_BUILTIN = 1, SCREEN_AFFINE = 2 };
+
+// Type of the rollout kernel's second argument: the cost forms for SCREEN_AFFINE, an empty struct otherwise.
+struct NoCostForms {};
+template <int SCREEN> struct ScreenForms { using type = NoCostForms; };
+template <> struct ScreenForms<SCREEN_AFFINE> { using type = CostForms; };
+
 // LINEAR: 0 fixed actions, 1 linear policy.  NORM: ARS V2 normalisation.  STATS: accumulate
-// shifted first/second moments of every visited state.  SCREEN: per-step simulator screening.
-template <int N, int VARIANT, int WMODE, bool NORM, bool STATS, bool SCREEN>
+// shifted first/second moments of every visited state.  SCREEN: per-step simulator screening (ScreenMode).
+// With SCREEN_AFFINE the forms travel as the second kernel argument (5.9 KB of the constant bank); the other
+// kernels' argument block grows by one empty byte only.
+template <int N, int VARIANT, int WMODE, bool NORM, bool STATS, int SCREEN>
 __global__ void __launch_bounds__(kRolloutBlock, SWM_ROLLOUT_MIN_BLOCKS)
-rollout_kernel(const RolloutArgs a) {
+rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms<SCREEN>::type forms) {
   constexpr int NO = 2 * N + 2, NA = N - 1, WS = NA * NO;
   constexpr bool LINEAR = (WMODE != W_NONE);
   extern __shared__ __align__(16) double smem[];
@@ -371,17 +406,38 @@ rollout_kernel(const RolloutArgs a) {
         if (VARIANT == 0) ut[k] = v * a.real.u_scale;
       }
     }
-    if (SCREEN) {
+    if (SCREEN != SCREEN_NONE) {
       // Safe_ARS.isSafe (safe_ars/ars.py:111-122): one simulator step from the current state.  The
-      // cost only looks at the new angular velocities, and the simulator starts from the same
-      // angles, so it shares this step's sines/cosines and needs only its own accelerations.
-      double sut[NA > 0 ? NA : 1], sgddx, sgddy, sthdd[N], sthd[N];
+      // simulator starts from the same angles, so it shares this step's sines/cosines and needs only
+      // its own accelerations.
+      double sut[NA > 0 ? NA : 1], sgddx, sgddy, sthdd[N];
 #pragma unroll
       for (int k = 0; k < NA; ++k) sut[k] = u[k] * a.sim.u_scale;
       gym_accel<N, FS>(a.sim, sn, cs, gdx, gdy, thd, sut, sgddx, sgddy, sthdd, sF);
+      double sim_cost;
+      if constexpr (SCREEN == SCREEN_AFFINE) {
+        // the whole simulated observation, explicit Euler as in gym_step_tracked.  Held in 2n+2 registers for
+        // n = 7 and formed per use otherwise: either way round, ptxas spills (8 B at n = 6, 36-56 B at n = 7).
+        double sob[N == 7 ? NO : 1];
+        auto sim_obs = [&](int k) {
+          if (k < 2) return fma(a.sim.h_gdd_c, k == 0 ? sgddx : sgddy, k == 0 ? gdx : gdy);
+          const int i = (k - 2) / 2;
+          return (k & 1) ? fma(a.sim.h, sthdd[i], thd[i]) : fma(a.sim.h, thd[i], th[i]);
+        };
+        if constexpr (N == 7) {
 #pragma unroll
-      for (int i = 0; i < N; ++i) sthd[i] = fma(a.sim.h, sthdd[i], thd[i]);
-      if (!(cost_max_abs_thd<N>(sthd) <= a.sim_thresh)) {
+          for (int k = 0; k < NO; ++k) sob[k] = sim_obs(k);
+        }
+        auto so = [&](int k) { return N == 7 ? sob[k] : sim_obs(k); };
+        sim_cost = cost_max_affine<NO>(forms, so);
+      } else {
+        // the built-in cost only looks at the new angular velocities
+        double sthd[N];
+#pragma unroll
+        for (int i = 0; i < N; ++i) sthd[i] = fma(a.sim.h, sthdd[i], thd[i]);
+        sim_cost = cost_max_abs_thd<N>(sthd);
+      }
+      if (!(sim_cost <= a.sim_thresh)) {
         // unsafe: nothing advances, and since obs and policy never change it never will again
         // (safe_ars/ars.py:151-152) -- the remaining H-t steps are this state repeated.
         frozen = t;
@@ -405,7 +461,14 @@ rollout_kernel(const RolloutArgs a) {
     } else {
       ret += swimmer_step<N, 1>(a.real, gdx, gdy, th, thd, u);
     }
-    if (SCREEN) viol += (cost_max_abs_thd<N>(thd) > a.real_thresh) ? 1 : 0;
+    if (SCREEN == SCREEN_BUILTIN) viol += (cost_max_abs_thd<N>(thd) > a.real_thresh) ? 1 : 0;
+    if constexpr (SCREEN == SCREEN_AFFINE) {
+      double x[NO];
+      x[0] = gdx; x[1] = gdy;
+#pragma unroll
+      for (int i = 0; i < N; ++i) { x[2 + 2 * i] = th[i]; x[3 + 2 * i] = thd[i]; }
+      viol += (cost_max_affine<NO>(forms, [&](int k) { return x[k]; }) > a.real_thresh) ? 1 : 0;
+    }
     if (STATS) {
       double x[NO];
       x[0] = gdx; x[1] = gdy;
@@ -440,7 +503,7 @@ rollout_kernel(const RolloutArgs a) {
 #pragma unroll
       for (int i = 0; i < N; ++i) o[1 + i] = make_double2(th[i], thd[i]);
     }
-    if (SCREEN) {
+    if (SCREEN != SCREEN_NONE) {
       if (a.violations) a.violations[e] = viol;
       if (a.frozen_at) a.frozen_at[e] = frozen;
     }

@@ -148,7 +148,9 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
                                        B = 2 * n_directions * rollouts_per_policy
                                        (+ deltas[D, n-1, 2n+2]: read delta_k from memory instead)
     dir_mask[D] int32 (base_policy modes): directions with 0 are not rolled out (returns NaN).
-    screen = dict(sim_params=..., sim_thresh=..., real_thresh=...) enables Safe_ARS screening.
+    screen = dict(sim_params=..., sim_thresh=..., real_thresh=...) enables Safe_ARS screening with the built-in
+    cost max_i |thd_i|; screen["cost"] = a max-of-affine cost (safe_ars.MaxAffineCost: `.n`, `.forms` [J, 2n+3])
+    screens with that cost instead (swm_rollout_costed; one thread per environment, one plain launch).
     stats_pivot[2n+2] enables the V2 moment accumulation.  `out` may carry preallocated
     tensors (returns, final_state, trajectory, stats_partial) to stay allocation-free in loops.
     kernel: _lib.KERNEL_AUTO (chosen from B, n and the SM count) / KERNEL_THREAD (one thread per
@@ -257,8 +259,17 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
         res.frozen_at = buf("frozen_at", (B,), torch.int32)
         cfg.screen.violations = res.violations.data_ptr()
         cfg.screen.frozen_at = res.frozen_at.data_ptr()
+    cost = screen.get("cost") if screen is not None else None
     with torch.cuda.device(dev):
-        _lib.check(_lib.lib().swm_rollout(ctypes.byref(params), ctypes.byref(cfg), _lib.stream_ptr()))
+        if cost is None:
+            _lib.check(_lib.lib().swm_rollout(ctypes.byref(params), ctypes.byref(cfg), _lib.stream_ptr()))
+        else:
+            if cost.n != n:
+                raise ValueError("the cost is for n=%d segments, the model has n=%d" % (cost.n, n))
+            forms = cost.forms  # host [J, 2n+3], copied into the launch's arguments
+            _lib.check(_lib.lib().swm_rollout_costed(ctypes.byref(params), ctypes.byref(cfg),
+                                                     forms.ctypes.data_as(ctypes.c_void_p), forms.shape[0],
+                                                     _lib.stream_ptr()))
     return res
 
 

@@ -4,14 +4,15 @@ state-constraint screening through a simulator environment, fused into the rollo
 (each step evaluates the simulator model and the real model from the same state in the same
 thread).
 
-The `cost` callable of the reference is arbitrary Python; the kernel implements the one the
-reference uses (safe_ars/experiment.py:44, cost(obs) = max_i |obs[3+2i]|).  A different callable
-is rejected loudly rather than silently evaluated on the host.
+The `cost` callable of the reference is arbitrary Python; the kernels implement the one the
+reference uses (safe_ars/experiment.py:44, cost(obs) = max_i |obs[3+2i]|) and any maximum of affine
+forms of the observation (MaxAffineCost).  A different callable is rejected loudly rather than
+silently evaluated on the host.
 """
 import numpy as np
 import torch
 
-from . import ops
+from . import _lib, ops
 from ._lib import ARS_TOPB
 from .engine import ArsEngine
 from .swimmer_env import SwimmerEnv
@@ -21,6 +22,35 @@ def builtin_cost(x):
     """cost(obs) = max_i |theta_dot_i| (safe_ars/experiment.py:44)."""
     x = np.asarray(x)
     return np.max(np.abs(x[3::2]))
+
+
+class MaxAffineCost:
+    """cost(obs) = max_j (A[j] . obs + b[j]) over J = 1..32 affine forms of the observation
+    obs = [Gdot_x, Gdot_y, th_1, thd_1, ..., th_n, thd_n]; NaN if any form is NaN (like np.max).
+
+    Covers bounds |obs_k| <= c (rows +-e_k), bending limits |th_i - th_{i+1}|, signed velocity bounds
+    and the built-in cost (rows +-e_{3+2i}).  A, b must be finite.  Safe_ARS screens with it on the GPU
+    (one thread per environment)."""
+
+    def __init__(self, A, b=None):
+        A = np.array(A, dtype=np.float64, copy=True)
+        if A.ndim != 2 or A.shape[1] % 2 or not _lib.MIN_SEGMENTS <= A.shape[1] // 2 - 1 <= _lib.MAX_SEGMENTS:
+            raise ValueError("A must be [J, 2n+2] with %d <= n <= %d, got shape %s"
+                             % (_lib.MIN_SEGMENTS, _lib.MAX_SEGMENTS, A.shape))
+        J = A.shape[0]
+        if not 1 <= J <= _lib.MAX_COST_FORMS:
+            raise ValueError("a cost has 1 to %d forms, got %d" % (_lib.MAX_COST_FORMS, J))
+        b = np.zeros(J) if b is None else np.array(b, dtype=np.float64, copy=True)
+        if b.shape != (J,):
+            raise ValueError("b must have shape (%d,), got %s" % (J, b.shape))
+        if not (np.isfinite(A).all() and np.isfinite(b).all()):
+            raise ValueError("the coefficients of a cost must be finite")
+        self.A, self.b = A, b
+        self.n = A.shape[1] // 2 - 1
+        self.forms = np.ascontiguousarray(np.hstack([A, b[:, None]]))  # [J, 2n+3]: the layout of swm_rollout_costed
+
+    def __call__(self, obs):
+        return float(np.max(self.A @ np.asarray(obs, dtype=np.float64) + self.b))
 
 
 def _check_cost(cost, n):
@@ -106,7 +136,11 @@ class Safe_ARS(Basic_ARS):
 
     def __init__(self, cost, real_threshold, sim_threshold, sim_env):
         assert isinstance(sim_env, SwimmerEnv)
-        _check_cost(cost, sim_env.n)
+        if isinstance(cost, MaxAffineCost):
+            if cost.n != sim_env.n:
+                raise ValueError("the cost is for n=%d segments, the environment has n=%d" % (cost.n, sim_env.n))
+        else:
+            _check_cost(cost, sim_env.n)
         self.cost = cost
         self.real_thresh = real_threshold
         self.sim_thresh = sim_threshold
@@ -114,8 +148,11 @@ class Safe_ARS(Basic_ARS):
 
     def _screen(self, real_env):
         assert self.sim_env.n == real_env.n
-        return dict(sim_params=self.sim_env.params(), sim_thresh=self.sim_thresh,
-                    real_thresh=self.real_thresh)
+        screen = dict(sim_params=self.sim_env.params(), sim_thresh=self.sim_thresh,
+                      real_thresh=self.real_thresh)
+        if isinstance(self.cost, MaxAffineCost):
+            screen["cost"] = self.cost
+        return screen
 
     def isSafe(self, cost, thresh, env, state, action):
         """Simulate `action` from `state` on `env` and compare the cost with the threshold
