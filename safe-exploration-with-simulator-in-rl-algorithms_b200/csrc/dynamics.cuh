@@ -285,6 +285,9 @@ struct JointForm {
   }
 };
 
+// k * x for a compile-time constant k, without the multiply when k is 1
+__device__ __forceinline__ double scaled(double k, double x) { return k == 1.0 ? x : k * x; }
+
 template <int N>
 __device__ __forceinline__ void gym_accelerations_joint(const Phys& P, const double (&s)[N],
                                                         const double (&c)[N], double gdx, double gdy,
@@ -328,11 +331,15 @@ __device__ __forceinline__ void gym_accelerations_joint(const Phys& P, const dou
     if (r >= 1 && r <= N - 2) du = ut[r - 1] - ut[r];
     else if (r >= 1) du = ut[r - 1];
     else if (r <= N - 2) du = -ut[r];
-    double f = T.A6[r][r] * vn[r];
+    // A6[r][r] is 0 for the middle segment of odd N: no multiply by a compile-time zero
+    double f = 0.0;
+    bool first = true;
 #pragma unroll
     for (int i = 0; i < N; ++i) {
-      if (i == r || T.A6[i][r] == 0.0) continue;
-      f = fma(T.A6[i][r], (i < r ? C[i][r] : C[r][i]) * vn[i], f);
+      if (T.A6[i][r] == 0.0) continue;
+      const double t = (i == r) ? vn[i] : (i < r ? C[i][r] : C[r][i]) * vn[i];
+      f = first ? T.A6[i][r] * t : fma(T.A6[i][r], t, f);
+      first = false;
     }
     double br = fma(P.m2kappa, f, fma(P.kappa, thd[r], du));
 #pragma unroll
@@ -342,7 +349,7 @@ __device__ __forceinline__ void gym_accelerations_joint(const Phys& P, const dou
     }
     b[r] = br;
 #pragma unroll
-    for (int q = r + 1; q < N; ++q) M[r][q] = T.K12[r][q] * C[r][q];
+    for (int q = r + 1; q < N; ++q) M[r][q] = scaled(T.K12[r][q], C[r][q]);
   }
   // unpivoted LDL^T, right-looking: after step k, M[i][j] (k < i <= j) holds the Schur complement and
   // L[k][i] = M[k][i] / d_k
@@ -359,7 +366,9 @@ __device__ __forceinline__ void gym_accelerations_joint(const Phys& P, const dou
 #pragma unroll
       for (int j = 0; j < k; ++j) mki = fma(-L[j][k], M[j][i], mki);
       M[k][i] = mki;
-      L[k][i] = mki * inv_d[k];
+      // first pivot a compile-time constant: L[0][i] = C[0][i] * (K12[0][i] / d_0), one multiply (none for n = 3,
+      // where the quotient is 1 for i = 1) instead of two
+      L[k][i] = (k == 0) ? scaled(T.K12[0][i] / (1.0 + T.K12[0][0]), C[0][i]) : mki * inv_d[k];
       b[i] = fma(-L[k][i], b[k], b[i]);
     }
   }
@@ -383,15 +392,41 @@ __device__ __forceinline__ void gym_accel(const Phys& P, const double (&s)[N], c
     gym_accelerations<N, FS>(P, s, c, gdx, gdy, thd, ut, psx, psy, thdd, fs);
 }
 
-// (sin, cos) of th + d from (sin, cos) of th for a small increment d: Taylor polynomials of sin d
-// and cos d - 1, then one 2x2 rotation -- no range reduction, no integer work (a full
-// double-precision sincos is ~27 FP64 + ~50 other instructions).  Two additive tiers:
+// (sin, cos) of th + d from (sin, cos) of th for a small increment d: polynomials of sin d and
+// cos d - 1, then one 2x2 rotation -- no range reduction, no integer work (a full double-precision
+// sincos is ~27 FP64 + ~50 other instructions).
+//
+// Per-thread rollout step (gym_step_tracked) for N <= kRotateOneTierMaxN: one polynomial for |d| <= 1/8, z = d^2,
+//   sin d = d + d^3 P(z),  cos d - 1 = z Q(z),  P and Q of degree 3
+// with P and Q Chebyshev-economised in z on [0, 1/64] (rotation_poly.py derives the coefficients in
+// exact rational arithmetic): truncation <= 2.8e-20 for sin d and <= 2.3e-18 for cos d - 1 over the
+// whole range, below one ulp of the rotated value.  Approximating P and Q rather than sin d itself
+// keeps the sine's error proportional to d^3.
+// It costs 3 FP64 operations per segment more than the base tier below and removes the per-lane tail branch:
+// measured on B200 (profiles/r04_summary.md) that wins for n = 3 with fast segments (config[1]: the tail ran on
+// about half of the warp-steps) and loses for n = 5 and n = 10 V2 rollouts, whose segments rarely leave the base
+// tier; longer chains keep the two tiers.
+constexpr int kRotateOneTierMaxN = 3;
+constexpr double kRotateP[4] = {-0.16666666666666666, 0.008333333333309446, -0.0001984126907688373,
+                                2.75494915427022e-06};
+constexpr double kRotateQ[4] = {-0.4999999999999999, 0.04166666666640392, -0.0013888888048092878,
+                                2.4792977072672542e-05};
+__device__ __forceinline__ void small_sincos(double d, double& sn, double& cm1) {
+  const double z = d * d;
+  const double p = fma(z, fma(z, fma(z, kRotateP[3], kRotateP[2]), kRotateP[1]), kRotateP[0]);
+  const double q = fma(z, fma(z, fma(z, kRotateQ[3], kRotateQ[2]), kRotateQ[1]), kRotateQ[0]);
+  sn = fma(d * z, p, d);
+  cm1 = z * q;
+}
+
+// Longer chains in the per-thread step and the lane-split kernels (lane_rollout.cuh, lane2_rollout.cuh): Taylor
+// polynomials in two additive tiers,
 //   base, |d| <= 1/32: sin to d^5, cos to d^6     truncation <= 5.8e-15 at the limit and ~(32 d)^7 of
 //                                                 that below it (1e-19 at |thd| = 7 rad/s, h = 1e-3)
 //   tail, |d| <= 1/8 : + the d^7, d^9 terms of sin and the d^8, d^10 terms of cos (truncation < 3e-17)
-// The tail is added under a per-lane branch: a warp whose lanes are all slow skips it, a mixed warp
-// pays 8 more operations per segment, and no lane's result depends on its neighbours.  The rollout
-// kernel re-evaluates (s, c) exactly from th every 64th step, so truncation never accumulates over
+// The tail is added under a per-lane branch in the per-thread step, and out of line or under a warp vote,
+// once per segment lane, in the lane-split kernels; no lane's result depends on its neighbours.  Every
+// rollout kernel re-evaluates (s, c) exactly from th every 64th step, so truncation never accumulates over
 // more than 63 steps.
 constexpr double kRotateShort = 0.03125, kRotateLong = 0.125;
 constexpr int kRotateShortHi = 0x3FA00000, kRotateLongHi = 0x3FC00000;  // high words of 1/32 and 1/8
@@ -700,25 +735,32 @@ __device__ __forceinline__ void gym_step_tracked(const Phys& P, double& gdx, dou
   }
   // Decided per lane from the lane's own data only, so that an environment's trajectory does not
   // depend on which other environments share its warp.  NaN falls through to sincos.
-  double z[N], sn[N], cm1[N];
+  double sn[N], cm1[N];
+  if constexpr (N <= kRotateOneTierMaxN) {
 #pragma unroll
-  for (int i = 0; i < N; ++i) small_sincos_base(d[i], z[i], sn[i], cm1[i]);
-#ifdef SWM_ANALYZE_TIER  // static SASS analysis of one fast path only (tools/fastpath_mix.sh); never shipped
-  if (SWM_ANALYZE_TIER == 1) {
+    for (int i = 0; i < N; ++i) small_sincos(d[i], sn[i], cm1[i]);
+  } else {
+    double z[N];
 #pragma unroll
-    for (int i = 0; i < N; ++i) small_sincos_tail(d[i], z[i], sn[i], cm1[i]);
+    for (int i = 0; i < N; ++i) small_sincos_base(d[i], z[i], sn[i], cm1[i]);
+#ifndef SWM_ANALYZE_TIER
+    // One branch for all segments of a lane.  (A branch per segment would skip the tail for segments that are
+    // slow in every lane, ~7 FP64 operations per step fewer for n = 3 -- measured 1.7 % SLOWER there and 18 %
+    // slower for n = 10: N divergent regions per step cost more than they save, profiles/r02_summary.md.)
+    if (dmax_hi > kRotateShortHi)
+#else  // static SASS analysis of one fast path only (tools/fastpath_mix.sh); never shipped
+    if (SWM_ANALYZE_TIER == 1)
+#endif
+    {
+#pragma unroll
+      for (int i = 0; i < N; ++i) small_sincos_tail(d[i], z[i], sn[i], cm1[i]);
+    }
   }
+#ifdef SWM_ANALYZE_TIER
 #pragma unroll
   for (int i = 0; i < N; ++i) rotate_by(sn[i], cm1[i], s[i], c[i]);
   return;
 #endif
-  // One branch for all segments of a lane.  (A branch per segment would skip the tail for segments that are
-  // slow in every lane, ~7 FP64 operations per step fewer for n = 3 -- measured 1.7 % SLOWER there and 18 %
-  // slower for n = 10: N divergent regions per step cost more than they save, profiles/r02_summary.md.)
-  if (dmax_hi > kRotateShortHi) {
-#pragma unroll
-    for (int i = 0; i < N; ++i) small_sincos_tail(d[i], z[i], sn[i], cm1[i]);
-  }
   if (resync || dmax_hi > kRotateLongHi) {
 #pragma unroll
     for (int i = 0; i < N; ++i) sincos(th[i], &s[i], &c[i]);

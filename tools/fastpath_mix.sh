@@ -1,5 +1,5 @@
 #!/bin/bash
-# Static FP64 issue-cost estimate of the rollout fast path (sincos resync removed, rotation tier TIER=0|1 only) for n in "$@".
+# Static FP64 issue-cost estimate of the rollout fast path (sincos resync removed, rotation tier TIER=0|1 only where n has two tiers) for n in "$@".
 # usage: tools/fastpath_mix.sh 3 5 10
 set -e
 ROOT=$(cd "$(dirname "$0")/.." && pwd)
@@ -10,7 +10,7 @@ for n in "$@"; do
 done
 wait
 for n in "$@"; do
-  for pat in "Li${n}ELi0ELi0ELb0ELb0ELb0E" "Li${n}ELi0ELi[123]ELb1ELb1ELb0E"; do
+  for pat in "Li${n}ELi0ELi0ELb0ELb0ELi0E" "Li${n}ELi0ELi[123]ELb1ELb1ELi0E"; do
     python $ROOT/tools/sass_mix.py /tmp/fastpath/n$n.o "$pat" | grep -E "^==|loop|reuse|DFMA|DMUL|DADD|UMOV|IMAD|LDS|STS" 
   done
 done
