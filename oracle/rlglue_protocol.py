@@ -181,7 +181,7 @@ def run_reference_protocol(par, n_it, seed):
     return {k: np.array(v) for k, v in out.items()}
 
 
-def restated_protocol(par, n_it, deltas):
+def restated_protocol(par, n_it, deltas, tables=None):
     """The same step-level loop restated over the C port (oracle_lib.step, rlglue variant): one agent state
     machine (SwimmerAgent.py:79-130), clip (:181-201), index order + sample stdev update (:214-241), and the
     experiment's load-state / freeze schedule (SwimmerExperiment.cpp:65-84).  deltas[n_it+1, N, n-1, 2n+2]
@@ -192,7 +192,8 @@ def restated_protocol(par, n_it, deltas):
         observation it was just given;
       * rollout k's return therefore sums the rewards of env steps kH+1 .. (k+1)H, and the last slot of the
         reward table (r- of the last direction) is filled at the first step of the NEXT iteration: it holds
-        the first reward (iteration 0) or the previous evaluation total plus that reward."""
+        the first reward (iteration 0) or the previous evaluation total plus that reward.
+    `tables` (a list): the reward table [2N] each update uses is appended to it."""
     from oracle import oracle_lib as O
     n, N, b, H = int(par["n_seg"]), int(par["N"]), int(par["b"]), int(par["H"])
     alpha, nu, max_u = par["alpha"], par["nu"], par["max_u"]
@@ -238,6 +239,8 @@ def restated_protocol(par, n_it, deltas):
             if not freeze:
                 count += 1
                 if count % (2 * N * H) == 0:
+                    if tables is not None:
+                        tables.append(np.array(rewards))
                     used = [rewards[2 * k + s] for k in range(b) for s in (0, 1)]
                     sigma = float(np.std(used, ddof=1))
                     grad = sum((rewards[2 * k] - rewards[2 * k + 1]) * deltas[it_deltas][k] for k in range(b))

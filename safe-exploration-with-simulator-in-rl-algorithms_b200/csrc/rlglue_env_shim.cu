@@ -31,6 +31,7 @@ double* d_out = nullptr;     // device [2n+2 next state | reward]
 double* h_in = nullptr;      // pinned mirror of d_in
 double* h_out = nullptr;     // pinned mirror of d_out
 cudaStream_t g_stream = nullptr;
+int g_sized_n = 0;           // chain length the buffers above are sized for (0: before env_init / after env_cleanup)
 std::string g_task_spec, g_param_msg;
 
 // private stand-ins for RLStruct_util.h (not exported: librlutils owns those names)
@@ -51,17 +52,27 @@ void die(const char* what) {
   abort();
 }
 
-void set_parameters(const char* path) {
+// Returns "" or why a requested n_seg was not applied: outside SWM_MIN_SEGMENTS..SWM_MAX_SEGMENTS, or a change
+// after env_init, whose observation, pinned and device buffers hold 2n+2 doubles of the chain they were sized for.
+std::string set_parameters(const char* path) {
   FILE* f = fopen(path, "r");
-  if (!f) { fprintf(stderr, "Unable to open file for setting environment parameters\n"); return; }
+  if (!f) { fprintf(stderr, "Unable to open file for setting environment parameters\n"); return ""; }
+  std::string refused;
   char name[128];
   char line[512];
   while (fgets(line, sizeof(line), f)) {
     double a = 0, b = 0;
     const int got = sscanf(line, "%127s %lf %lf", name, &a, &b);
     if (got < 2) continue;
-    if (!strcmp(name, "n_seg")) g_params.n = (int)a;
-    else if (!strcmp(name, "max_u")) g_params.max_u = a;
+    if (!strcmp(name, "n_seg")) {
+      if (!(a >= SWM_MIN_SEGMENTS && a <= SWM_MAX_SEGMENTS && a == (int)a))
+        refused = "n_seg must be an integer in " + std::to_string(SWM_MIN_SEGMENTS) + ".." +
+                  std::to_string(SWM_MAX_SEGMENTS);
+      else if (g_sized_n && (int)a != g_sized_n)
+        refused = "n_seg cannot change between env_init and env_cleanup";
+      else
+        g_params.n = (int)a;
+    } else if (!strcmp(name, "max_u")) g_params.max_u = a;
     else if (!strcmp(name, "l_i")) g_params.l_i = a;
     else if (!strcmp(name, "k")) g_params.k = a;
     else if (!strcmp(name, "m_i")) g_params.m_i = a;
@@ -69,6 +80,7 @@ void set_parameters(const char* path) {
     else if (!strcmp(name, "direction") && got == 3) { g_params.direction[0] = a; g_params.direction[1] = b; }
   }
   fclose(f);
+  return refused;
 }
 
 void copy_obs(observation_t& dst, const observation_t& src) {
@@ -83,6 +95,7 @@ extern "C" {
 /* Programmatic alternative to the "set parameters" message (the reference has file globals). */
 int swm_rlglue_set_params(const swm_params_t* p) {
   if (!p || p->n < SWM_MIN_SEGMENTS || p->n > SWM_MAX_SEGMENTS) return SWM_ERR_BAD_ARG;
+  if (g_sized_n && p->n != g_sized_n) return SWM_ERR_BAD_ARG;
   g_params = *p;
   return SWM_OK;
 }
@@ -100,6 +113,7 @@ const char* env_init(void) {
       cudaMallocHost(&h_out, sizeof(double) * (n_obs + 1)) != cudaSuccess ||
       cudaStreamCreateWithFlags(&g_stream, cudaStreamNonBlocking) != cudaSuccess)
     die("device / pinned allocation failed");
+  g_sized_n = g_params.n;
   g_task_spec = "VERSION RL-Glue-3.0 PROBLEMTYPE continuing DISCOUNTFACTOR 0.9 OBSERVATIONS DOUBLES (" +
                 std::to_string(n_obs) + " UNSPEC UNSPEC) ACTIONS DOUBLES (" + std::to_string(n_action) +
                 " " + std::to_string(-g_params.max_u) + " " + std::to_string(g_params.max_u) +
@@ -146,6 +160,7 @@ void env_cleanup(void) {
   if (g_stream) cudaStreamDestroy(g_stream);
   d_in = d_out = h_in = h_out = nullptr;
   g_stream = nullptr;
+  g_sized_n = 0;
 }
 
 const char* env_message(const char* message) {
@@ -160,8 +175,9 @@ const char* env_message(const char* message) {
   }
   if (strncmp(message, "set parameters", 14) == 0) {
     const char* path = message[14] == ' ' ? message + 15 : getenv("SWM_PARAMETERS_FILE");
-    set_parameters(path ? path : "../parameters.txt");
-    g_param_msg = "Environment parameters are: n_seg=" + std::to_string(g_params.n) +
+    const std::string refused = set_parameters(path ? path : "../parameters.txt");
+    g_param_msg = (refused.empty() ? "" : "Refused: " + refused + "; n_seg unchanged. ") +
+                  "Environment parameters are: n_seg=" + std::to_string(g_params.n) +
                   "; max_u=" + std::to_string(g_params.max_u) + "; l_i=" + std::to_string(g_params.l_i) +
                   "; k=" + std::to_string(g_params.k) + "; m_i=" + std::to_string(g_params.m_i) +
                   "; h_global=" + std::to_string(g_params.h);
