@@ -110,7 +110,8 @@ typedef struct {
 
 /* Per-step state-constraint screening (safe_ars/ars.py:111-153, Safe_ARS.isSafe/rollout) with the
  * built-in cost of safe_ars/experiment.py:44, cost(obs) = max_i |thd_i| (swm_rollout), or with a
- * max-of-affine cost of the whole observation (swm_rollout_costed). */
+ * max-of-affine cost of the whole observation (swm_rollout_costed), by one simulator model or by an ensemble of
+ * them (swm_rollout_ensemble). */
 typedef struct {
   int32_t enabled;
   int32_t _pad;
@@ -217,6 +218,23 @@ SWM_API int swm_rollout(const swm_params_t* params, const swm_rollout_t* cfg, vo
 SWM_API int swm_rollout_costed(const swm_params_t* params, const swm_rollout_t* cfg,
                                const double* forms /* HOST [n_forms, 2n+3]: A row, then b */,
                                int n_forms, void* stream);
+/* swm_rollout with per-step screening by an ensemble of simulator models: before every real step each of the
+ * n_models models takes one simulator step from the current state with the current action, and the real step is
+ * taken only if cost(next obs of model m) <= sim_thresh for EVERY m (a NaN cost from any model is unsafe); an
+ * unsafe step freezes the environment for good, as in swm_rollout.  The cost is the built-in max_i |thd_i| when
+ * `forms` is NULL (n_forms is then ignored), else the max-of-affine cost of swm_rollout_costed (same layout).
+ * `sim_models` is a HOST array of n_models structs with the real model's n; models and forms are copied into the
+ * launch's arguments, so they may be freed or changed as soon as the call returns (a captured CUDA graph keeps the
+ * values of the call).  cfg->screen carries the thresholds and the outputs; cfg->screen.sim is not read.  With one
+ * model the results are those of swm_rollout (kernel THREAD) / swm_rollout_costed bit for bit.
+ * SWM_ERR_BAD_ARG: screening not enabled, n_models outside 1..SWM_MAX_SIM_MODELS, sim_models NULL, a model that is
+ * not a valid swm_params_t or has another n, forms non-NULL with n_forms outside 1..SWM_MAX_COST_FORMS or a
+ * non-finite coefficient, or whatever swm_rollout rejects.  SWM_ERR_UNSUPPORTED: as swm_rollout_costed. */
+#define SWM_MAX_SIM_MODELS 16
+SWM_API int swm_rollout_ensemble(const swm_params_t* params, const swm_rollout_t* cfg,
+                                 const swm_params_t* sim_models /* HOST [n_models] */, int n_models,
+                                 const double* forms /* HOST [n_forms, 2n+3], or NULL: built-in cost */,
+                                 int n_forms, void* stream);
 /* number of per-block rows swm_rollout writes into stats_partial for this cfg when launched on `stream` of the
  * current device (depends on the kernel and the schedule it will choose; the schedule may differ while `stream`
  * is capturing a CUDA graph) */

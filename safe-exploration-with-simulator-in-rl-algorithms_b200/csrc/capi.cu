@@ -483,12 +483,12 @@ extern "C" int swm_rollout(const swm_params_t* params, const swm_rollout_t* cfg,
   return launch_thread_kernel(params->n, a, f, st);
 }
 
-extern "C" int swm_rollout_costed(const swm_params_t* params, const swm_rollout_t* cfg, const double* forms,
-                                  int n_forms, void* stream) {
-  if (!params_ok(params) || !cfg || !cfg->screen.enabled || !forms) return SWM_ERR_BAD_ARG;
-  if (n_forms < 1 || n_forms > SWM_MAX_COST_FORMS) return SWM_ERR_BAD_ARG;
-  const int cols = 2 * params->n + 3;  // A row (2n+2), then b
-  CostForms cf;
+namespace {
+
+// Copies and checks the host cost forms [n_forms, 2n+3] of swm_rollout_costed / swm_rollout_ensemble.
+int read_cost_forms(int n, const double* forms, int n_forms, CostForms& cf) {
+  if (!forms || n_forms < 1 || n_forms > SWM_MAX_COST_FORMS) return SWM_ERR_BAD_ARG;
+  const int cols = 2 * n + 3;  // A row (2n+2), then b
   memset(&cf, 0, sizeof(cf));
   cf.J = n_forms;
   for (int j = 0; j < n_forms; ++j)
@@ -497,18 +497,71 @@ extern "C" int swm_rollout_costed(const swm_params_t* params, const swm_rollout_
       if (!isfinite(v)) return SWM_ERR_BAD_ARG;
       cf.row[j][k] = v;
     }
-  RolloutArgs a;
-  RolloutFlags f;
-  int rc = build_rollout_args(params, cfg, a, f);
-  if (rc != SWM_OK) return rc;
-  // the costed cost runs on the one-thread-per-environment kernel only, always as one plain launch
+  return SWM_OK;
+}
+
+// The screening configurations of the costed and ensemble kernels: the one-thread-per-environment kernel only,
+// always as one plain launch, gym dynamics, linear policies, ARS V1 without statistics.
+int check_thread_screen(const swm_rollout_t* cfg, const RolloutFlags& f) {
   if (is_lane_kernel(cfg->kernel) || cfg->schedule_sub > 0) return SWM_ERR_UNSUPPORTED;
   if (cfg->variant != SWM_DYN_GYM || !f.linear || f.norm || f.stats) return SWM_ERR_UNSUPPORTED;
+  return SWM_OK;
+}
+
+}  // namespace
+
+extern "C" int swm_rollout_costed(const swm_params_t* params, const swm_rollout_t* cfg, const double* forms,
+                                  int n_forms, void* stream) {
+  if (!params_ok(params) || !cfg || !cfg->screen.enabled) return SWM_ERR_BAD_ARG;
+  CostForms cf;
+  int rc = read_cost_forms(params->n, forms, n_forms, cf);
+  if (rc != SWM_OK) return rc;
+  RolloutArgs a;
+  RolloutFlags f;
+  rc = build_rollout_args(params, cfg, a, f);
+  if (rc != SWM_OK) return rc;
+  rc = check_thread_screen(cfg, f);
+  if (rc != SWM_OK) return rc;
   if (cfg->B == 0) return SWM_OK;  // empty batch: nothing to do, pointers may be NULL
   rc = check_rollout_buffers(cfg, f);
   if (rc != SWM_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
 #define CALL(K) launch_rollout_costed_n<K>(a, cf, f, st)
+  SWM_DISPATCH_N(params->n, CALL)
+#undef CALL
+}
+
+extern "C" int swm_rollout_ensemble(const swm_params_t* params, const swm_rollout_t* cfg,
+                                    const swm_params_t* sim_models, int n_models, const double* forms, int n_forms,
+                                    void* stream) {
+  if (!params_ok(params) || !cfg || !cfg->screen.enabled) return SWM_ERR_BAD_ARG;
+  if (!sim_models || n_models < 1 || n_models > SWM_MAX_SIM_MODELS) return SWM_ERR_BAD_ARG;
+  SimModels sm;
+  memset(&sm, 0, sizeof(sm));
+  sm.M = n_models;
+  for (int m = 0; m < n_models; ++m) {
+    if (!params_ok(&sim_models[m]) || sim_models[m].n != params->n) return SWM_ERR_BAD_ARG;
+    sm.p[m] = make_phys(sim_models[m]);
+  }
+  CostForms cf;
+  if (forms) {
+    const int rc = read_cost_forms(params->n, forms, n_forms, cf);
+    if (rc != SWM_OK) return rc;
+  }
+  // cfg->screen.sim is not read: the kernel takes its models from `sm`
+  swm_rollout_t c = *cfg;
+  c.screen.sim = sim_models[0];
+  RolloutArgs a;
+  RolloutFlags f;
+  int rc = build_rollout_args(params, &c, a, f);
+  if (rc != SWM_OK) return rc;
+  rc = check_thread_screen(&c, f);
+  if (rc != SWM_OK) return rc;
+  if (c.B == 0) return SWM_OK;  // empty batch: nothing to do, pointers may be NULL
+  rc = check_rollout_buffers(&c, f);
+  if (rc != SWM_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+#define CALL(K) launch_rollout_ensemble_n<K>(a, sm, forms ? &cf : nullptr, f, st)
   SWM_DISPATCH_N(params->n, CALL)
 #undef CALL
 }

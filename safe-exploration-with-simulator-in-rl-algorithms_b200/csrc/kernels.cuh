@@ -192,18 +192,40 @@ __device__ __forceinline__ double cost_max_affine(const CostForms& f, const Obs&
   return m;
 }
 
-// Screening modes of the rollout kernel: none, the built-in cost max_i |thd_i|, or max-of-affine forms.
-enum ScreenMode { SCREEN_NONE = 0, SCREEN_BUILTIN = 1, SCREEN_AFFINE = 2 };
+// Screening modes of the rollout kernel: none, the built-in cost max_i |thd_i|, or max-of-affine forms, judged by
+// the simulator model of RolloutArgs::sim or (ENSEMBLE*) by every model of an ensemble.
+enum ScreenMode {
+  SCREEN_NONE = 0, SCREEN_BUILTIN = 1, SCREEN_AFFINE = 2, SCREEN_ENSEMBLE = 3, SCREEN_ENSEMBLE_AFFINE = 4
+};
 
-// Type of the rollout kernel's second argument: the cost forms for SCREEN_AFFINE, an empty struct otherwise.
+// The simulator models of ensemble screening (M = 1..SWM_MAX_SIM_MODELS; entries from M on are not read).
+struct SimModels {
+  int M;
+  Phys p[SWM_MAX_SIM_MODELS];
+};
+struct SimModelsForms {
+  SimModels models;
+  CostForms forms;
+};
+
+// Type of the rollout kernel's second argument: the cost forms and / or the simulator models of the screening
+// mode, an empty struct without either.
 struct NoCostForms {};
 template <int SCREEN> struct ScreenForms { using type = NoCostForms; };
 template <> struct ScreenForms<SCREEN_AFFINE> { using type = CostForms; };
+template <> struct ScreenForms<SCREEN_ENSEMBLE> { using type = SimModels; };
+template <> struct ScreenForms<SCREEN_ENSEMBLE_AFFINE> { using type = SimModelsForms; };
+
+__device__ __forceinline__ const CostForms& cost_forms_of(const CostForms& f) { return f; }
+__device__ __forceinline__ const CostForms& cost_forms_of(const SimModelsForms& f) { return f.forms; }
+__device__ __forceinline__ const SimModels& sim_models_of(const SimModels& s) { return s; }
+__device__ __forceinline__ const SimModels& sim_models_of(const SimModelsForms& s) { return s.models; }
 
 // LINEAR: 0 fixed actions, 1 linear policy.  NORM: ARS V2 normalisation.  STATS: accumulate
 // shifted first/second moments of every visited state.  SCREEN: per-step simulator screening (ScreenMode).
-// With SCREEN_AFFINE the forms travel as the second kernel argument (5.9 KB of the constant bank); the other
-// kernels' argument block grows by one empty byte only.
+// With SCREEN_AFFINE the forms travel as the second kernel argument (5.9 KB of the constant bank), with
+// SCREEN_ENSEMBLE the models (2.3 KB), with SCREEN_ENSEMBLE_AFFINE both (8.2 KB); the other kernels' argument
+// block grows by one empty byte only.
 template <int N, int VARIANT, int WMODE, bool NORM, bool STATS, int SCREEN>
 __global__ void __launch_bounds__(kRolloutBlock, SWM_ROLLOUT_MIN_BLOCKS)
 rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms<SCREEN>::type forms) {
@@ -406,7 +428,7 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
         if (VARIANT == 0) ut[k] = v * a.real.u_scale;
       }
     }
-    if (SCREEN != SCREEN_NONE) {
+    if (SCREEN == SCREEN_BUILTIN || SCREEN == SCREEN_AFFINE) {
       // Safe_ARS.isSafe (safe_ars/ars.py:111-122): one simulator step from the current state.  The
       // simulator starts from the same angles, so it shares this step's sines/cosines and needs only
       // its own accelerations.
@@ -452,6 +474,63 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
         break;
       }
     }
+    if constexpr (SCREEN == SCREEN_ENSEMBLE || SCREEN == SCREEN_ENSEMBLE_AFFINE) {
+      // The block above once per simulator model (written out separately so that the single-model kernels keep
+      // their code): every model must judge the step safe.  The decisions are OR-ed (not the costs maxed), so that
+      // the order of the models cannot matter.  No early exit: a safe step needs all M evaluations, and an unsafe one
+      // ends the rollout.  Models 1..M-1 run in a loop, reading their constants from the constant bank through the
+      // runtime index m; model 0 runs last, in straight-line code directly before the real step, as in the
+      // single-model kernels.  That keeps one model bit-identical to them: there the compiler shares the
+      // model-independent products of the simulator's accelerations (of the sines, cosines and velocities) with the
+      // real step, which then keeps them as separately rounded multiplies; without the shared copy the real step
+      // fuses one of them into an FMA instead (one ulp in the real trajectory).  The loop works on opaque copies of
+      // the sines, cosines and velocities, so that none of its products is hoisted and shared with the code after
+      // it (which would keep them live across the loop).
+      const SimModels& sm = sim_models_of(forms);
+      auto model_unsafe = [&](const Phys& P, const double (&s)[N], const double (&c)[N],
+                              const double (&w)[N]) -> bool {
+        double sut[NA > 0 ? NA : 1], sgddx, sgddy, sthdd[N];
+#pragma unroll
+        for (int k = 0; k < NA; ++k) sut[k] = u[k] * P.u_scale;
+        gym_accel<N, FS>(P, s, c, gdx, gdy, w, sut, sgddx, sgddy, sthdd, sF);
+        double sim_cost;
+        if constexpr (SCREEN == SCREEN_ENSEMBLE_AFFINE) {
+          auto so = [&](int k) {
+            if (k < 2) return fma(P.h_gdd_c, k == 0 ? sgddx : sgddy, k == 0 ? gdx : gdy);
+            const int i = (k - 2) / 2;
+            return (k & 1) ? fma(P.h, sthdd[i], w[i]) : fma(P.h, w[i], th[i]);
+          };
+          sim_cost = cost_max_affine<NO>(cost_forms_of(forms), so);
+        } else {
+          double sthd[N];
+#pragma unroll
+          for (int i = 0; i < N; ++i) sthd[i] = fma(P.h, sthdd[i], w[i]);
+          sim_cost = cost_max_abs_thd<N>(sthd);
+        }
+        return !(sim_cost <= a.sim_thresh);
+      };
+      bool unsafe = false;
+#pragma unroll 1
+      for (int m = 1; m < sm.M; ++m) {
+        double s[N], c[N], w[N];
+#pragma unroll
+        for (int i = 0; i < N; ++i) { s[i] = opaque(sn[i]); c[i] = opaque(cs[i]); w[i] = opaque(thd[i]); }
+        unsafe |= model_unsafe(sm.p[m], s, c, w);
+      }
+      unsafe |= model_unsafe(sm.p[0], sn, cs, thd);
+      if (unsafe) {
+        frozen = t;
+        if (traj && active) {
+          for (int tt = t; tt < a.H; ++tt) {
+            double* o = traj + (long long)tt * traj_step;
+            o[0] = gdx; o[1] = gdy;
+#pragma unroll
+            for (int i = 0; i < N; ++i) { o[2 + 2 * i] = th[i]; o[3 + 2 * i] = thd[i]; }
+          }
+        }
+        break;
+      }
+    }
     if (VARIANT == 0) {
       // reward_t = Gdot_t . direction (remy_swimmer_env.py:238-243); the two components are summed
       // separately and dotted with the direction once, after the loop
@@ -461,13 +540,14 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
     } else {
       ret += swimmer_step<N, 1>(a.real, gdx, gdy, th, thd, u);
     }
-    if (SCREEN == SCREEN_BUILTIN) viol += (cost_max_abs_thd<N>(thd) > a.real_thresh) ? 1 : 0;
-    if constexpr (SCREEN == SCREEN_AFFINE) {
+    if (SCREEN == SCREEN_BUILTIN || SCREEN == SCREEN_ENSEMBLE)
+      viol += (cost_max_abs_thd<N>(thd) > a.real_thresh) ? 1 : 0;
+    if constexpr (SCREEN == SCREEN_AFFINE || SCREEN == SCREEN_ENSEMBLE_AFFINE) {
       double x[NO];
       x[0] = gdx; x[1] = gdy;
 #pragma unroll
       for (int i = 0; i < N; ++i) { x[2 + 2 * i] = th[i]; x[3 + 2 * i] = thd[i]; }
-      viol += (cost_max_affine<NO>(forms, [&](int k) { return x[k]; }) > a.real_thresh) ? 1 : 0;
+      viol += (cost_max_affine<NO>(cost_forms_of(forms), [&](int k) { return x[k]; }) > a.real_thresh) ? 1 : 0;
     }
     if (STATS) {
       double x[NO];

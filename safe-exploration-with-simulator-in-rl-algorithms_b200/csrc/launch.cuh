@@ -18,6 +18,8 @@ template <int N> int launch_step_n(const Phys& P, int variant, bool acc_only, co
 template <int N> int launch_rollout_n(const RolloutArgs& a, const RolloutFlags& f, cudaStream_t st);
 template <int N> int launch_rollout_costed_n(const RolloutArgs& a, const CostForms& forms, const RolloutFlags& f,
                                              cudaStream_t st);
+template <int N> int launch_rollout_ensemble_n(const RolloutArgs& a, const SimModels& models, const CostForms* forms,
+                                               const RolloutFlags& f, cudaStream_t st);
 template <int N> int launch_step_models_n(const PhysSet& set, long long envs_per_model, const double* state_in,
                                           const double* action, double* out, double* reward, long long B,
                                           cudaStream_t st);
@@ -72,6 +74,33 @@ int launch_rollout_costed_n(const RolloutArgs& a, const CostForms& forms, const 
   } else {
     if (f.group_w) return launch_rollout_costed_one<N, W_SMEM_GROUP>(a, forms, st);
     return launch_rollout_costed_one<N, W_SMEM_THREAD>(a, forms, st);
+  }
+}
+
+// Ensemble screening: SCREEN_ENSEMBLE with the built-in cost (forms == nullptr), else SCREEN_ENSEMBLE_AFFINE.
+template <int N, int WMODE>
+static int launch_rollout_ensemble_one(const RolloutArgs& a, const SimModels& models, const CostForms* forms,
+                                       cudaStream_t st) {
+  const size_t smem = rollout_smem<N, 0, WMODE, false>();
+  if (!forms) return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_ENSEMBLE>, smem, a.B, st,
+                                         a, models);
+  SimModelsForms mf;
+  mf.models = models;
+  mf.forms = *forms;
+  return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_ENSEMBLE_AFFINE>, smem, a.B, st, a, mf);
+}
+
+// Same configurations as the costed kernel.
+template <int N>
+int launch_rollout_ensemble_n(const RolloutArgs& a, const SimModels& models, const CostForms* forms,
+                              const RolloutFlags& f, cudaStream_t st) {
+  constexpr int WS = (N - 1) * (2 * N + 2);
+  if (f.variant != SWM_DYN_GYM || !f.linear || !f.screen || f.norm || f.stats) return SWM_ERR_UNSUPPORTED;
+  if constexpr (WS <= kRegPolicyMax) {
+    return launch_rollout_ensemble_one<N, W_REG>(a, models, forms, st);
+  } else {
+    if (f.group_w) return launch_rollout_ensemble_one<N, W_SMEM_GROUP>(a, models, forms, st);
+    return launch_rollout_ensemble_one<N, W_SMEM_THREAD>(a, models, forms, st);
   }
 }
 
@@ -136,6 +165,8 @@ template int launch_step_n<SWM_INSTANTIATE_N>(const Phys&, int, bool, const doub
 template int launch_rollout_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const RolloutFlags&, cudaStream_t);
 template int launch_rollout_costed_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const CostForms&, const RolloutFlags&,
                                                         cudaStream_t);
+template int launch_rollout_ensemble_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const SimModels&, const CostForms*,
+                                                          const RolloutFlags&, cudaStream_t);
 
 #endif  // SWM_INSTANTIATE_N
 

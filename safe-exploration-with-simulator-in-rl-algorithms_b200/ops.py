@@ -151,6 +151,8 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
     screen = dict(sim_params=..., sim_thresh=..., real_thresh=...) enables Safe_ARS screening with the built-in
     cost max_i |thd_i|; screen["cost"] = a max-of-affine cost (safe_ars.MaxAffineCost: `.n`, `.forms` [J, 2n+3])
     screens with that cost instead (swm_rollout_costed; one thread per environment, one plain launch).
+    screen["sim_params"] = a list or tuple of 1..16 params (the real model's n) screens by the whole ensemble, with
+    either cost: a step is taken only if every model judges it safe (swm_rollout_ensemble; same kernel and launch).
     stats_pivot[2n+2] enables the V2 moment accumulation.  `out` may carry preallocated
     tensors (returns, final_state, trajectory, stats_partial) to stay allocation-free in loops.
     kernel: _lib.KERNEL_AUTO (chosen from B, n and the SM count) / KERNEL_THREAD (one thread per
@@ -250,9 +252,13 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
         res.samples = float(B) * float(H)
         cfg.stats_partial, cfg.stats_pivot = res.stats_partial.data_ptr(), stats_pivot.data_ptr()
         keep.append(stats_pivot)
+    sim_models = None
     if screen is not None:
         cfg.screen.enabled = 1
-        cfg.screen.sim = screen["sim_params"]
+        if isinstance(screen["sim_params"], (list, tuple)):
+            sim_models = screen["sim_params"]  # an ensemble: cfg.screen.sim is not read
+        else:
+            cfg.screen.sim = screen["sim_params"]
         cfg.screen.sim_thresh = float(screen["sim_thresh"])
         cfg.screen.real_thresh = float(screen["real_thresh"])
         res.violations = buf("violations", (B,), torch.int32)
@@ -260,13 +266,19 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
         cfg.screen.violations = res.violations.data_ptr()
         cfg.screen.frozen_at = res.frozen_at.data_ptr()
     cost = screen.get("cost") if screen is not None else None
+    if cost is not None and cost.n != n:
+        raise ValueError("the cost is for n=%d segments, the model has n=%d" % (cost.n, n))
+    forms = cost.forms if cost is not None else None  # host [J, 2n+3], copied into the launch's arguments
     with torch.cuda.device(dev):
-        if cost is None:
+        if sim_models is not None:
+            models = (_lib.SwmParams * len(sim_models))(*sim_models)  # host copies, copied into the launch's arguments
+            _lib.check(_lib.lib().swm_rollout_ensemble(
+                ctypes.byref(params), ctypes.byref(cfg), models, len(sim_models),
+                None if forms is None else forms.ctypes.data_as(ctypes.c_void_p),
+                0 if forms is None else forms.shape[0], _lib.stream_ptr()))
+        elif cost is None:
             _lib.check(_lib.lib().swm_rollout(ctypes.byref(params), ctypes.byref(cfg), _lib.stream_ptr()))
         else:
-            if cost.n != n:
-                raise ValueError("the cost is for n=%d segments, the model has n=%d" % (cost.n, n))
-            forms = cost.forms  # host [J, 2n+3], copied into the launch's arguments
             _lib.check(_lib.lib().swm_rollout_costed(ctypes.byref(params), ctypes.byref(cfg),
                                                      forms.ctypes.data_as(ctypes.c_void_p), forms.shape[0],
                                                      _lib.stream_ptr()))

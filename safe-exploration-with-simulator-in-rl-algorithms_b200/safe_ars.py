@@ -132,31 +132,54 @@ class Basic_ARS:
 
 
 class Safe_ARS(Basic_ARS):
-    """ARS V1 with per-step safe exploration through a simulator (safe_ars/ars.py:103-153)."""
+    """ARS V1 with per-step safe exploration through a simulator (safe_ars/ars.py:103-153).
+
+    `sim_env` may also be a sequence of 1..16 SwimmerEnv (an ensemble of simulator models, e.g. points of the set
+    the real parameters are known to lie in): a step is then taken only if every model judges it safe."""
 
     def __init__(self, cost, real_threshold, sim_threshold, sim_env):
-        assert isinstance(sim_env, SwimmerEnv)
-        if isinstance(cost, MaxAffineCost):
-            if cost.n != sim_env.n:
-                raise ValueError("the cost is for n=%d segments, the environment has n=%d" % (cost.n, sim_env.n))
+        if isinstance(sim_env, SwimmerEnv):
+            n = sim_env.n
         else:
-            _check_cost(cost, sim_env.n)
+            envs = list(sim_env)
+            if not 1 <= len(envs) <= _lib.MAX_SIM_MODELS:
+                raise ValueError("an ensemble has 1 to %d simulator models, got %d" % (_lib.MAX_SIM_MODELS, len(envs)))
+            assert all(isinstance(e, SwimmerEnv) for e in envs)
+            n = envs[0].n
+            if any(e.n != n for e in envs):
+                raise ValueError("the simulator models of an ensemble must have the same n, got %s"
+                                 % [e.n for e in envs])
+            sim_env = envs
+        if isinstance(cost, MaxAffineCost):
+            if cost.n != n:
+                raise ValueError("the cost is for n=%d segments, the environment has n=%d" % (cost.n, n))
+        else:
+            _check_cost(cost, n)
         self.cost = cost
         self.real_thresh = real_threshold
         self.sim_thresh = sim_threshold
         self.sim_env = sim_env
 
     def _screen(self, real_env):
-        assert self.sim_env.n == real_env.n
-        screen = dict(sim_params=self.sim_env.params(), sim_thresh=self.sim_thresh,
-                      real_thresh=self.real_thresh)
+        if isinstance(self.sim_env, SwimmerEnv):
+            assert self.sim_env.n == real_env.n
+            sim = self.sim_env.params()
+        else:
+            if self.sim_env[0].n != real_env.n:
+                raise ValueError("the simulator models have n=%d segments, the real environment has n=%d"
+                                 % (self.sim_env[0].n, real_env.n))
+            sim = [e.params() for e in self.sim_env]
+        screen = dict(sim_params=sim, sim_thresh=self.sim_thresh, real_thresh=self.real_thresh)
         if isinstance(self.cost, MaxAffineCost):
             screen["cost"] = self.cost
         return screen
 
     def isSafe(self, cost, thresh, env, state, action):
         """Simulate `action` from `state` on `env` and compare the cost with the threshold
-        (safe_ars/ars.py:111-122).  Leaves env in the simulated state, like the reference."""
+        (safe_ars/ars.py:111-122).  Leaves env in the simulated state, like the reference.  With a sequence of
+        environments: True only if every one of them is safe; each is left in its simulated state."""
+        if not isinstance(env, SwimmerEnv):
+            return all([self.isSafe(cost, thresh, e, state, action) for e in env])
         env.set_state(state)
         obs, _, _, _ = env.step(action)
         return cost(obs) <= thresh
