@@ -235,6 +235,20 @@ SWM_API int swm_rollout_ensemble(const swm_params_t* params, const swm_rollout_t
                                  const swm_params_t* sim_models /* HOST [n_models] */, int n_models,
                                  const double* forms /* HOST [n_forms, 2n+3], or NULL: built-in cost */,
                                  int n_forms, void* stream);
+/* Model-set rollouts: the rollouts of swm_rollout under each of n_models models (HOST array, 1..SWM_MAX_SIM_MODELS
+ * structs with the same n) in one launch.  Rollout e of model m is exactly what environment e of swm_rollout with
+ * params = &models[m] would run (same policy, perturbation, Philox counters, start state and init_perturb); only its
+ * physics comes from model m.  cfg->B is the number of environments PER MODEL; returns is [n_models, B] and
+ * final_state [n_models, B, 2n+2] or NULL; every other field means what it does for swm_rollout and is shared by all
+ * models.  The models are copied into the launch's arguments (a captured CUDA graph keeps the values of the call).
+ * Kernel: cfg->kernel, or under AUTO the one swm_rollout picks for a plain batch of n_models * B environments; always
+ * one launch, model m in CTA row m.  Bit-identical to swm_rollout of each model on the same kernel.
+ * This is the simulator side of reward-constraint screening by an ensemble (swm_screen_mask_models).
+ * SWM_ERR_BAD_ARG: n_models outside 1..SWM_MAX_SIM_MODELS, models NULL, a model that is not a valid swm_params_t or
+ * has another n than models[0], or whatever swm_rollout rejects.  SWM_ERR_UNSUPPORTED: the rlglue variant, fixed
+ * actions, screen.enabled, stats_partial, trajectory, clip_actions, schedule_sub > 0. */
+SWM_API int swm_rollout_models(const swm_params_t* models /* HOST [n_models] */, int n_models,
+                               const swm_rollout_t* cfg, void* stream);
 /* number of per-block rows swm_rollout writes into stats_partial for this cfg when launched on `stream` of the
  * current device (depends on the kernel and the schedule it will choose; the schedule may differ while `stream`
  * is capturing a CUDA graph) */
@@ -299,6 +313,14 @@ SWM_API int swm_ars_update(double* W, int wsize, const double* returns, int N, c
  * device int64 running total (+= survivors), e.g. the screened fraction of a whole training run. */
 SWM_API int swm_screen_mask(const double* sim_returns, int N, double threshold, int32_t* mask,
                             int32_t* n_pass, int64_t* n_pass_total, void* stream);
+
+/* swm_screen_mask over an ensemble: sim_returns is [n_models, 2N] (row m = the 2N simulated returns under model m,
+ * as swm_rollout_models writes them for R = 1) and
+ *   mask[k] = AND over m of (sim_returns[m, 2k] > threshold && sim_returns[m, 2k+1] > threshold),
+ * NaN screened out.  n_pass / n_pass_total as for swm_screen_mask, which is this call with n_models = 1.
+ * SWM_ERR_BAD_ARG: n_models outside 1..SWM_MAX_SIM_MODELS, N < 1, sim_returns or mask NULL. */
+SWM_API int swm_screen_mask_models(const double* sim_returns, int n_models, int N, double threshold, int32_t* mask,
+                                   int32_t* n_pass, int64_t* n_pass_total, void* stream);
 
 /* select_action for a batch (ars/environment.py:19-35): actions[B, n-1] = W_e obs_e (V1) or
  * (W_e diag(inv_sigma)) (obs_e - mean) (V2); env e uses policy e / rollouts_per_policy of

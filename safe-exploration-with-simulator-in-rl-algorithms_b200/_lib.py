@@ -128,6 +128,7 @@ def lib():
     L.swm_rollout.argtypes = [pp, ctypes.POINTER(SwmRollout), _dp]
     L.swm_rollout_costed.argtypes = [pp, ctypes.POINTER(SwmRollout), _dp, c_int, _dp]
     L.swm_rollout_ensemble.argtypes = [pp, ctypes.POINTER(SwmRollout), pp, c_int, _dp, c_int, _dp]
+    L.swm_rollout_models.argtypes = [pp, c_int, ctypes.POINTER(SwmRollout), _dp]
     L.swm_rollout_stats_blocks.argtypes = [pp, ctypes.POINTER(SwmRollout), _dp]
     L.swm_rollout_stats_blocks.restype = i64
     L.swm_rollout_kernel_choice.argtypes = [pp, ctypes.POINTER(SwmRollout)]
@@ -139,6 +140,7 @@ def lib():
     L.swm_ars_update.argtypes = [_dp, c_int, _dp, c_int, _dp, c_int, _dp, dbl, c_int, dbl,
                                  ctypes.POINTER(SwmPhilox), _dp, _dp, _dp]
     L.swm_screen_mask.argtypes = [_dp, c_int, dbl, _dp, _dp, _dp, _dp]
+    L.swm_screen_mask_models.argtypes = [_dp, c_int, c_int, dbl, _dp, _dp, _dp, _dp]
     L.swm_policy_actions.argtypes = [pp, _dp, _dp, c_int, _dp, _dp, c_int, _dp, i64, _dp]
     L.swm_philox_deltas.argtypes = [ctypes.POINTER(SwmPhilox), c_int, c_int, _dp, _dp]
     L.swm_fp64_probe.argtypes = [c_int, c_int, c_int, _dp, ctypes.POINTER(dbl), _dp]

@@ -41,8 +41,13 @@ def _env_params(p, variant_direction=(1.0, 0.0)):
 class ARSAgent:
     def __init__(self, real_env_param, agent_param, data_path=None, seed=None, guess_param=None,
                  approx_error=None, sim_thresh=None, *, delta_source="numpy", keep_states=False,
-                 record_trajectories=None, device=None, group=None, distributed=None):
+                 record_trajectories=None, device=None, group=None, distributed=None, sim_models=None):
+        """sim_models: optional list of 1..16 EnvParam (the real model's n).  In safe mode a direction is then rolled
+        out in the real world only if both its simulated returns exceed sim_threshold under EVERY one of these
+        models, instead of under the single estimated_param (which is still computed as the reference does)."""
         assert delta_source in ("numpy", "philox")
+        if sim_models is not None and not agent_param.safe:
+            raise ValueError("sim_models screens directions in safe mode only")
         self.real_env_param = real_env_param
         self.real_world = Environment(real_env_param, device=device)
         self.agent_param = agent_param
@@ -93,7 +98,8 @@ class ARSAgent:
             _env_params(real_env_param), N=agent_param.N, b=agent_param.b, alpha=agent_param.alpha,
             nu=agent_param.nu, H=agent_param.H, v2=not agent_param.V1, semantics=ARS_AGENT,
             seed=seed, initial_policy=W0, device=device, group=group, distributed=distributed,
-            sim_params=_env_params(self.estimated_param) if agent_param.safe else None,
+            sim_params=(None if not agent_param.safe else _env_params(self.estimated_param) if sim_models is None
+                        else [_env_params(p) for p in sim_models]),
             sim_threshold=self.sim_threshold)
         self.record_trajectories = record_trajectories
         self.saved_states = []

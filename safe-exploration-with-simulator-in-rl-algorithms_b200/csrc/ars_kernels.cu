@@ -124,9 +124,9 @@ ars_update_kernel(double* __restrict__ W, int wsize, const double* __restrict__ 
   }
 }
 
-// mask[k] = both simulated returns of direction k exceed the simulator threshold
-// (ars_agent.py:150-157: `reward <= sim_threshold` => no real rollout).
-__global__ void screen_mask_kernel(const double* __restrict__ sim_returns, int N, double threshold,
+// mask[k] = both simulated returns of direction k exceed the simulator threshold under every one of the M models
+// (rows of 2N returns) (ars_agent.py:150-157: `reward <= sim_threshold` => no real rollout).
+__global__ void screen_mask_kernel(const double* __restrict__ sim_returns, int M, int N, double threshold,
                                    int* __restrict__ mask, int* __restrict__ n_pass,
                                    long long* __restrict__ n_pass_total) {
   __shared__ double red[kArsBlock / 32];
@@ -134,7 +134,12 @@ __global__ void screen_mask_kernel(const double* __restrict__ sim_returns, int N
   for (int k = threadIdx.x; k < N; k += kArsBlock) {
     // The reference skips on `reward <= sim_threshold`; a NaN simulator return (diverged simulation) compares
     // false there and would be rolled out in the real world.  Declared deviation: NaN is screened out too.
-    const bool skip = !((sim_returns[2 * k] > threshold) && (sim_returns[2 * k + 1] > threshold));
+    bool pass = true;
+    for (int m = 0; m < M; ++m) {
+      const double* r = sim_returns + (long long)m * 2 * N;
+      pass = pass && (r[2 * k] > threshold) && (r[2 * k + 1] > threshold);
+    }
+    const bool skip = !pass;
     mask[k] = skip ? 0 : 1;
     c += skip ? 0.0 : 1.0;
   }
@@ -324,8 +329,13 @@ extern "C" int swm_ars_update(double* W, int wsize, const double* returns, int N
 
 extern "C" int swm_screen_mask(const double* sim_returns, int N, double threshold, int32_t* mask,
                                int32_t* n_pass, int64_t* n_pass_total, void* stream) {
-  if (!sim_returns || !mask || N < 1) return SWM_ERR_BAD_ARG;
-  screen_mask_kernel<<<1, kArsBlock, 0, (cudaStream_t)stream>>>(sim_returns, N, threshold, mask, n_pass,
+  return swm_screen_mask_models(sim_returns, 1, N, threshold, mask, n_pass, n_pass_total, stream);
+}
+
+extern "C" int swm_screen_mask_models(const double* sim_returns, int n_models, int N, double threshold, int32_t* mask,
+                                      int32_t* n_pass, int64_t* n_pass_total, void* stream) {
+  if (!sim_returns || !mask || N < 1 || n_models < 1 || n_models > SWM_MAX_SIM_MODELS) return SWM_ERR_BAD_ARG;
+  screen_mask_kernel<<<1, kArsBlock, 0, (cudaStream_t)stream>>>(sim_returns, n_models, N, threshold, mask, n_pass,
                                                               reinterpret_cast<long long*>(n_pass_total));
   return SWM_CHECK_LAUNCH();
 }

@@ -566,6 +566,46 @@ extern "C" int swm_rollout_ensemble(const swm_params_t* params, const swm_rollou
 #undef CALL
 }
 
+extern "C" int swm_rollout_models(const swm_params_t* models, int n_models, const swm_rollout_t* cfg, void* stream) {
+  if (!models || n_models < 1 || n_models > SWM_MAX_SIM_MODELS || !cfg) return SWM_ERR_BAD_ARG;
+  SimModels sm;
+  memset(&sm, 0, sizeof(sm));
+  sm.M = n_models;
+  for (int m = 0; m < n_models; ++m) {
+    if (!params_ok(&models[m]) || models[m].n != models[0].n) return SWM_ERR_BAD_ARG;
+    sm.p[m] = make_phys(models[m]);
+  }
+  RolloutArgs a;
+  RolloutFlags f;
+  int rc = build_rollout_args(&models[0], cfg, a, f);
+  if (rc != SWM_OK) return rc;
+  // what the model-set kernels implement: the simulator rollouts of ARS screening (V1 / V2 without moments)
+  if (cfg->variant != SWM_DYN_GYM || !f.linear || f.screen || f.stats || cfg->trajectory || cfg->clip_actions ||
+      cfg->schedule_sub > 0)
+    return SWM_ERR_UNSUPPORTED;
+  if (cfg->B == 0) return SWM_OK;  // empty batch: nothing to do, pointers may be NULL
+  rc = check_rollout_buffers(cfg, f);
+  if (rc != SWM_OK) return rc;
+  // the kernel swm_rollout would pick for all n_models * B environments as one plain batch
+  swm_rollout_t whole = *cfg;
+  whole.B = (int64_t)n_models * cfg->B;
+  RolloutArgs wa;
+  RolloutFlags wf;
+  rc = build_rollout_args(&models[0], &whole, wa, wf);
+  if (rc != SWM_OK) return rc;
+  const int kernel = choose_kernel(models[0].n, &whole, wa, wf);
+  if (kernel < 0) return kernel;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (is_lane_kernel(kernel)) {
+#define CALL(K) launch_lane_rollout_models_n<K>(a, sm, f, kernel == SWM_KERNEL_LANES3 ? 2 : kernel == SWM_KERNEL_LANES2 ? 1 : 0, st)
+    SWM_DISPATCH_N(models[0].n, CALL)
+#undef CALL
+  }
+#define CALL(K) launch_rollout_models_n<K>(a, sm, f, st)
+  SWM_DISPATCH_N(models[0].n, CALL)
+#undef CALL
+}
+
 // Layout self-check for language bindings: sizes of the ABI structs as this build sees them.
 extern "C" int swm_abi_struct_sizes(int* params, int* philox, int* screen, int* rollout) {
   if (params) *params = (int)sizeof(swm_params_t);

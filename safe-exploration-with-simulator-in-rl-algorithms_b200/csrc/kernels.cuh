@@ -209,12 +209,26 @@ struct SimModelsForms {
 };
 
 // Type of the rollout kernel's second argument: the cost forms and / or the simulator models of the screening
-// mode, an empty struct without either.
+// mode, an empty struct without either.  MODELS (model-set mode, unscreened only): the models whose physics the
+// rollouts run, one per CTA row blockIdx.y; the lane-split kernels take the same argument.
 struct NoCostForms {};
-template <int SCREEN> struct ScreenForms { using type = NoCostForms; };
+template <int SCREEN, bool MODELS = false> struct ScreenForms { using type = NoCostForms; };
 template <> struct ScreenForms<SCREEN_AFFINE> { using type = CostForms; };
 template <> struct ScreenForms<SCREEN_ENSEMBLE> { using type = SimModels; };
 template <> struct ScreenForms<SCREEN_ENSEMBLE_AFFINE> { using type = SimModelsForms; };
+template <> struct ScreenForms<SCREEN_NONE, true> { using type = SimModels; };
+
+// The physics of a rollout: RolloutArgs::real, or in the model-set mode model blockIdx.y (warp- and CTA-uniform, read
+// from the constant bank through that index).  Rollout e of model m writes its outputs at row m * B + e.
+template <bool MODELS, typename F>
+__device__ __forceinline__ const Phys& rollout_model(const RolloutArgs& a, const F& f) {
+  if constexpr (MODELS) return f.p[blockIdx.y];
+  else return a.real;
+}
+template <bool MODELS>
+__device__ __forceinline__ long long output_row(const RolloutArgs& a, long long e) {
+  return MODELS ? (long long)blockIdx.y * a.B + e : e;
+}
 
 __device__ __forceinline__ const CostForms& cost_forms_of(const CostForms& f) { return f; }
 __device__ __forceinline__ const CostForms& cost_forms_of(const SimModelsForms& f) { return f.forms; }
@@ -225,12 +239,15 @@ __device__ __forceinline__ const SimModels& sim_models_of(const SimModelsForms& 
 // shifted first/second moments of every visited state.  SCREEN: per-step simulator screening (ScreenMode).
 // With SCREEN_AFFINE the forms travel as the second kernel argument (5.9 KB of the constant bank), with
 // SCREEN_ENSEMBLE the models (2.3 KB), with SCREEN_ENSEMBLE_AFFINE both (8.2 KB); the other kernels' argument
-// block grows by one empty byte only.
-template <int N, int VARIANT, int WMODE, bool NORM, bool STATS, int SCREEN>
+// block grows by one empty byte only.  MODELS: the model-set mode (SCREEN_NONE, gym dynamics, no statistics, no
+// trajectory), the models (2.3 KB) as the second argument.
+template <int N, int VARIANT, int WMODE, bool NORM, bool STATS, int SCREEN, bool MODELS>
 __global__ void __launch_bounds__(kRolloutBlock, SWM_ROLLOUT_MIN_BLOCKS)
-rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms<SCREEN>::type forms) {
+rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms<SCREEN, MODELS>::type forms) {
+  static_assert(!MODELS || (SCREEN == SCREEN_NONE && VARIANT == 0 && !STATS), "model set: unscreened gym rollouts");
   constexpr int NO = 2 * N + 2, NA = N - 1, WS = NA * NO;
   constexpr bool LINEAR = (WMODE != W_NONE);
+  const Phys& P = rollout_model<MODELS>(a, forms);
   extern __shared__ __align__(16) double smem[];
   const int tid = threadIdx.x;
   const long long e0 = (long long)blockIdx.x * kRolloutBlock + tid;
@@ -390,7 +407,7 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
     for (int i = 0; i < N; ++i) sincos(th[i], &sn[i], &cs[i]);
     if (!LINEAR) {
 #pragma unroll
-      for (int k = 0; k < NA; ++k) ut[k] = u[k] * a.real.u_scale;
+      for (int k = 0; k < NA; ++k) ut[k] = u[k] * P.u_scale;
     }
   }
 
@@ -423,9 +440,9 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
 #pragma unroll
       for (int k = 0; k < NA; ++k) {
         double v = acc[k];
-        if (a.clip) v = fmin(fmax(v, -a.real.max_u), a.real.max_u);
+        if (a.clip) v = fmin(fmax(v, -P.max_u), P.max_u);
         u[k] = v;
-        if (VARIANT == 0) ut[k] = v * a.real.u_scale;
+        if (VARIANT == 0) ut[k] = v * P.u_scale;
       }
     }
     if (SCREEN == SCREEN_BUILTIN || SCREEN == SCREEN_AFFINE) {
@@ -534,11 +551,11 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
     if (VARIANT == 0) {
       // reward_t = Gdot_t . direction (remy_swimmer_env.py:238-243); the two components are summed
       // separately and dotted with the direction once, after the loop
-      gym_step_tracked<N, FS>(a.real, gdx, gdy, th, thd, sn, cs, ut, (t & 63) == 63, sF);
+      gym_step_tracked<N, FS>(P, gdx, gdy, th, thd, sn, cs, ut, (t & 63) == 63, sF);
       sgx += gdx;
       sgy += gdy;
     } else {
-      ret += swimmer_step<N, 1>(a.real, gdx, gdy, th, thd, u);
+      ret += swimmer_step<N, 1>(P, gdx, gdy, th, thd, u);
     }
     if (SCREEN == SCREEN_BUILTIN || SCREEN == SCREEN_ENSEMBLE)
       viol += (cost_max_abs_thd<N>(thd) > a.real_thresh) ? 1 : 0;
@@ -574,11 +591,12 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
     }
   }
 
-  if (VARIANT == 0) ret += fma(sgx, a.real.dirx, sgy * a.real.diry);
+  if (VARIANT == 0) ret += fma(sgx, P.dirx, sgy * P.diry);
   if (active) {
-    a.returns[e] = a.accumulate ? a.returns[e] + ret : ret;
+    const long long eo = output_row<MODELS>(a, e);
+    a.returns[eo] = a.accumulate ? a.returns[eo] + ret : ret;
     if (a.final_state) {
-      double2* o = reinterpret_cast<double2*>(a.final_state + e * NO);
+      double2* o = reinterpret_cast<double2*>(a.final_state + eo * NO);
       o[0] = make_double2(gdx, gdy);
 #pragma unroll
       for (int i = 0; i < N; ++i) o[1 + i] = make_double2(th[i], thd[i]);

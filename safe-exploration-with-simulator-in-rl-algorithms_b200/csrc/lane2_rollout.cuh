@@ -46,9 +46,11 @@ __device__ __forceinline__ void named_bar_arrive(int id) { asm volatile("bar.arr
 // the non-dimensional form the joint matrix only depends on the angles, so the simulator's accelerations are a second
 // right-hand side dotted with the SAME solution rows; an environment judged unsafe freezes for the rest of the horizon
 // (its lanes keep taking part in the exchanges, nothing of it advances).
-template <int N, bool LINEAR, bool NORM, bool STATS, int NF = 1, bool SCREEN = false>
+// MODELS: the model-set mode of rollout_kernel (CTA row blockIdx.y runs model blockIdx.y; warp F needs no model).
+template <int N, bool LINEAR, bool NORM, bool STATS, int NF, bool SCREEN, bool MODELS>
 __global__ void __launch_bounds__(32 * (1 + NF))
-lane2_rollout_kernel(const RolloutArgs a) {
+lane2_rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms<SCREEN_NONE, MODELS>::type models) {
+  static_assert(!MODELS || (!STATS && !SCREEN), "model set: no statistics, no screening");
   static_assert(NF == 1 || NF == 2, "one or two operator warps");
   static_assert(!SCREEN || (LINEAR && !NORM && !STATS), "screening: plain linear policies only");
   constexpr int L = LaneSplit<N>::L, G = LaneSplit<N>::G;
@@ -75,7 +77,7 @@ lane2_rollout_kernel(const RolloutArgs a) {
   const bool active = e0 < a.B;
   const long long e = active ? e0 : a.B - 1;
   const unsigned int iteration = a.iteration + (a.iter_dev ? *a.iter_dev : 0u);
-  const Phys& P = a.real;
+  const Phys& P = rollout_model<MODELS>(a, models);
 
   // ---- initial state (both warps): this lane's pair of the observation ----
   const int jpair = is_seg ? 2 + 2 * seg : 0;
@@ -263,7 +265,7 @@ lane2_rollout_kernel(const RolloutArgs a) {
   if (LINEAR && a.dir_mask) skipped = a.dir_mask[(e / a.R) >> 1] == 0;
   const bool live = active && !skipped;
   if (active && skipped && a.final_state && seg <= N) {
-    double2* o = reinterpret_cast<double2*>(a.final_state + e * NO + jpair);
+    double2* o = reinterpret_cast<double2*>(a.final_state + output_row<MODELS>(a, e) * NO + jpair);
     *o = is_seg ? make_double2(th, thd) : make_double2(gdx, gdy);
   }
   double sgx = 0.0, sgy = 0.0;
@@ -431,10 +433,11 @@ lane2_rollout_kernel(const RolloutArgs a) {
   if (live) {
     if (seg == 0) {
       const double ret = fma(sgx, P.dirx, sgy * P.diry);
-      a.returns[e] = a.accumulate ? a.returns[e] + ret : ret;
+      const long long eo = output_row<MODELS>(a, e);
+      a.returns[eo] = a.accumulate ? a.returns[eo] + ret : ret;
     }
     if (a.final_state && seg <= N) {
-      *reinterpret_cast<double2*>(a.final_state + e * NO + jpair) =
+      *reinterpret_cast<double2*>(a.final_state + output_row<MODELS>(a, e) * NO + jpair) =
           is_seg ? make_double2(th, thd) : make_double2(gdx, gdy);
     }
     if (SCREEN && seg == 0) {
@@ -442,7 +445,7 @@ lane2_rollout_kernel(const RolloutArgs a) {
       if (a.frozen_at) a.frozen_at[e] = frozen;
     }
   } else if (active && seg == 0) {
-    a.returns[e] = __longlong_as_double(0x7ff8000000000000LL);
+    a.returns[output_row<MODELS>(a, e)] = __longlong_as_double(0x7ff8000000000000LL);
     if (SCREEN) {  // masked out: never judged unsafe, no real step taken (as rollout_kernel)
       if (a.violations) a.violations[e] = 0;
       if (a.frozen_at) a.frozen_at[e] = a.H;

@@ -22,6 +22,9 @@ inline bool lane_split_supported(const RolloutArgs& a, const RolloutFlags& f, in
 // f_warps: 0 = one warp per lane group (lane_rollout.cuh); 1 / 2 = the warp-specialised form with that many
 // operator warps beside the main warp (lane2_rollout.cuh)
 template <int N> int launch_lane_rollout_n(const RolloutArgs& a, const RolloutFlags& f, int f_warps, cudaStream_t st);
+// model-set mode (see launch_rollout_models_n): linear policies, V1 / V2 without statistics, no screening
+template <int N> int launch_lane_rollout_models_n(const RolloutArgs& a, const SimModels& models, const RolloutFlags& f,
+                                                  int f_warps, cudaStream_t st);
 
 #ifdef SWM_INSTANTIATE_LANE_N
 
@@ -30,9 +33,10 @@ static int launch_lane_one(const RolloutArgs& a, int f_warps, cudaStream_t st) {
   constexpr int G = LaneSplit<N>::G;
   const long long blocks = (a.B + G - 1) / G;
   if (blocks > 0x7fffffffLL) return SWM_ERR_BAD_ARG;
-  if (f_warps == 2) lane2_rollout_kernel<N, LINEAR, NORM, STATS, 2><<<(unsigned)blocks, 96, 0, st>>>(a);
-  else if (f_warps == 1) lane2_rollout_kernel<N, LINEAR, NORM, STATS, 1><<<(unsigned)blocks, 64, 0, st>>>(a);
-  else lane_rollout_kernel<N, LINEAR, NORM, STATS><<<(unsigned)blocks, kLaneBlock, 0, st>>>(a);
+  const NoCostForms none;
+  if (f_warps == 2) lane2_rollout_kernel<N, LINEAR, NORM, STATS, 2, false, false><<<(unsigned)blocks, 96, 0, st>>>(a, none);
+  else if (f_warps == 1) lane2_rollout_kernel<N, LINEAR, NORM, STATS, 1, false, false><<<(unsigned)blocks, 64, 0, st>>>(a, none);
+  else lane_rollout_kernel<N, LINEAR, NORM, STATS, false><<<(unsigned)blocks, kLaneBlock, 0, st>>>(a, none);
   return cudaPeekAtLastError() == cudaSuccess ? SWM_OK : SWM_ERR_CUDA;
 }
 
@@ -41,8 +45,9 @@ static int launch_lane_screen(const RolloutArgs& a, int f_warps, cudaStream_t st
   constexpr int G = LaneSplit<N>::G;
   const long long blocks = (a.B + G - 1) / G;
   if (blocks > 0x7fffffffLL) return SWM_ERR_BAD_ARG;
-  if (f_warps == 2) lane2_rollout_kernel<N, true, false, false, 2, true><<<(unsigned)blocks, 96, 0, st>>>(a);
-  else lane2_rollout_kernel<N, true, false, false, 1, true><<<(unsigned)blocks, 64, 0, st>>>(a);
+  const NoCostForms none;
+  if (f_warps == 2) lane2_rollout_kernel<N, true, false, false, 2, true, false><<<(unsigned)blocks, 96, 0, st>>>(a, none);
+  else lane2_rollout_kernel<N, true, false, false, 1, true, false><<<(unsigned)blocks, 64, 0, st>>>(a, none);
   return cudaPeekAtLastError() == cudaSuccess ? SWM_OK : SWM_ERR_CUDA;
 }
 
@@ -56,7 +61,29 @@ int launch_lane_rollout_n(const RolloutArgs& a, const RolloutFlags& f, int f_war
   return launch_lane_one<N, true, false, false>(a, f_warps, st);
 }
 
+template <int N, bool NORM>
+static int launch_lane_models_one(const RolloutArgs& a, const SimModels& models, int f_warps, cudaStream_t st) {
+  constexpr int G = LaneSplit<N>::G;
+  const long long blocks = (a.B + G - 1) / G;
+  if (blocks > 0x7fffffffLL) return SWM_ERR_BAD_ARG;
+  const dim3 grid((unsigned)blocks, (unsigned)models.M);
+  if (f_warps == 2) lane2_rollout_kernel<N, true, NORM, false, 2, false, true><<<grid, 96, 0, st>>>(a, models);
+  else if (f_warps == 1) lane2_rollout_kernel<N, true, NORM, false, 1, false, true><<<grid, 64, 0, st>>>(a, models);
+  else lane_rollout_kernel<N, true, NORM, false, true><<<grid, kLaneBlock, 0, st>>>(a, models);
+  return cudaPeekAtLastError() == cudaSuccess ? SWM_OK : SWM_ERR_CUDA;
+}
+
+template <int N>
+int launch_lane_rollout_models_n(const RolloutArgs& a, const SimModels& models, const RolloutFlags& f, int f_warps,
+                                 cudaStream_t st) {
+  if (!lane_split_supported(a, f, f_warps) || !f.linear || f.screen || f.stats) return SWM_ERR_UNSUPPORTED;
+  if (f.norm) return launch_lane_models_one<N, true>(a, models, f_warps, st);
+  return launch_lane_models_one<N, false>(a, models, f_warps, st);
+}
+
 template int launch_lane_rollout_n<SWM_INSTANTIATE_LANE_N>(const RolloutArgs&, const RolloutFlags&, int, cudaStream_t);
+template int launch_lane_rollout_models_n<SWM_INSTANTIATE_LANE_N>(const RolloutArgs&, const SimModels&,
+                                                                  const RolloutFlags&, int, cudaStream_t);
 
 #endif  // SWM_INSTANTIATE_LANE_N
 

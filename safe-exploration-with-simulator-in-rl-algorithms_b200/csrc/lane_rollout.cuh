@@ -99,9 +99,11 @@ __device__ __forceinline__ double group_max_abs(double v) {
   return __longlong_as_double(b);
 }
 
-template <int N, bool LINEAR, bool NORM, bool STATS>
+// MODELS: the model-set mode of rollout_kernel (CTA row blockIdx.y runs model blockIdx.y; no statistics)
+template <int N, bool LINEAR, bool NORM, bool STATS, bool MODELS>
 __global__ void __launch_bounds__(kLaneBlock)
-lane_rollout_kernel(const RolloutArgs a) {
+lane_rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms<SCREEN_NONE, MODELS>::type models) {
+  static_assert(!MODELS || !STATS, "model set: no statistics");
   constexpr int L = LaneSplit<N>::L, G = LaneSplit<N>::G;
   constexpr int NO = 2 * N + 2, NA = N - 1, WS = NA * NO, J = N - 1;
   constexpr unsigned FULL = 0xffffffffu;
@@ -122,7 +124,7 @@ lane_rollout_kernel(const RolloutArgs a) {
   const bool active = e0 < a.B;
   const long long e = active ? e0 : a.B - 1;  // idle groups shadow the last env, never store
   const unsigned int iteration = a.iteration + (a.iter_dev ? *a.iter_dev : 0u);
-  const Phys& P = a.real;
+  const Phys& P = rollout_model<MODELS>(a, models);
 
   // ---- initial state: this lane's pair of the observation, Gdot replicated on every lane ----
   const int jpair = is_seg ? 2 + 2 * seg : 0;  // observation index of this lane's pair (lanes > N: unused)
@@ -213,7 +215,7 @@ lane_rollout_kernel(const RolloutArgs a) {
   if (LINEAR && a.dir_mask) skipped = a.dir_mask[(e / a.R) >> 1] == 0;
   const bool live = active && !skipped;
   if (active && skipped && a.final_state && seg <= N) {
-    double2* o = reinterpret_cast<double2*>(a.final_state + e * NO + jpair);
+    double2* o = reinterpret_cast<double2*>(a.final_state + output_row<MODELS>(a, e) * NO + jpair);
     *o = is_seg ? make_double2(th, thd) : make_double2(gdx, gdy);
   }
 
@@ -419,14 +421,15 @@ lane_rollout_kernel(const RolloutArgs a) {
   if (live) {
     if (seg == 0) {
       const double ret = fma(sgx, P.dirx, sgy * P.diry);
-      a.returns[e] = a.accumulate ? a.returns[e] + ret : ret;
+      const long long eo = output_row<MODELS>(a, e);
+      a.returns[eo] = a.accumulate ? a.returns[eo] + ret : ret;
     }
     if (a.final_state && seg <= N) {
-      *reinterpret_cast<double2*>(a.final_state + e * NO + jpair) =
+      *reinterpret_cast<double2*>(a.final_state + output_row<MODELS>(a, e) * NO + jpair) =
           is_seg ? make_double2(th, thd) : make_double2(gdx, gdy);
     }
   } else if (active && seg == 0) {
-    a.returns[e] = __longlong_as_double(0x7ff8000000000000LL);  // screened out: NaN (see rollout_kernel)
+    a.returns[output_row<MODELS>(a, e)] = __longlong_as_double(0x7ff8000000000000LL);  // screened out: NaN (see rollout_kernel)
   }
 
   if (STATS) {

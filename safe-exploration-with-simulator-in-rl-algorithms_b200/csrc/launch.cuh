@@ -20,6 +20,9 @@ template <int N> int launch_rollout_costed_n(const RolloutArgs& a, const CostFor
                                              cudaStream_t st);
 template <int N> int launch_rollout_ensemble_n(const RolloutArgs& a, const SimModels& models, const CostForms* forms,
                                                const RolloutFlags& f, cudaStream_t st);
+// model-set mode: cfg->B environments for each of models.M models, one CTA row per model (f as for launch_rollout_n)
+template <int N> int launch_rollout_models_n(const RolloutArgs& a, const SimModels& models, const RolloutFlags& f,
+                                             cudaStream_t st);
 template <int N> int launch_step_models_n(const PhysSet& set, long long envs_per_model, const double* state_in,
                                           const double* action, double* out, double* reward, long long B,
                                           cudaStream_t st);
@@ -38,8 +41,10 @@ static size_t rollout_smem() {
   return smem;
 }
 
+// grid_y: CTA rows (the models of the model-set mode, else 1)
 template <typename Kernel, typename... Args>
-static int launch_rollout_grid(Kernel kern, size_t smem, long long B, cudaStream_t st, const Args&... args) {
+static int launch_rollout_grid(Kernel kern, size_t smem, long long B, unsigned grid_y, cudaStream_t st,
+                               const Args&... args) {
   // dynamic + static shared memory (s_mu, s_piv, the moment reduction scratch: < 2 KB) above the default
   // 48 KB limit needs the opt-in attribute
   if (smem + 2048 > 48 * 1024) {
@@ -47,20 +52,20 @@ static int launch_rollout_grid(Kernel kern, size_t smem, long long B, cudaStream
     if (err != cudaSuccess) return SWM_ERR_CUDA;
   }
   const long long blocks = (B + kRolloutBlock - 1) / kRolloutBlock;
-  kern<<<(unsigned)blocks, kRolloutBlock, smem, st>>>(args...);
+  kern<<<dim3((unsigned)blocks, grid_y), kRolloutBlock, smem, st>>>(args...);
   return cudaPeekAtLastError() == cudaSuccess ? SWM_OK : SWM_ERR_CUDA;  // capi.cu note_launch reads + clears it
 }
 
 template <int N, int VARIANT, int WMODE, bool NORM, bool STATS, bool SCREEN>
 static int launch_rollout_one(const RolloutArgs& a, cudaStream_t st) {
-  return launch_rollout_grid(rollout_kernel<N, VARIANT, WMODE, NORM, STATS, SCREEN ? SCREEN_BUILTIN : SCREEN_NONE>,
-                             rollout_smem<N, VARIANT, WMODE, STATS>(), a.B, st, a, NoCostForms{});
+  return launch_rollout_grid(rollout_kernel<N, VARIANT, WMODE, NORM, STATS, SCREEN ? SCREEN_BUILTIN : SCREEN_NONE, false>,
+                             rollout_smem<N, VARIANT, WMODE, STATS>(), a.B, 1, st, a, NoCostForms{});
 }
 
 template <int N, int WMODE>
 static int launch_rollout_costed_one(const RolloutArgs& a, const CostForms& forms, cudaStream_t st) {
-  return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_AFFINE>,
-                             rollout_smem<N, 0, WMODE, false>(), a.B, st, a, forms);
+  return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_AFFINE, false>,
+                             rollout_smem<N, 0, WMODE, false>(), a.B, 1, st, a, forms);
 }
 
 // The costed kernel exists for what per-step screening supports on the thread kernel: gym dynamics, linear
@@ -82,12 +87,13 @@ template <int N, int WMODE>
 static int launch_rollout_ensemble_one(const RolloutArgs& a, const SimModels& models, const CostForms* forms,
                                        cudaStream_t st) {
   const size_t smem = rollout_smem<N, 0, WMODE, false>();
-  if (!forms) return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_ENSEMBLE>, smem, a.B, st,
-                                         a, models);
+  if (!forms) return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_ENSEMBLE, false>, smem, a.B,
+                                         1, st, a, models);
   SimModelsForms mf;
   mf.models = models;
   mf.forms = *forms;
-  return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_ENSEMBLE_AFFINE>, smem, a.B, st, a, mf);
+  return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_ENSEMBLE_AFFINE, false>, smem, a.B, 1, st,
+                             a, mf);
 }
 
 // Same configurations as the costed kernel.
@@ -101,6 +107,30 @@ int launch_rollout_ensemble_n(const RolloutArgs& a, const SimModels& models, con
   } else {
     if (f.group_w) return launch_rollout_ensemble_one<N, W_SMEM_GROUP>(a, models, forms, st);
     return launch_rollout_ensemble_one<N, W_SMEM_THREAD>(a, models, forms, st);
+  }
+}
+
+template <int N, int WMODE>
+static int launch_rollout_models_one(const RolloutArgs& a, const SimModels& models, bool norm, cudaStream_t st) {
+  const size_t smem = rollout_smem<N, 0, WMODE, false>();
+  if (norm)
+    return launch_rollout_grid(rollout_kernel<N, 0, WMODE, true, false, SCREEN_NONE, true>, smem, a.B, models.M, st, a,
+                               models);
+  return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_NONE, true>, smem, a.B, models.M, st, a,
+                             models);
+}
+
+// The model-set kernels exist for the simulator rollouts of ARS screening: gym dynamics, linear policies, V1 or V2
+// without statistics, no per-step screening.
+template <int N>
+int launch_rollout_models_n(const RolloutArgs& a, const SimModels& models, const RolloutFlags& f, cudaStream_t st) {
+  constexpr int WS = (N - 1) * (2 * N + 2);
+  if (f.variant != SWM_DYN_GYM || !f.linear || f.screen || f.stats) return SWM_ERR_UNSUPPORTED;
+  if constexpr (WS <= kRegPolicyMax) {
+    return launch_rollout_models_one<N, W_REG>(a, models, f.norm, st);
+  } else {
+    if (f.group_w) return launch_rollout_models_one<N, W_SMEM_GROUP>(a, models, f.norm, st);
+    return launch_rollout_models_one<N, W_SMEM_THREAD>(a, models, f.norm, st);
   }
 }
 
@@ -167,6 +197,8 @@ template int launch_rollout_costed_n<SWM_INSTANTIATE_N>(const RolloutArgs&, cons
                                                         cudaStream_t);
 template int launch_rollout_ensemble_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const SimModels&, const CostForms*,
                                                           const RolloutFlags&, cudaStream_t);
+template int launch_rollout_models_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const SimModels&, const RolloutFlags&,
+                                                        cudaStream_t);
 
 #endif  // SWM_INSTANTIATE_N
 

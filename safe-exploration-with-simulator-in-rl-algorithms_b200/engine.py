@@ -3,6 +3,8 @@ ARSAgent.runOneIteration (ars/ars_agent.py:132-185) and Basic_ARS.train (safe_ar
 
 One iteration =
   1. [reward-constraint safe mode] 2N simulator rollouts -> screening mask        (swm_rollout, swm_screen_mask)
+     (an ensemble of M simulator models: M x 2N rollouts in one launch, a direction survives only if it
+     clears the threshold under every model                                        (swm_rollout_models, swm_screen_mask_models))
   2. 2N (x R) real rollouts, all in one fused kernel launch                        (swm_rollout)
      (V1 safe mode: 1 and 2 run side by side on two streams, the mask is applied to the returns in step 3 --
      `speculate`; otherwise 2 rolls out the survivors of 1 only)
@@ -97,8 +99,17 @@ class ArsEngine:
         self.mean = torch.zeros(self.no, **f64)
         self.inv_sigma = torch.ones(self.no, **f64)
         self.pivot = ops.reset_state(n, variant, self.device)
-        # reward-constraint screening through a simulator model (ars_agent.py:144-157)
+        # reward-constraint screening through a simulator model (ars_agent.py:144-157), or through every model of a
+        # list: a direction reaches the real world only if both its returns clear sim_threshold under each of them
         self.sim_params, self.sim_threshold = sim_params, sim_threshold
+        n_sim = None
+        if isinstance(sim_params, (list, tuple)):
+            n_sim = len(sim_params)
+            if not 1 <= n_sim <= _lib.MAX_SIM_MODELS or any(p.n != params.n for p in sim_params):
+                raise ValueError("sim_params must be 1 to %d models with the real model's n=%d"
+                                 % (_lib.MAX_SIM_MODELS, params.n))
+            if variant != GYM or clip_actions:
+                raise ValueError("screening by several simulator models needs gym dynamics without action clipping")
         # speculate: the real-world rollouts of ALL directions run beside the simulator rollouts that screen them
         # (second stream; both are small batches that leave most of the chip idle) and the screening mask is
         # applied to their returns afterwards (swm_ars_pack_exchange writes NaN for screened-out directions).
@@ -112,7 +123,8 @@ class ArsEngine:
         Bl = 2 * self.N_local * self.R
         self.B_local = Bl
         self._out = {"returns": torch.empty(Bl, **f64)}
-        self._sim_out = {"returns": torch.empty(Bl, **f64)} if sim_params is not None else None
+        lead = () if n_sim is None else (n_sim,)  # model lists: one row per model
+        self._sim_out = {"returns": torch.empty(lead + (Bl,), **f64)} if sim_params is not None else None
         self.returns = torch.zeros(2 * self.N, **f64)        # last iteration, all ranks
         self._records = torch.zeros(self.world, 1 + 2 * self.no, **f64)
         self.order = torch.zeros(self.N, dtype=torch.int32, device=self.device)
@@ -123,7 +135,7 @@ class ArsEngine:
             self.n_pass_local = torch.zeros(1, dtype=torch.int32, device=self.device)
             self.n_pass_total = torch.zeros(1, dtype=torch.int64, device=self.device)  # survivors so far (this rank)
             self.mask = torch.ones(self.N, dtype=torch.int32, device=self.device)
-            self.sim_returns = torch.zeros(2 * self.N_local, **f64)
+            self.sim_returns = torch.zeros(lead + (2 * self.N_local,), **f64)
         self.last = None
         # per-iteration record exchange (one packed record per rank): peer-memory kernel or collective
         self.layout = RecordLayout(self.N_local, self.no if self.v2 else 0, has_mask=sim_params is not None)
@@ -163,7 +175,8 @@ class ArsEngine:
         if (self._chunked is not None and params is self.params and not want_trajectory and screen is None
                 and want_stats == self.v2):
             return self._chunked.run(dir0=self.dir0, deltas=deltas_local, dir_mask=dir_mask)
-        return ops.rollout(
+        fn = ops.rollout_models if isinstance(params, (list, tuple)) else ops.rollout
+        return fn(
             params, self.H, B=self.B_local, variant=self.variant, base_policy=self.W, nu=self.nu,
             deltas=deltas_local, dir_mask=dir_mask, init_perturb=self.init_perturb, seed=self.seed,
             iteration=0, iteration_dev=self.iter_dev, dir0=self.dir0, delta_dist=self.delta_dist,

@@ -14,7 +14,7 @@ from . import _lib
 from ._lib import (ARS_AGENT, ARS_RLGLUE, ARS_TOPB, DELTA_01, DELTA_PM1, GYM, POLICY_DELTAS,
                    POLICY_EXPLICIT, POLICY_FIXED_ACTION, POLICY_PHILOX, RLGLUE)
 
-__all__ = ["step_batched", "step_batched_models", "accelerations_batched", "rollout", "RolloutResult", "ChunkedRollout", "plan_chunks", "philox_deltas",
+__all__ = ["step_batched", "step_batched_models", "accelerations_batched", "rollout", "rollout_models", "RolloutResult", "ChunkedRollout", "plan_chunks", "philox_deltas",
            "ars_topb", "ars_update", "pack_exchange", "counter_add", "record_nanmean", "stats_finalize", "stats_merge", "reduce_returns", "screen_mask", "policy_actions", "update_args",
            "EstimateData", "prediction_error", "cmaes_default_popsize", "cmaes_state_doubles", "cmaes_view", "cmaes_init",
            "cmaes_sample", "cmaes_update", "cmaes_generation",
@@ -138,7 +138,7 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
             seed=0, iteration=0, iteration_dev=None, dir0=0, delta_dist=DELTA_PM1, rollouts_per_policy=1, mean=None,
             inv_sigma=None, clip_actions=False, init_state=None, want_final=False,
             want_trajectory=False, stats_pivot=None, screen=None, out=None, device=None,
-            accumulate_returns=False, kernel=0, schedule=None):
+            accumulate_returns=False, kernel=0, schedule=None, _models=None):
     """One fused H-step rollout of B environments (swm_rollout).
 
     Exactly one of
@@ -159,6 +159,7 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
     environment) / KERNEL_LANES (one environment over 4/8/16 lanes; small batches).
     schedule: None = the library decides between one plain launch and a chunked schedule (needs want_final;
     swm_rollout_t.schedule_sub); "plain" = always one launch; (n_sub, chunk) = forced.
+    _models: see rollout_models.
     """
     _lib.require_cuda()
     n = params.n
@@ -227,6 +228,7 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
         keep.append(init_state)
     res = RolloutResult()
     out = out or {}
+    lead = () if _models is None else (len(_models),)  # model-set mode: one row of outputs per model
 
     def buf(name, shape, dtype=torch.float64):
         t = out.get(name)
@@ -235,10 +237,10 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
         assert tuple(t.shape) == tuple(shape) and t.is_contiguous()
         return t
 
-    res.returns = buf("returns", (B,))
+    res.returns = buf("returns", lead + (B,))
     cfg.returns = res.returns.data_ptr()
     if want_final:
-        res.final_state = buf("final_state", (B, no))
+        res.final_state = buf("final_state", lead + (B, no))
         cfg.final_state = res.final_state.data_ptr()
     if want_trajectory:
         res.trajectory = buf("trajectory", (H, B, no))
@@ -270,7 +272,10 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
         raise ValueError("the cost is for n=%d segments, the model has n=%d" % (cost.n, n))
     forms = cost.forms if cost is not None else None  # host [J, 2n+3], copied into the launch's arguments
     with torch.cuda.device(dev):
-        if sim_models is not None:
+        if _models is not None:
+            models = (_lib.SwmParams * len(_models))(*_models)  # host copies, copied into the launch's arguments
+            _lib.check(_lib.lib().swm_rollout_models(models, len(_models), ctypes.byref(cfg), _lib.stream_ptr()))
+        elif sim_models is not None:
             models = (_lib.SwmParams * len(sim_models))(*sim_models)  # host copies, copied into the launch's arguments
             _lib.check(_lib.lib().swm_rollout_ensemble(
                 ctypes.byref(params), ctypes.byref(cfg), models, len(sim_models),
@@ -283,6 +288,20 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
                                                      forms.ctypes.data_as(ctypes.c_void_p), forms.shape[0],
                                                      _lib.stream_ptr()))
     return res
+
+
+def rollout_models(params_list, H, **kw):
+    """The rollout of `rollout(params, H, **kw)` under each of 1..MAX_SIM_MODELS models with the same n, in one launch
+    (swm_rollout_models): env e of model m runs exactly what env e of rollout(params_list[m], ...) runs, with
+    model m's physics.  B counts the environments per model; returns is [M, B], final_state [M, B, 2n+2].  For the
+    simulator rollouts of ARS screening: linear policies, V1 or V2 without statistics, no screening, trajectory
+    or clipping (the library refuses them).  kernel: as for rollout, AUTO chosen for M * B environments."""
+    params_list = list(params_list)
+    if not 1 <= len(params_list) <= _lib.MAX_SIM_MODELS:
+        raise ValueError("need 1 to %d models, got %d" % (_lib.MAX_SIM_MODELS, len(params_list)))
+    if any(p.n != params_list[0].n for p in params_list):
+        raise ValueError("every model must have the same number of segments")
+    return rollout(params_list[0], H, _models=params_list, **kw)
 
 
 def plan_chunks(B, unit, n_sub, H, chunk):
@@ -478,15 +497,22 @@ def ars_update(W, returns, N, *, order=None, n_order=None, divisor=0.0, ddof=0, 
 
 def screen_mask(sim_returns, threshold, mask_out=None, n_pass_out=None, n_pass_total=None):
     """mask[k] = r_sim+_k > threshold and r_sim-_k > threshold (ars_agent.py:150-157).  n_pass_total: optional
-    int64 device tensor accumulating the number of survivors over calls."""
-    N = sim_returns.numel() // 2
+    int64 device tensor accumulating the number of survivors over calls.  A 2-D sim_returns [M, 2N] holds the
+    returns under M models (swm_screen_mask_models): a direction passes only if it passes under every model."""
     dev = sim_returns.device
+    M = sim_returns.shape[0] if sim_returns.dim() == 2 else None
+    N = sim_returns.numel() // 2 if M is None else sim_returns.shape[1] // 2
     mask = torch.empty(N, dtype=torch.int32, device=dev) if mask_out is None else mask_out
     n_pass = torch.empty(1, dtype=torch.int32, device=dev) if n_pass_out is None else n_pass_out
     with torch.cuda.device(dev):
-        _lib.check(_lib.lib().swm_screen_mask(_lib.ptr(sim_returns), N, float(threshold),
-                                              _lib.ptr(mask), _lib.ptr(n_pass), _lib.ptr(n_pass_total),
-                                              _lib.stream_ptr()))
+        if M is None:
+            _lib.check(_lib.lib().swm_screen_mask(_lib.ptr(sim_returns), N, float(threshold),
+                                                  _lib.ptr(mask), _lib.ptr(n_pass), _lib.ptr(n_pass_total),
+                                                  _lib.stream_ptr()))
+        else:
+            _lib.check(_lib.lib().swm_screen_mask_models(_lib.ptr(sim_returns), M, N, float(threshold),
+                                                         _lib.ptr(mask), _lib.ptr(n_pass), _lib.ptr(n_pass_total),
+                                                         _lib.stream_ptr()))
     return mask, n_pass
 
 

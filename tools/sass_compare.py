@@ -1,7 +1,9 @@
 """Compares the SASS instruction sequence (cuobjdump -sass, addresses and encodings stripped) of every kernel of OLD
-with the same kernel of NEW; exit status 1 if one is missing or differs.  Kernel names are matched after two
-renamings that do not change code: anonymous namespaces (named from a hash of their translation unit) and
-rollout_kernel's SCREEN argument turning from bool into ScreenMode with a second, empty kernel argument.
+with the same kernel of NEW; exit status 1 if one is missing or differs.  Kernel names are matched after renamings
+that do not change code: anonymous namespaces (named from a hash of their translation unit), rollout_kernel's SCREEN
+argument turning from bool into ScreenMode with a second, empty kernel argument, and the rollout kernels' MODELS
+argument (model-set mode) with, for the lane-split kernels, that same empty second argument.  screen_mask_kernel
+gained a model count M: it is matched to its new name, and its code differs by that loop.
 usage: python tools/sass_compare.py OLD NEW   (objects or shared libraries, e.g. a parent commit's libswimmer_ars.so)"""
 import re, subprocess, sys
 
@@ -24,8 +26,19 @@ def anon(k):
 
 def rename(k):
     # rollout_kernel<..., bool SCREEN>(RolloutArgs) became rollout_kernel<..., int SCREEN>(RolloutArgs, ScreenForms<SCREEN>::type)
-    return re.sub(r"^(_ZN3swm14rollout_kernelI.*)Lb([01])EEEvNS_11RolloutArgsE$",
-                  r"\1Li\2EEEvNS_11RolloutArgsENS_11ScreenFormsIXT4_EE4typeE", k)
+    k = re.sub(r"^(_ZN3swm14rollout_kernelI.*)Lb([01])EEEvNS_11RolloutArgsE$",
+               r"\1Li\2EEEvNS_11RolloutArgsENS_11ScreenFormsIXT4_EE4typeE", k)
+    # ... then rollout_kernel<..., int SCREEN, bool MODELS>(RolloutArgs, ScreenForms<SCREEN, MODELS>::type)
+    k = re.sub(r"^(_ZN3swm14rollout_kernelI.*)EEvNS_11RolloutArgsENS_11ScreenFormsIXT4_EE4typeE$",
+               r"\1Lb0EEEvNS_11RolloutArgsENS_11ScreenFormsIXT4_EXT5_EE4typeE", k)
+    # lane_rollout_kernel<N, LINEAR, NORM, STATS, bool MODELS>(RolloutArgs, ScreenForms<SCREEN_NONE, MODELS>::type)
+    k = re.sub(r"^(_ZN3swm19lane_rollout_kernelI.*)EEvNS_11RolloutArgsE$",
+               r"\1Lb0EEEvNS_11RolloutArgsENS_11ScreenFormsILi0EXT3_EE4typeE", k)
+    # lane2_rollout_kernel<N, LINEAR, NORM, STATS, NF, SCREEN, bool MODELS>(RolloutArgs, ScreenForms<..>::type)
+    k = re.sub(r"^(_ZN3swm20lane2_rollout_kernelI.*)EEvNS_11RolloutArgsE$",
+               r"\1Lb0EEEvNS_11RolloutArgsENS_11ScreenFormsILi0EXT5_EE4typeE", k)
+    # screen_mask_kernel(sim_returns, N, ...) -> screen_mask_kernel(sim_returns, M, N, ...)
+    return k.replace("_ZN3swm18screen_mask_kernelEPKdidPiS2_Px", "_ZN3swm18screen_mask_kernelEPKdiidPiS2_Px")
 
 old = {anon(rename(k)): v for k, v in kernels(sys.argv[1]).items()}
 new = {anon(k): v for k, v in kernels(sys.argv[2]).items()}
