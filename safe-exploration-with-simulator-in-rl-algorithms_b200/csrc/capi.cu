@@ -508,49 +508,36 @@ int check_thread_screen(const swm_rollout_t* cfg, const RolloutFlags& f) {
   return SWM_OK;
 }
 
-}  // namespace
-
-extern "C" int swm_rollout_costed(const swm_params_t* params, const swm_rollout_t* cfg, const double* forms,
-                                  int n_forms, void* stream) {
-  if (!params_ok(params) || !cfg || !cfg->screen.enabled) return SWM_ERR_BAD_ARG;
-  CostForms cf;
-  int rc = read_cost_forms(params->n, forms, n_forms, cf);
-  if (rc != SWM_OK) return rc;
-  RolloutArgs a;
-  RolloutFlags f;
-  rc = build_rollout_args(params, cfg, a, f);
-  if (rc != SWM_OK) return rc;
-  rc = check_thread_screen(cfg, f);
-  if (rc != SWM_OK) return rc;
-  if (cfg->B == 0) return SWM_OK;  // empty batch: nothing to do, pointers may be NULL
-  rc = check_rollout_buffers(cfg, f);
-  if (rc != SWM_OK) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-#define CALL(K) launch_rollout_costed_n<K>(a, cf, f, st)
-  SWM_DISPATCH_N(params->n, CALL)
-#undef CALL
-}
-
-extern "C" int swm_rollout_ensemble(const swm_params_t* params, const swm_rollout_t* cfg,
-                                    const swm_params_t* sim_models, int n_models, const double* forms, int n_forms,
-                                    void* stream) {
-  if (!params_ok(params) || !cfg || !cfg->screen.enabled) return SWM_ERR_BAD_ARG;
-  if (!sim_models || n_models < 1 || n_models > SWM_MAX_SIM_MODELS) return SWM_ERR_BAD_ARG;
-  SimModels sm;
+// Copies and checks a host model list: 1..SWM_MAX_SIM_MODELS valid models with the same segment count.
+int read_sim_models(const swm_params_t* models, int n_models, SimModels& sm) {
+  if (!models || n_models < 1 || n_models > SWM_MAX_SIM_MODELS) return SWM_ERR_BAD_ARG;
   memset(&sm, 0, sizeof(sm));
   sm.M = n_models;
   for (int m = 0; m < n_models; ++m) {
-    if (!params_ok(&sim_models[m]) || sim_models[m].n != params->n) return SWM_ERR_BAD_ARG;
-    sm.p[m] = make_phys(sim_models[m]);
+    if (!params_ok(&models[m]) || models[m].n != models[0].n) return SWM_ERR_BAD_ARG;
+    sm.p[m] = make_phys(models[m]);
+  }
+  return SWM_OK;
+}
+
+// swm_rollout_costed (sim_models == nullptr: the simulator is cfg->screen.sim, the forms are required) and
+// swm_rollout_ensemble (the simulators are sim_models; without forms the built-in cost).
+int rollout_screened(const swm_params_t* params, const swm_rollout_t* cfg, const swm_params_t* sim_models,
+                     int n_models, const double* forms, int n_forms, void* stream) {
+  if (!params_ok(params) || !cfg || !cfg->screen.enabled) return SWM_ERR_BAD_ARG;
+  swm_rollout_t c = *cfg;
+  SimModels sm;
+  if (sim_models) {
+    const int rc = read_sim_models(sim_models, n_models, sm);
+    if (rc != SWM_OK) return rc;
+    if (sim_models[0].n != params->n) return SWM_ERR_BAD_ARG;
+    c.screen.sim = sim_models[0];  // cfg->screen.sim is not read: the kernel takes its models from `sm`
   }
   CostForms cf;
-  if (forms) {
+  if (forms || !sim_models) {
     const int rc = read_cost_forms(params->n, forms, n_forms, cf);
     if (rc != SWM_OK) return rc;
   }
-  // cfg->screen.sim is not read: the kernel takes its models from `sm`
-  swm_rollout_t c = *cfg;
-  c.screen.sim = sim_models[0];
   RolloutArgs a;
   RolloutFlags f;
   int rc = build_rollout_args(params, &c, a, f);
@@ -561,23 +548,33 @@ extern "C" int swm_rollout_ensemble(const swm_params_t* params, const swm_rollou
   rc = check_rollout_buffers(&c, f);
   if (rc != SWM_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-#define CALL(K) launch_rollout_ensemble_n<K>(a, sm, forms ? &cf : nullptr, f, st)
+#define CALL(K) launch_rollout_screened_n<K>(a, sim_models ? &sm : nullptr, forms ? &cf : nullptr, f, st)
   SWM_DISPATCH_N(params->n, CALL)
 #undef CALL
 }
 
+}  // namespace
+
+extern "C" int swm_rollout_costed(const swm_params_t* params, const swm_rollout_t* cfg, const double* forms,
+                                  int n_forms, void* stream) {
+  return rollout_screened(params, cfg, nullptr, 0, forms, n_forms, stream);
+}
+
+extern "C" int swm_rollout_ensemble(const swm_params_t* params, const swm_rollout_t* cfg,
+                                    const swm_params_t* sim_models, int n_models, const double* forms, int n_forms,
+                                    void* stream) {
+  if (!sim_models) return SWM_ERR_BAD_ARG;
+  return rollout_screened(params, cfg, sim_models, n_models, forms, n_forms, stream);
+}
+
 extern "C" int swm_rollout_models(const swm_params_t* models, int n_models, const swm_rollout_t* cfg, void* stream) {
-  if (!models || n_models < 1 || n_models > SWM_MAX_SIM_MODELS || !cfg) return SWM_ERR_BAD_ARG;
   SimModels sm;
-  memset(&sm, 0, sizeof(sm));
-  sm.M = n_models;
-  for (int m = 0; m < n_models; ++m) {
-    if (!params_ok(&models[m]) || models[m].n != models[0].n) return SWM_ERR_BAD_ARG;
-    sm.p[m] = make_phys(models[m]);
-  }
+  int rc = read_sim_models(models, n_models, sm);
+  if (rc != SWM_OK) return rc;
+  if (!cfg) return SWM_ERR_BAD_ARG;
   RolloutArgs a;
   RolloutFlags f;
-  int rc = build_rollout_args(&models[0], cfg, a, f);
+  rc = build_rollout_args(&models[0], cfg, a, f);
   if (rc != SWM_OK) return rc;
   // what the model-set kernels implement: the simulator rollouts of ARS screening (V1 / V2 without moments)
   if (cfg->variant != SWM_DYN_GYM || !f.linear || f.screen || f.stats || cfg->trajectory || cfg->clip_actions ||

@@ -2,7 +2,8 @@
 // One thread owns one environment; the state (2n+2 doubles), its sines/cosines and (for
 // n <= 5) the environment's own perturbed policy live in registers for the whole rollout.
 // Nothing but the final return (8 B/env), optional final state and optional trajectory is
-// written to HBM.
+// written to HBM.  Per-step screening (every ScreenMode) is one block of the step loop with one
+// freeze path, and the real observation is formed once for the affine cost and the moments.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -247,6 +248,8 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
   static_assert(!MODELS || (SCREEN == SCREEN_NONE && VARIANT == 0 && !STATS), "model set: unscreened gym rollouts");
   constexpr int NO = 2 * N + 2, NA = N - 1, WS = NA * NO;
   constexpr bool LINEAR = (WMODE != W_NONE);
+  constexpr bool ENSEMBLE = SCREEN == SCREEN_ENSEMBLE || SCREEN == SCREEN_ENSEMBLE_AFFINE;
+  constexpr bool AFFINE = SCREEN == SCREEN_AFFINE || SCREEN == SCREEN_ENSEMBLE_AFFINE;
   const Phys& P = rollout_model<MODELS>(a, forms);
   extern __shared__ __align__(16) double smem[];
   const int tid = threadIdx.x;
@@ -445,97 +448,88 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
         if (VARIANT == 0) ut[k] = v * P.u_scale;
       }
     }
-    if (SCREEN == SCREEN_BUILTIN || SCREEN == SCREEN_AFFINE) {
+    if constexpr (SCREEN != SCREEN_NONE) {
       // Safe_ARS.isSafe (safe_ars/ars.py:111-122): one simulator step from the current state.  The
       // simulator starts from the same angles, so it shares this step's sines/cosines and needs only
       // its own accelerations.
-      double sut[NA > 0 ? NA : 1], sgddx, sgddy, sthdd[N];
-#pragma unroll
-      for (int k = 0; k < NA; ++k) sut[k] = u[k] * a.sim.u_scale;
-      gym_accel<N, FS>(a.sim, sn, cs, gdx, gdy, thd, sut, sgddx, sgddy, sthdd, sF);
-      double sim_cost;
-      if constexpr (SCREEN == SCREEN_AFFINE) {
-        // the whole simulated observation, explicit Euler as in gym_step_tracked.  Held in 2n+2 registers for
-        // n = 7 and formed per use otherwise: either way round, ptxas spills (8 B at n = 6, 36-56 B at n = 7).
-        double sob[N == 7 ? NO : 1];
-        auto sim_obs = [&](int k) {
-          if (k < 2) return fma(a.sim.h_gdd_c, k == 0 ? sgddx : sgddy, k == 0 ? gdx : gdy);
-          const int i = (k - 2) / 2;
-          return (k & 1) ? fma(a.sim.h, sthdd[i], thd[i]) : fma(a.sim.h, thd[i], th[i]);
-        };
-        if constexpr (N == 7) {
-#pragma unroll
-          for (int k = 0; k < NO; ++k) sob[k] = sim_obs(k);
-        }
-        auto so = [&](int k) { return N == 7 ? sob[k] : sim_obs(k); };
-        sim_cost = cost_max_affine<NO>(forms, so);
-      } else {
-        // the built-in cost only looks at the new angular velocities
-        double sthd[N];
-#pragma unroll
-        for (int i = 0; i < N; ++i) sthd[i] = fma(a.sim.h, sthdd[i], thd[i]);
-        sim_cost = cost_max_abs_thd<N>(sthd);
-      }
-      if (!(sim_cost <= a.sim_thresh)) {
-        // unsafe: nothing advances, and since obs and policy never change it never will again
-        // (safe_ars/ars.py:151-152) -- the remaining H-t steps are this state repeated.
-        frozen = t;
-        if (traj && active) {
-          for (int tt = t; tt < a.H; ++tt) {
-            double* o = traj + (long long)tt * traj_step;
-            o[0] = gdx; o[1] = gdy;
-#pragma unroll
-            for (int i = 0; i < N; ++i) { o[2 + 2 * i] = th[i]; o[3 + 2 * i] = thd[i]; }
-          }
-        }
-        break;
-      }
-    }
-    if constexpr (SCREEN == SCREEN_ENSEMBLE || SCREEN == SCREEN_ENSEMBLE_AFFINE) {
-      // The block above once per simulator model (written out separately so that the single-model kernels keep
-      // their code): every model must judge the step safe.  The decisions are OR-ed (not the costs maxed), so that
-      // the order of the models cannot matter.  No early exit: a safe step needs all M evaluations, and an unsafe one
-      // ends the rollout.  Models 1..M-1 run in a loop, reading their constants from the constant bank through the
-      // runtime index m; model 0 runs last, in straight-line code directly before the real step, as in the
-      // single-model kernels.  That keeps one model bit-identical to them: there the compiler shares the
-      // model-independent products of the simulator's accelerations (of the sines, cosines and velocities) with the
-      // real step, which then keeps them as separately rounded multiplies; without the shared copy the real step
-      // fuses one of them into an FMA instead (one ulp in the real trajectory).  The loop works on opaque copies of
-      // the sines, cosines and velocities, so that none of its products is hoisted and shared with the code after
-      // it (which would keep them live across the loop).
-      const SimModels& sm = sim_models_of(forms);
-      auto model_unsafe = [&](const Phys& P, const double (&s)[N], const double (&c)[N],
-                              const double (&w)[N]) -> bool {
+      bool unsafe = false;
+      if constexpr (!ENSEMBLE) {
         double sut[NA > 0 ? NA : 1], sgddx, sgddy, sthdd[N];
 #pragma unroll
-        for (int k = 0; k < NA; ++k) sut[k] = u[k] * P.u_scale;
-        gym_accel<N, FS>(P, s, c, gdx, gdy, w, sut, sgddx, sgddy, sthdd, sF);
+        for (int k = 0; k < NA; ++k) sut[k] = u[k] * a.sim.u_scale;
+        gym_accel<N, FS>(a.sim, sn, cs, gdx, gdy, thd, sut, sgddx, sgddy, sthdd, sF);
         double sim_cost;
-        if constexpr (SCREEN == SCREEN_ENSEMBLE_AFFINE) {
-          auto so = [&](int k) {
-            if (k < 2) return fma(P.h_gdd_c, k == 0 ? sgddx : sgddy, k == 0 ? gdx : gdy);
+        if constexpr (AFFINE) {
+          // the whole simulated observation, explicit Euler as in gym_step_tracked.  Held in 2n+2 registers for
+          // n = 7 and formed per use otherwise: either way round, ptxas spills (8 B at n = 6, 36-56 B at n = 7).
+          double sob[N == 7 ? NO : 1];
+          auto sim_obs = [&](int k) {
+            if (k < 2) return fma(a.sim.h_gdd_c, k == 0 ? sgddx : sgddy, k == 0 ? gdx : gdy);
             const int i = (k - 2) / 2;
-            return (k & 1) ? fma(P.h, sthdd[i], w[i]) : fma(P.h, w[i], th[i]);
+            return (k & 1) ? fma(a.sim.h, sthdd[i], thd[i]) : fma(a.sim.h, thd[i], th[i]);
           };
-          sim_cost = cost_max_affine<NO>(cost_forms_of(forms), so);
+          if constexpr (N == 7) {
+#pragma unroll
+            for (int k = 0; k < NO; ++k) sob[k] = sim_obs(k);
+          }
+          auto so = [&](int k) { return N == 7 ? sob[k] : sim_obs(k); };
+          sim_cost = cost_max_affine<NO>(forms, so);
         } else {
+          // the built-in cost only looks at the new angular velocities
           double sthd[N];
 #pragma unroll
-          for (int i = 0; i < N; ++i) sthd[i] = fma(P.h, sthdd[i], w[i]);
+          for (int i = 0; i < N; ++i) sthd[i] = fma(a.sim.h, sthdd[i], thd[i]);
           sim_cost = cost_max_abs_thd<N>(sthd);
         }
-        return !(sim_cost <= a.sim_thresh);
-      };
-      bool unsafe = false;
-#pragma unroll 1
-      for (int m = 1; m < sm.M; ++m) {
-        double s[N], c[N], w[N];
+        unsafe = !(sim_cost <= a.sim_thresh);
+      } else {
+        // The judgement above once per simulator model: every model must judge the step safe.  The decisions are
+        // OR-ed (not the costs maxed), so that the order of the models cannot matter.  No early exit: a safe step
+        // needs all M evaluations, and an unsafe one ends the rollout.  Models 1..M-1 run in a loop, reading their
+        // constants from the constant bank through the runtime index m; model 0 runs last, in straight-line code
+        // directly before the real step, as in the single-model kernels.  That keeps one model bit-identical to
+        // them: there the compiler shares the model-independent products of the simulator's accelerations (of the
+        // sines, cosines and velocities) with the real step, which then keeps them as separately rounded multiplies;
+        // without the shared copy the real step fuses one of them into an FMA instead (one ulp in the real
+        // trajectory).  The loop works on opaque copies of the sines, cosines and velocities, so that none of its
+        // products is hoisted and shared with the code after it (which would keep them live across the loop).
+        // The single-model modes keep the judgement inline: called through model_unsafe their kernels compile to the
+        // same instructions and spills but other registers and another order.
+        const SimModels& sm = sim_models_of(forms);
+        auto model_unsafe = [&](const Phys& P, const double (&s)[N], const double (&c)[N],
+                                const double (&w)[N]) -> bool {
+          double sut[NA > 0 ? NA : 1], sgddx, sgddy, sthdd[N];
 #pragma unroll
-        for (int i = 0; i < N; ++i) { s[i] = opaque(sn[i]); c[i] = opaque(cs[i]); w[i] = opaque(thd[i]); }
-        unsafe |= model_unsafe(sm.p[m], s, c, w);
+          for (int k = 0; k < NA; ++k) sut[k] = u[k] * P.u_scale;
+          gym_accel<N, FS>(P, s, c, gdx, gdy, w, sut, sgddx, sgddy, sthdd, sF);
+          double sim_cost;
+          if constexpr (AFFINE) {
+            auto so = [&](int k) {
+              if (k < 2) return fma(P.h_gdd_c, k == 0 ? sgddx : sgddy, k == 0 ? gdx : gdy);
+              const int i = (k - 2) / 2;
+              return (k & 1) ? fma(P.h, sthdd[i], w[i]) : fma(P.h, w[i], th[i]);
+            };
+            sim_cost = cost_max_affine<NO>(cost_forms_of(forms), so);
+          } else {
+            double sthd[N];
+#pragma unroll
+            for (int i = 0; i < N; ++i) sthd[i] = fma(P.h, sthdd[i], w[i]);
+            sim_cost = cost_max_abs_thd<N>(sthd);
+          }
+          return !(sim_cost <= a.sim_thresh);
+        };
+#pragma unroll 1
+        for (int m = 1; m < sm.M; ++m) {
+          double s[N], c[N], w[N];
+#pragma unroll
+          for (int i = 0; i < N; ++i) { s[i] = opaque(sn[i]); c[i] = opaque(cs[i]); w[i] = opaque(thd[i]); }
+          unsafe |= model_unsafe(sm.p[m], s, c, w);
+        }
+        unsafe |= model_unsafe(sm.p[0], sn, cs, thd);
       }
-      unsafe |= model_unsafe(sm.p[0], sn, cs, thd);
       if (unsafe) {
+        // unsafe: nothing advances, and since obs and policy never change it never will again
+        // (safe_ars/ars.py:151-152) -- the remaining H-t steps are this state repeated.
         frozen = t;
         if (traj && active) {
           for (int tt = t; tt < a.H; ++tt) {
@@ -559,27 +553,24 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
     }
     if (SCREEN == SCREEN_BUILTIN || SCREEN == SCREEN_ENSEMBLE)
       viol += (cost_max_abs_thd<N>(thd) > a.real_thresh) ? 1 : 0;
-    if constexpr (SCREEN == SCREEN_AFFINE || SCREEN == SCREEN_ENSEMBLE_AFFINE) {
-      double x[NO];
+    if constexpr (AFFINE || STATS) {
+      double x[NO];  // the real observation after the step
       x[0] = gdx; x[1] = gdy;
 #pragma unroll
       for (int i = 0; i < N; ++i) { x[2 + 2 * i] = th[i]; x[3 + 2 * i] = thd[i]; }
-      viol += (cost_max_affine<NO>(cost_forms_of(forms), [&](int k) { return x[k]; }) > a.real_thresh) ? 1 : 0;
-    }
-    if (STATS) {
-      double x[NO];
-      x[0] = gdx; x[1] = gdy;
+      if constexpr (AFFINE)
+        viol += (cost_max_affine<NO>(cost_forms_of(forms), [&](int k) { return x[k]; }) > a.real_thresh) ? 1 : 0;
+      if constexpr (STATS) {
 #pragma unroll
-      for (int i = 0; i < N; ++i) { x[2 + 2 * i] = th[i]; x[3 + 2 * i] = thd[i]; }
-#pragma unroll
-      for (int j = 0; j < NO; ++j) {
-        const double d = x[j] - s_piv[j];
-        if (STATS_SMEM) {
-          sS[j * kRolloutBlock] += d;
-          sS[(NO + j) * kRolloutBlock] = fma(d, d, sS[(NO + j) * kRolloutBlock]);
-        } else {
-          s1[j] += d;
-          s2[j] = fma(d, d, s2[j]);
+        for (int j = 0; j < NO; ++j) {
+          const double d = x[j] - s_piv[j];
+          if (STATS_SMEM) {
+            sS[j * kRolloutBlock] += d;
+            sS[(NO + j) * kRolloutBlock] = fma(d, d, sS[(NO + j) * kRolloutBlock]);
+          } else {
+            s1[j] += d;
+            s2[j] = fma(d, d, s2[j]);
+          }
         }
       }
     }

@@ -28,57 +28,37 @@ template <int N> int launch_lane_rollout_models_n(const RolloutArgs& a, const Si
 
 #ifdef SWM_INSTANTIATE_LANE_N
 
-template <int N, bool LINEAR, bool NORM, bool STATS>
-static int launch_lane_one(const RolloutArgs& a, int f_warps, cudaStream_t st) {
+// One launch of the lane-split kernel of f_warps (the warp-specialised form whenever SCREEN) with the second kernel
+// argument `second` (the models of the model-set mode, else empty) and grid_y CTA rows.
+template <int N, bool LINEAR, bool NORM, bool STATS, bool SCREEN, bool MODELS, typename Second>
+static int launch_lane(const RolloutArgs& a, const Second& second, unsigned grid_y, int f_warps, cudaStream_t st) {
   constexpr int G = LaneSplit<N>::G;
   const long long blocks = (a.B + G - 1) / G;
   if (blocks > 0x7fffffffLL) return SWM_ERR_BAD_ARG;
-  const NoCostForms none;
-  if (f_warps == 2) lane2_rollout_kernel<N, LINEAR, NORM, STATS, 2, false, false><<<(unsigned)blocks, 96, 0, st>>>(a, none);
-  else if (f_warps == 1) lane2_rollout_kernel<N, LINEAR, NORM, STATS, 1, false, false><<<(unsigned)blocks, 64, 0, st>>>(a, none);
-  else lane_rollout_kernel<N, LINEAR, NORM, STATS, false><<<(unsigned)blocks, kLaneBlock, 0, st>>>(a, none);
-  return cudaPeekAtLastError() == cudaSuccess ? SWM_OK : SWM_ERR_CUDA;
-}
-
-template <int N>
-static int launch_lane_screen(const RolloutArgs& a, int f_warps, cudaStream_t st) {
-  constexpr int G = LaneSplit<N>::G;
-  const long long blocks = (a.B + G - 1) / G;
-  if (blocks > 0x7fffffffLL) return SWM_ERR_BAD_ARG;
-  const NoCostForms none;
-  if (f_warps == 2) lane2_rollout_kernel<N, true, false, false, 2, true, false><<<(unsigned)blocks, 96, 0, st>>>(a, none);
-  else lane2_rollout_kernel<N, true, false, false, 1, true, false><<<(unsigned)blocks, 64, 0, st>>>(a, none);
+  const dim3 grid((unsigned)blocks, grid_y);
+  if (f_warps == 2) lane2_rollout_kernel<N, LINEAR, NORM, STATS, 2, SCREEN, MODELS><<<grid, 96, 0, st>>>(a, second);
+  else if (f_warps == 1 || SCREEN) lane2_rollout_kernel<N, LINEAR, NORM, STATS, 1, SCREEN, MODELS><<<grid, 64, 0, st>>>(a, second);
+  else lane_rollout_kernel<N, LINEAR, NORM, STATS, MODELS><<<grid, kLaneBlock, 0, st>>>(a, second);
   return cudaPeekAtLastError() == cudaSuccess ? SWM_OK : SWM_ERR_CUDA;
 }
 
 template <int N>
 int launch_lane_rollout_n(const RolloutArgs& a, const RolloutFlags& f, int f_warps, cudaStream_t st) {
   if (!lane_split_supported(a, f, f_warps)) return SWM_ERR_UNSUPPORTED;
-  if (f.screen) return launch_lane_screen<N>(a, f_warps, st);
-  if (!f.linear) return launch_lane_one<N, false, false, false>(a, f_warps, st);
-  if (f.norm && f.stats) return launch_lane_one<N, true, true, true>(a, f_warps, st);
-  if (f.norm) return launch_lane_one<N, true, true, false>(a, f_warps, st);
-  return launch_lane_one<N, true, false, false>(a, f_warps, st);
-}
-
-template <int N, bool NORM>
-static int launch_lane_models_one(const RolloutArgs& a, const SimModels& models, int f_warps, cudaStream_t st) {
-  constexpr int G = LaneSplit<N>::G;
-  const long long blocks = (a.B + G - 1) / G;
-  if (blocks > 0x7fffffffLL) return SWM_ERR_BAD_ARG;
-  const dim3 grid((unsigned)blocks, (unsigned)models.M);
-  if (f_warps == 2) lane2_rollout_kernel<N, true, NORM, false, 2, false, true><<<grid, 96, 0, st>>>(a, models);
-  else if (f_warps == 1) lane2_rollout_kernel<N, true, NORM, false, 1, false, true><<<grid, 64, 0, st>>>(a, models);
-  else lane_rollout_kernel<N, true, NORM, false, true><<<grid, kLaneBlock, 0, st>>>(a, models);
-  return cudaPeekAtLastError() == cudaSuccess ? SWM_OK : SWM_ERR_CUDA;
+  const NoCostForms none;
+  if (f.screen) return launch_lane<N, true, false, false, true, false>(a, none, 1, f_warps, st);
+  if (!f.linear) return launch_lane<N, false, false, false, false, false>(a, none, 1, f_warps, st);
+  if (f.norm && f.stats) return launch_lane<N, true, true, true, false, false>(a, none, 1, f_warps, st);
+  if (f.norm) return launch_lane<N, true, true, false, false, false>(a, none, 1, f_warps, st);
+  return launch_lane<N, true, false, false, false, false>(a, none, 1, f_warps, st);
 }
 
 template <int N>
 int launch_lane_rollout_models_n(const RolloutArgs& a, const SimModels& models, const RolloutFlags& f, int f_warps,
                                  cudaStream_t st) {
   if (!lane_split_supported(a, f, f_warps) || !f.linear || f.screen || f.stats) return SWM_ERR_UNSUPPORTED;
-  if (f.norm) return launch_lane_models_one<N, true>(a, models, f_warps, st);
-  return launch_lane_models_one<N, false>(a, models, f_warps, st);
+  if (f.norm) return launch_lane<N, true, true, false, false, true>(a, models, models.M, f_warps, st);
+  return launch_lane<N, true, false, false, false, true>(a, models, models.M, f_warps, st);
 }
 
 template int launch_lane_rollout_n<SWM_INSTANTIATE_LANE_N>(const RolloutArgs&, const RolloutFlags&, int, cudaStream_t);

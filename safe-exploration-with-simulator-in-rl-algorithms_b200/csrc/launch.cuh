@@ -1,6 +1,11 @@
 // Host-side template dispatch for one segment count N.  Each rollout_nK.cu translation unit
-// instantiates launch_*_n<K> so the (N x mode) kernel matrix compiles in parallel.
+// instantiates launch_*_n<K> so the (N x mode) kernel matrix compiles in parallel.  Three rollout
+// families: plain (swm_rollout, with the built-in screen), screened with cost forms and / or an
+// ensemble (swm_rollout_costed / swm_rollout_ensemble) and the model set (swm_rollout_models); all
+// take the policy storage from with_policy_storage.
 #pragma once
+#include <type_traits>
+
 #include "kernels.cuh"
 
 namespace swm {
@@ -16,9 +21,9 @@ template <int N> int launch_step_n(const Phys& P, int variant, bool acc_only, co
                                    const double* action, double* out, double* reward, long long B,
                                    cudaStream_t st);
 template <int N> int launch_rollout_n(const RolloutArgs& a, const RolloutFlags& f, cudaStream_t st);
-template <int N> int launch_rollout_costed_n(const RolloutArgs& a, const CostForms& forms, const RolloutFlags& f,
-                                             cudaStream_t st);
-template <int N> int launch_rollout_ensemble_n(const RolloutArgs& a, const SimModels& models, const CostForms* forms,
+// per-step screening with cost forms and / or an ensemble of simulator models: SCREEN_AFFINE without models (forms
+// required), else SCREEN_ENSEMBLE (no forms: the built-in cost) or SCREEN_ENSEMBLE_AFFINE
+template <int N> int launch_rollout_screened_n(const RolloutArgs& a, const SimModels* models, const CostForms* forms,
                                                const RolloutFlags& f, cudaStream_t st);
 // model-set mode: cfg->B environments for each of models.M models, one CTA row per model (f as for launch_rollout_n)
 template <int N> int launch_rollout_models_n(const RolloutArgs& a, const SimModels& models, const RolloutFlags& f,
@@ -56,82 +61,61 @@ static int launch_rollout_grid(Kernel kern, size_t smem, long long B, unsigned g
   return cudaPeekAtLastError() == cudaSuccess ? SWM_OK : SWM_ERR_CUDA;  // capi.cu note_launch reads + clears it
 }
 
+// Where a linear policy lives: registers up to kRegPolicyMax doubles, else shared memory, one copy per warp when
+// the warp's rollouts share one policy (group_w).  Calls launch(std::integral_constant<int, WMODE>).
+template <int N, typename Launch>
+static int with_policy_storage(bool group_w, Launch&& launch) {
+  if constexpr ((N - 1) * (2 * N + 2) <= kRegPolicyMax) {
+    return launch(std::integral_constant<int, W_REG>{});
+  } else {
+    if (group_w) return launch(std::integral_constant<int, W_SMEM_GROUP>{});
+    return launch(std::integral_constant<int, W_SMEM_THREAD>{});
+  }
+}
+
 template <int N, int VARIANT, int WMODE, bool NORM, bool STATS, bool SCREEN>
 static int launch_rollout_one(const RolloutArgs& a, cudaStream_t st) {
   return launch_rollout_grid(rollout_kernel<N, VARIANT, WMODE, NORM, STATS, SCREEN ? SCREEN_BUILTIN : SCREEN_NONE, false>,
                              rollout_smem<N, VARIANT, WMODE, STATS>(), a.B, 1, st, a, NoCostForms{});
 }
 
-template <int N, int WMODE>
-static int launch_rollout_costed_one(const RolloutArgs& a, const CostForms& forms, cudaStream_t st) {
-  return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_AFFINE, false>,
-                             rollout_smem<N, 0, WMODE, false>(), a.B, 1, st, a, forms);
-}
-
-// The costed kernel exists for what per-step screening supports on the thread kernel: gym dynamics, linear
-// policies, ARS V1 without statistics.
+// The screened kernels with cost forms or models exist for what per-step screening supports on the thread kernel:
+// gym dynamics, linear policies, ARS V1 without statistics.
 template <int N>
-int launch_rollout_costed_n(const RolloutArgs& a, const CostForms& forms, const RolloutFlags& f, cudaStream_t st) {
-  constexpr int WS = (N - 1) * (2 * N + 2);
-  if (f.variant != SWM_DYN_GYM || !f.linear || !f.screen || f.norm || f.stats) return SWM_ERR_UNSUPPORTED;
-  if constexpr (WS <= kRegPolicyMax) {
-    return launch_rollout_costed_one<N, W_REG>(a, forms, st);
-  } else {
-    if (f.group_w) return launch_rollout_costed_one<N, W_SMEM_GROUP>(a, forms, st);
-    return launch_rollout_costed_one<N, W_SMEM_THREAD>(a, forms, st);
-  }
-}
-
-// Ensemble screening: SCREEN_ENSEMBLE with the built-in cost (forms == nullptr), else SCREEN_ENSEMBLE_AFFINE.
-template <int N, int WMODE>
-static int launch_rollout_ensemble_one(const RolloutArgs& a, const SimModels& models, const CostForms* forms,
-                                       cudaStream_t st) {
-  const size_t smem = rollout_smem<N, 0, WMODE, false>();
-  if (!forms) return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_ENSEMBLE, false>, smem, a.B,
-                                         1, st, a, models);
-  SimModelsForms mf;
-  mf.models = models;
-  mf.forms = *forms;
-  return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_ENSEMBLE_AFFINE, false>, smem, a.B, 1, st,
-                             a, mf);
-}
-
-// Same configurations as the costed kernel.
-template <int N>
-int launch_rollout_ensemble_n(const RolloutArgs& a, const SimModels& models, const CostForms* forms,
+int launch_rollout_screened_n(const RolloutArgs& a, const SimModels* models, const CostForms* forms,
                               const RolloutFlags& f, cudaStream_t st) {
-  constexpr int WS = (N - 1) * (2 * N + 2);
   if (f.variant != SWM_DYN_GYM || !f.linear || !f.screen || f.norm || f.stats) return SWM_ERR_UNSUPPORTED;
-  if constexpr (WS <= kRegPolicyMax) {
-    return launch_rollout_ensemble_one<N, W_REG>(a, models, forms, st);
-  } else {
-    if (f.group_w) return launch_rollout_ensemble_one<N, W_SMEM_GROUP>(a, models, forms, st);
-    return launch_rollout_ensemble_one<N, W_SMEM_THREAD>(a, models, forms, st);
-  }
-}
-
-template <int N, int WMODE>
-static int launch_rollout_models_one(const RolloutArgs& a, const SimModels& models, bool norm, cudaStream_t st) {
-  const size_t smem = rollout_smem<N, 0, WMODE, false>();
-  if (norm)
-    return launch_rollout_grid(rollout_kernel<N, 0, WMODE, true, false, SCREEN_NONE, true>, smem, a.B, models.M, st, a,
-                               models);
-  return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_NONE, true>, smem, a.B, models.M, st, a,
-                             models);
+  return with_policy_storage<N>(f.group_w, [&](auto w) {
+    constexpr int WMODE = decltype(w)::value;
+    const size_t smem = rollout_smem<N, 0, WMODE, false>();
+    if (!models)
+      return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_AFFINE, false>, smem, a.B, 1, st, a,
+                                 *forms);
+    if (!forms)
+      return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_ENSEMBLE, false>, smem, a.B, 1, st, a,
+                                 *models);
+    SimModelsForms mf;
+    mf.models = *models;
+    mf.forms = *forms;
+    return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_ENSEMBLE_AFFINE, false>, smem, a.B, 1,
+                               st, a, mf);
+  });
 }
 
 // The model-set kernels exist for the simulator rollouts of ARS screening: gym dynamics, linear policies, V1 or V2
 // without statistics, no per-step screening.
 template <int N>
 int launch_rollout_models_n(const RolloutArgs& a, const SimModels& models, const RolloutFlags& f, cudaStream_t st) {
-  constexpr int WS = (N - 1) * (2 * N + 2);
   if (f.variant != SWM_DYN_GYM || !f.linear || f.screen || f.stats) return SWM_ERR_UNSUPPORTED;
-  if constexpr (WS <= kRegPolicyMax) {
-    return launch_rollout_models_one<N, W_REG>(a, models, f.norm, st);
-  } else {
-    if (f.group_w) return launch_rollout_models_one<N, W_SMEM_GROUP>(a, models, f.norm, st);
-    return launch_rollout_models_one<N, W_SMEM_THREAD>(a, models, f.norm, st);
-  }
+  return with_policy_storage<N>(f.group_w, [&](auto w) {
+    constexpr int WMODE = decltype(w)::value;
+    const size_t smem = rollout_smem<N, 0, WMODE, false>();
+    if (f.norm)
+      return launch_rollout_grid(rollout_kernel<N, 0, WMODE, true, false, SCREEN_NONE, true>, smem, a.B, models.M, st,
+                                 a, models);
+    return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_NONE, true>, smem, a.B, models.M, st, a,
+                               models);
+  });
 }
 
 template <int N, int WMODE>
@@ -152,18 +136,12 @@ static int launch_rollout_linear(const RolloutArgs& a, const RolloutFlags& f, cu
 
 template <int N>
 int launch_rollout_n(const RolloutArgs& a, const RolloutFlags& f, cudaStream_t st) {
-  constexpr int WS = (N - 1) * (2 * N + 2);
   if (!f.linear) {
     if (f.norm || f.stats || f.screen) return SWM_ERR_UNSUPPORTED;
     return f.variant == SWM_DYN_GYM ? launch_rollout_one<N, 0, W_NONE, false, false, false>(a, st)
                                     : launch_rollout_one<N, 1, W_NONE, false, false, false>(a, st);
   }
-  if constexpr (WS <= kRegPolicyMax) {
-    return launch_rollout_linear<N, W_REG>(a, f, st);
-  } else {
-    if (f.group_w) return launch_rollout_linear<N, W_SMEM_GROUP>(a, f, st);
-    return launch_rollout_linear<N, W_SMEM_THREAD>(a, f, st);
-  }
+  return with_policy_storage<N>(f.group_w, [&](auto w) { return launch_rollout_linear<N, decltype(w)::value>(a, f, st); });
 }
 
 template <int N>
@@ -193,9 +171,7 @@ template int launch_step_models_n<SWM_INSTANTIATE_N>(const PhysSet&, long long, 
 template int launch_step_n<SWM_INSTANTIATE_N>(const Phys&, int, bool, const double*, const double*,
                                               double*, double*, long long, cudaStream_t);
 template int launch_rollout_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const RolloutFlags&, cudaStream_t);
-template int launch_rollout_costed_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const CostForms&, const RolloutFlags&,
-                                                        cudaStream_t);
-template int launch_rollout_ensemble_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const SimModels&, const CostForms*,
+template int launch_rollout_screened_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const SimModels*, const CostForms*,
                                                           const RolloutFlags&, cudaStream_t);
 template int launch_rollout_models_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const SimModels&, const RolloutFlags&,
                                                         cudaStream_t);

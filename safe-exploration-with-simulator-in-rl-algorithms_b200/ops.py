@@ -271,14 +271,15 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
     if cost is not None and cost.n != n:
         raise ValueError("the cost is for n=%d segments, the model has n=%d" % (cost.n, n))
     forms = cost.forms if cost is not None else None  # host [J, 2n+3], copied into the launch's arguments
+    model_list = _models if _models is not None else sim_models  # the list of the call made below
+    if model_list is not None:
+        models = (_lib.SwmParams * len(model_list))(*model_list)  # host copies, copied into the launch's arguments
     with torch.cuda.device(dev):
         if _models is not None:
-            models = (_lib.SwmParams * len(_models))(*_models)  # host copies, copied into the launch's arguments
-            _lib.check(_lib.lib().swm_rollout_models(models, len(_models), ctypes.byref(cfg), _lib.stream_ptr()))
-        elif sim_models is not None:
-            models = (_lib.SwmParams * len(sim_models))(*sim_models)  # host copies, copied into the launch's arguments
+            _lib.check(_lib.lib().swm_rollout_models(models, len(model_list), ctypes.byref(cfg), _lib.stream_ptr()))
+        elif model_list is not None:
             _lib.check(_lib.lib().swm_rollout_ensemble(
-                ctypes.byref(params), ctypes.byref(cfg), models, len(sim_models),
+                ctypes.byref(params), ctypes.byref(cfg), models, len(model_list),
                 None if forms is None else forms.ctypes.data_as(ctypes.c_void_p),
                 0 if forms is None else forms.shape[0], _lib.stream_ptr()))
         elif cost is None:

@@ -512,6 +512,13 @@ def test_engine_rejects_bad_model_lists(S):
             S.ops.rollout_models(sims[:2], 10, B=8, base_policy=W, clip_actions=True, kernel=k)
     with pytest.raises(S._lib.SwimmerLibError):
         S.ops.rollout_models(sims[:2], 10, B=8, base_policy=W, want_trajectory=True)
+    # per-step screening is refused whatever its models; an ensemble screen leaves cfg.screen.sim unset (bad argument)
+    screen = dict(sim_thresh=1e9, real_thresh=1e9)
+    with pytest.raises(S._lib.SwimmerLibError, match="unsupported configuration"):
+        S.ops.rollout_models(sims[:4], 10, B=8, base_policy=W, screen=dict(screen, sim_params=sims[0]))
+    for ens in (sims[:1], sims[:7]):
+        with pytest.raises(S._lib.SwimmerLibError, match="bad argument"):
+            S.ops.rollout_models(sims[:4], 10, B=8, base_policy=W, screen=dict(screen, sim_params=ens))
     with pytest.raises(ValueError):
         S.ops.rollout_models([], 10, B=8, base_policy=W)
 
