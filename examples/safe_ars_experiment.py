@@ -26,6 +26,9 @@ parser.add_argument("--alpha", help="step size", type=float, default=0.0075)
 parser.add_argument("--nu", help="perturbations standard deviation", type=float, default=0.01)
 parser.add_argument("--path", help="directory for saving the results", type=str, default="results/safe_ars/")
 parser.add_argument("--n_seeds", help="number of random seeds", type=int, default=2)
+parser.add_argument("--backup", help="shield: the action tried when the simulator rejects a step (none: freeze, as the "
+                    "reference; zero: zero torque; damping: torque damping the joint velocities)",
+                    choices=["none", "zero", "damping"], default="none")
 args = parser.parse_args()
 
 n = 3
@@ -40,10 +43,19 @@ sim_env = SwimmerEnv("Simulator", n=3, m_i=theta_sim[0], l_i=theta_sim[1], k=the
 cost = lambda x: np.max([abs(x[3 + 2 * i]) for i in range(n)])  # noqa: E731
 
 
+backup = {}
+if args.backup != "none":
+    W_b = np.zeros((n - 1, 2 * n + 2))
+    if args.backup == "damping":  # torque_k = -0.5 (theta_dot_k - theta_dot_{k+1})
+        for k in range(n - 1):
+            W_b[k, 3 + 2 * k], W_b[k, 5 + 2 * k] = -0.5, 0.5
+    backup = dict(backup_policy=W_b)
+
+
 def experience(seed):
     unsafe_agent = Basic_ARS()
     sim_thresh = args.thresh - 1
-    safe_agent = Safe_ARS(cost, args.thresh, sim_thresh, sim_env)
+    safe_agent = Safe_ARS(cost, args.thresh, sim_thresh, sim_env, **backup)
     np.random.seed(seed)
     unsafe_returns, unsafe_states = unsafe_agent.train(args.n_iter, real_env, args.N, args.b, args.alpha, args.nu,
                                                        args.n_rollout)

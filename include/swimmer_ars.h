@@ -235,6 +235,23 @@ SWM_API int swm_rollout_ensemble(const swm_params_t* params, const swm_rollout_t
                                  const swm_params_t* sim_models /* HOST [n_models] */, int n_models,
                                  const double* forms /* HOST [n_forms, 2n+3], or NULL: built-in cost */,
                                  int n_forms, void* stream);
+/* swm_rollout_ensemble with a shield: when the models judge the policy's action a unsafe, the backup action
+ *     b = W_b obs + u_0     (obs the raw observation; clipped to +-max_u like a when clip_actions is set)
+ * is judged by every model by the same rule, and if it is safe the real step takes b instead of a and
+ * overrides[e] counts one more; only if b is unsafe too does the environment freeze, as in swm_rollout_ensemble.
+ * The next step starts again from the policy's action.  Returns sum every real step taken; violations count the
+ * real post-step costs above real_thresh on steps of both kinds.  `backup` is a HOST array of (n-1)(2n+2) + (n-1)
+ * doubles, W_b [n-1, 2n+2] row-major followed by u_0 [n-1] (either may be zero); it is copied into the launch's
+ * arguments like the models and forms.  `overrides` is a DEVICE int32 [B] or NULL; directions skipped by dir_mask
+ * report 0.  An environment that never takes the backup gets the results of swm_rollout_ensemble bit for bit.
+ * SWM_ERR_BAD_ARG: whatever swm_rollout_ensemble rejects, in the same order, then backup NULL or a non-finite
+ * entry (also for an empty batch).  SWM_ERR_UNSUPPORTED: as swm_rollout_ensemble. */
+SWM_API int swm_rollout_shielded(const swm_params_t* params, const swm_rollout_t* cfg,
+                                 const swm_params_t* sim_models /* HOST [n_models] */, int n_models,
+                                 const double* forms /* HOST [n_forms, 2n+3], or NULL: built-in cost */,
+                                 int n_forms,
+                                 const double* backup /* HOST [(n-1)(2n+2) + (n-1)]: W_b row-major, then u_0 */,
+                                 int32_t* overrides /* DEVICE [B] or NULL */, void* stream);
 /* Model-set rollouts: the rollouts of swm_rollout under each of n_models models (HOST array, 1..SWM_MAX_SIM_MODELS
  * structs with the same n) in one launch.  Rollout e of model m is exactly what environment e of swm_rollout with
  * params = &models[m] would run (same policy, perturbation, Philox counters, start state and init_perturb); only its

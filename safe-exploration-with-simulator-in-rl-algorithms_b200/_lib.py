@@ -128,6 +128,7 @@ def lib():
     L.swm_rollout.argtypes = [pp, ctypes.POINTER(SwmRollout), _dp]
     L.swm_rollout_costed.argtypes = [pp, ctypes.POINTER(SwmRollout), _dp, c_int, _dp]
     L.swm_rollout_ensemble.argtypes = [pp, ctypes.POINTER(SwmRollout), pp, c_int, _dp, c_int, _dp]
+    L.swm_rollout_shielded.argtypes = [pp, ctypes.POINTER(SwmRollout), pp, c_int, _dp, c_int, _dp, _dp, _dp]
     L.swm_rollout_models.argtypes = [pp, c_int, ctypes.POINTER(SwmRollout), _dp]
     L.swm_rollout_stats_blocks.argtypes = [pp, ctypes.POINTER(SwmRollout), _dp]
     L.swm_rollout_stats_blocks.restype = i64

@@ -520,10 +520,28 @@ int read_sim_models(const swm_params_t* models, int n_models, SimModels& sm) {
   return SWM_OK;
 }
 
-// swm_rollout_costed (sim_models == nullptr: the simulator is cfg->screen.sim, the forms are required) and
-// swm_rollout_ensemble (the simulators are sim_models; without forms the built-in cost).
+// Copies and checks the host backup of swm_rollout_shielded: W_b [n-1, 2n+2] row-major, then u_0 [n-1], finite.
+int read_backup(int n, const double* backup, int32_t* overrides, Backup& bk) {
+  if (!backup) return SWM_ERR_BAD_ARG;
+  const int na = n - 1, no = 2 * n + 2;
+  memset(&bk, 0, sizeof(bk));
+  for (int k = 0; k < na; ++k)
+    for (int j = 0; j <= no; ++j) {
+      const double v = j < no ? backup[(size_t)k * no + j] : backup[(size_t)na * no + k];
+      if (!isfinite(v)) return SWM_ERR_BAD_ARG;
+      if (j < no) bk.W[k][j] = v;
+      else bk.u0[k] = v;
+    }
+  bk.overrides = overrides;
+  return SWM_OK;
+}
+
+// swm_rollout_costed (sim_models == nullptr: the simulator is cfg->screen.sim, the forms are required),
+// swm_rollout_ensemble (the simulators are sim_models; without forms the built-in cost) and swm_rollout_shielded
+// (shield: the ensemble with a backup action, checked after the forms).
 int rollout_screened(const swm_params_t* params, const swm_rollout_t* cfg, const swm_params_t* sim_models,
-                     int n_models, const double* forms, int n_forms, void* stream) {
+                     int n_models, const double* forms, int n_forms, void* stream, bool shield = false,
+                     const double* backup = nullptr, int32_t* overrides = nullptr) {
   if (!params_ok(params) || !cfg || !cfg->screen.enabled) return SWM_ERR_BAD_ARG;
   swm_rollout_t c = *cfg;
   SimModels sm;
@@ -538,6 +556,11 @@ int rollout_screened(const swm_params_t* params, const swm_rollout_t* cfg, const
     const int rc = read_cost_forms(params->n, forms, n_forms, cf);
     if (rc != SWM_OK) return rc;
   }
+  Backup bk;
+  if (shield) {
+    const int rc = read_backup(params->n, backup, overrides, bk);
+    if (rc != SWM_OK) return rc;
+  }
   RolloutArgs a;
   RolloutFlags f;
   int rc = build_rollout_args(params, &c, a, f);
@@ -548,7 +571,7 @@ int rollout_screened(const swm_params_t* params, const swm_rollout_t* cfg, const
   rc = check_rollout_buffers(&c, f);
   if (rc != SWM_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-#define CALL(K) launch_rollout_screened_n<K>(a, sim_models ? &sm : nullptr, forms ? &cf : nullptr, f, st)
+#define CALL(K) launch_rollout_screened_n<K>(a, sim_models ? &sm : nullptr, forms ? &cf : nullptr, shield ? &bk : nullptr, f, st)
   SWM_DISPATCH_N(params->n, CALL)
 #undef CALL
 }
@@ -565,6 +588,13 @@ extern "C" int swm_rollout_ensemble(const swm_params_t* params, const swm_rollou
                                     void* stream) {
   if (!sim_models) return SWM_ERR_BAD_ARG;
   return rollout_screened(params, cfg, sim_models, n_models, forms, n_forms, stream);
+}
+
+extern "C" int swm_rollout_shielded(const swm_params_t* params, const swm_rollout_t* cfg,
+                                    const swm_params_t* sim_models, int n_models, const double* forms, int n_forms,
+                                    const double* backup, int32_t* overrides, void* stream) {
+  if (!sim_models) return SWM_ERR_BAD_ARG;
+  return rollout_screened(params, cfg, sim_models, n_models, forms, n_forms, stream, true, backup, overrides);
 }
 
 extern "C" int swm_rollout_models(const swm_params_t* models, int n_models, const swm_rollout_t* cfg, void* stream) {

@@ -195,8 +195,10 @@ __device__ __forceinline__ double cost_max_affine(const CostForms& f, const Obs&
 
 // Screening modes of the rollout kernel: none, the built-in cost max_i |thd_i|, or max-of-affine forms, judged by
 // the simulator model of RolloutArgs::sim or (ENSEMBLE*) by every model of an ensemble.
+// SHIELD*: the ensemble modes with a backup action that is tried when the policy's action is judged unsafe.
 enum ScreenMode {
-  SCREEN_NONE = 0, SCREEN_BUILTIN = 1, SCREEN_AFFINE = 2, SCREEN_ENSEMBLE = 3, SCREEN_ENSEMBLE_AFFINE = 4
+  SCREEN_NONE = 0, SCREEN_BUILTIN = 1, SCREEN_AFFINE = 2, SCREEN_ENSEMBLE = 3, SCREEN_ENSEMBLE_AFFINE = 4,
+  SCREEN_SHIELD = 5, SCREEN_SHIELD_AFFINE = 6
 };
 
 // The simulator models of ensemble screening (M = 1..SWM_MAX_SIM_MODELS; entries from M on are not read).
@@ -209,6 +211,23 @@ struct SimModelsForms {
   CostForms forms;
 };
 
+// The backup action of the shield, b = W . obs + u0 of the raw observation (row k of W: action k; entries past
+// n-1 actions and 2n+2 observations are not read), and the per-environment count of steps that took it.
+struct Backup {
+  double W[SWM_MAX_SEGMENTS - 1][2 * SWM_MAX_SEGMENTS + 2];
+  double u0[SWM_MAX_SEGMENTS - 1];
+  int* overrides;  // device [B] or nullptr
+};
+struct SimModelsBackup {
+  SimModels models;
+  Backup backup;
+};
+struct SimModelsFormsBackup {
+  SimModels models;
+  CostForms forms;
+  Backup backup;
+};
+
 // Type of the rollout kernel's second argument: the cost forms and / or the simulator models of the screening
 // mode, an empty struct without either.  MODELS (model-set mode, unscreened only): the models whose physics the
 // rollouts run, one per CTA row blockIdx.y; the lane-split kernels take the same argument.
@@ -217,6 +236,8 @@ template <int SCREEN, bool MODELS = false> struct ScreenForms { using type = NoC
 template <> struct ScreenForms<SCREEN_AFFINE> { using type = CostForms; };
 template <> struct ScreenForms<SCREEN_ENSEMBLE> { using type = SimModels; };
 template <> struct ScreenForms<SCREEN_ENSEMBLE_AFFINE> { using type = SimModelsForms; };
+template <> struct ScreenForms<SCREEN_SHIELD> { using type = SimModelsBackup; };
+template <> struct ScreenForms<SCREEN_SHIELD_AFFINE> { using type = SimModelsFormsBackup; };
 template <> struct ScreenForms<SCREEN_NONE, true> { using type = SimModels; };
 
 // The physics of a rollout: RolloutArgs::real, or in the model-set mode model blockIdx.y (warp- and CTA-uniform, read
@@ -235,21 +256,58 @@ __device__ __forceinline__ const CostForms& cost_forms_of(const CostForms& f) { 
 __device__ __forceinline__ const CostForms& cost_forms_of(const SimModelsForms& f) { return f.forms; }
 __device__ __forceinline__ const SimModels& sim_models_of(const SimModels& s) { return s; }
 __device__ __forceinline__ const SimModels& sim_models_of(const SimModelsForms& s) { return s.models; }
+__device__ __forceinline__ const CostForms& cost_forms_of(const SimModelsFormsBackup& f) { return f.forms; }
+__device__ __forceinline__ const SimModels& sim_models_of(const SimModelsBackup& s) { return s.models; }
+__device__ __forceinline__ const SimModels& sim_models_of(const SimModelsFormsBackup& s) { return s.models; }
+__device__ __forceinline__ const Backup& backup_of(const SimModelsBackup& s) { return s.backup; }
+__device__ __forceinline__ const Backup& backup_of(const SimModelsFormsBackup& s) { return s.backup; }
+
+// The judgement of the ensemble modes by one simulator model P: one simulator step with the action `act` from the
+// state (gdx, gdy, th, w) with sines s and cosines c, unsafe unless cost <= sim_thresh (a NaN cost is unsafe).
+template <int N, int FS, bool AFFINE, typename F>
+__device__ __forceinline__ bool model_unsafe(const F& forms, const Phys& P, double sim_thresh, double gdx, double gdy,
+                                             const double (&th)[N], const double (&s)[N], const double (&c)[N],
+                                             const double (&w)[N], const double (&act)[N > 1 ? N - 1 : 1],
+                                             double* sF) {
+  constexpr int NA = N - 1, NO = 2 * N + 2;
+  double sut[NA > 0 ? NA : 1], sgddx, sgddy, sthdd[N];
+#pragma unroll
+  for (int k = 0; k < NA; ++k) sut[k] = act[k] * P.u_scale;
+  gym_accel<N, FS>(P, s, c, gdx, gdy, w, sut, sgddx, sgddy, sthdd, sF);
+  double sim_cost;
+  if constexpr (AFFINE) {
+    auto so = [&](int k) {
+      if (k < 2) return fma(P.h_gdd_c, k == 0 ? sgddx : sgddy, k == 0 ? gdx : gdy);
+      const int i = (k - 2) / 2;
+      return (k & 1) ? fma(P.h, sthdd[i], w[i]) : fma(P.h, w[i], th[i]);
+    };
+    sim_cost = cost_max_affine<NO>(cost_forms_of(forms), so);
+  } else {
+    double sthd[N];
+#pragma unroll
+    for (int i = 0; i < N; ++i) sthd[i] = fma(P.h, sthdd[i], w[i]);
+    sim_cost = cost_max_abs_thd<N>(sthd);
+  }
+  return !(sim_cost <= sim_thresh);
+}
 
 // LINEAR: 0 fixed actions, 1 linear policy.  NORM: ARS V2 normalisation.  STATS: accumulate
 // shifted first/second moments of every visited state.  SCREEN: per-step simulator screening (ScreenMode).
 // With SCREEN_AFFINE the forms travel as the second kernel argument (5.9 KB of the constant bank), with
-// SCREEN_ENSEMBLE the models (2.3 KB), with SCREEN_ENSEMBLE_AFFINE both (8.2 KB); the other kernels' argument
-// block grows by one empty byte only.  MODELS: the model-set mode (SCREEN_NONE, gym dynamics, no statistics, no
-// trajectory), the models (2.3 KB) as the second argument.
+// SCREEN_ENSEMBLE the models (2.3 KB), with SCREEN_ENSEMBLE_AFFINE both (8.2 KB), and the SHIELD modes add the
+// backup (1.7 KB, so at most 9.9 KB); the other kernels' argument block grows by one empty byte only.  MODELS: the
+// model-set mode (SCREEN_NONE, gym dynamics, no statistics, no trajectory), the models (2.3 KB) as the second
+// argument.
 template <int N, int VARIANT, int WMODE, bool NORM, bool STATS, int SCREEN, bool MODELS>
 __global__ void __launch_bounds__(kRolloutBlock, SWM_ROLLOUT_MIN_BLOCKS)
 rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms<SCREEN, MODELS>::type forms) {
   static_assert(!MODELS || (SCREEN == SCREEN_NONE && VARIANT == 0 && !STATS), "model set: unscreened gym rollouts");
   constexpr int NO = 2 * N + 2, NA = N - 1, WS = NA * NO;
   constexpr bool LINEAR = (WMODE != W_NONE);
-  constexpr bool ENSEMBLE = SCREEN == SCREEN_ENSEMBLE || SCREEN == SCREEN_ENSEMBLE_AFFINE;
-  constexpr bool AFFINE = SCREEN == SCREEN_AFFINE || SCREEN == SCREEN_ENSEMBLE_AFFINE;
+  constexpr bool SHIELD = SCREEN == SCREEN_SHIELD || SCREEN == SCREEN_SHIELD_AFFINE;
+  constexpr bool ENSEMBLE = SCREEN == SCREEN_ENSEMBLE || SCREEN == SCREEN_ENSEMBLE_AFFINE || SHIELD;
+  constexpr bool AFFINE = SCREEN == SCREEN_AFFINE || SCREEN == SCREEN_ENSEMBLE_AFFINE || SCREEN == SCREEN_SHIELD_AFFINE;
+  static_assert(!SHIELD || (VARIANT == 0 && LINEAR && !NORM && !STATS), "shield: gym dynamics, linear V1 policies");
   const Phys& P = rollout_model<MODELS>(a, forms);
   extern __shared__ __align__(16) double smem[];
   const int tid = threadIdx.x;
@@ -398,7 +456,7 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
 
   double ret = skipped ? __longlong_as_double(0x7ff8000000000000LL) : 0.0;
   double sgx = 0.0, sgy = 0.0;  // gym variant: sum_t Gdot_t
-  int viol = 0, frozen = a.H;
+  int viol = 0, frozen = a.H, ovr = 0;
   double* traj = a.trajectory ? a.trajectory + e * NO : nullptr;
   const long long traj_step = a.B * NO;
 
@@ -414,6 +472,8 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
     }
   }
 
+  // SHIELD: this step is re-run with the backup action because the models rejected the policy's action
+  bool backup_turn = false;
   for (int t = 0; t < steps; ++t) {
     if (LINEAR) {
       // action_k = sum_j W[k][j] * obs_j, observation-major: the NA accumulators advance together so
@@ -424,8 +484,23 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
       double acc[NA > 0 ? NA : 1];
 #pragma unroll
       for (int k = 0; k < NA; ++k) acc[k] = 0.0;
+      if constexpr (SHIELD) {
+        if (backup_turn) {
+          // the backup action b = W_b . obs + u0 of the raw observation, in the order of the policy's product; the
+          // coefficients are warp-uniform kernel arguments, read from the constant bank like the cost forms
+          const Backup& bk = backup_of(forms);
 #pragma unroll
-      for (int j = 0; j < NO; ++j) {
+          for (int j = 0; j < NO; ++j) {
+            const double x = (j == 0) ? gdx : (j == 1) ? gdy : ((j & 1) ? thd[(j - 3) / 2] : th[(j - 2) / 2]);
+#pragma unroll
+            for (int k = 0; k < NA; ++k) acc[k] = fma(x, bk.W[k][j], acc[k]);
+          }
+#pragma unroll
+          for (int k = 0; k < NA; ++k) acc[k] += bk.u0[k];
+        }
+      }
+#pragma unroll
+      for (int j = 0; j < NO && !(SHIELD && backup_turn); ++j) {
         double x = (j == 0) ? gdx : (j == 1) ? gdy : ((j & 1) ? thd[(j - 3) / 2] : th[(j - 2) / 2]);
         if (NORM) x -= s_mu[j];
 #pragma unroll
@@ -496,36 +571,29 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
         // The single-model modes keep the judgement inline: called through model_unsafe their kernels compile to the
         // same instructions and spills but other registers and another order.
         const SimModels& sm = sim_models_of(forms);
-        auto model_unsafe = [&](const Phys& P, const double (&s)[N], const double (&c)[N],
-                                const double (&w)[N]) -> bool {
-          double sut[NA > 0 ? NA : 1], sgddx, sgddy, sthdd[N];
-#pragma unroll
-          for (int k = 0; k < NA; ++k) sut[k] = u[k] * P.u_scale;
-          gym_accel<N, FS>(P, s, c, gdx, gdy, w, sut, sgddx, sgddy, sthdd, sF);
-          double sim_cost;
-          if constexpr (AFFINE) {
-            auto so = [&](int k) {
-              if (k < 2) return fma(P.h_gdd_c, k == 0 ? sgddx : sgddy, k == 0 ? gdx : gdy);
-              const int i = (k - 2) / 2;
-              return (k & 1) ? fma(P.h, sthdd[i], w[i]) : fma(P.h, w[i], th[i]);
-            };
-            sim_cost = cost_max_affine<NO>(cost_forms_of(forms), so);
-          } else {
-            double sthd[N];
-#pragma unroll
-            for (int i = 0; i < N; ++i) sthd[i] = fma(P.h, sthdd[i], w[i]);
-            sim_cost = cost_max_abs_thd<N>(sthd);
-          }
-          return !(sim_cost <= a.sim_thresh);
-        };
 #pragma unroll 1
         for (int m = 1; m < sm.M; ++m) {
           double s[N], c[N], w[N];
 #pragma unroll
           for (int i = 0; i < N; ++i) { s[i] = opaque(sn[i]); c[i] = opaque(cs[i]); w[i] = opaque(thd[i]); }
-          unsafe |= model_unsafe(sm.p[m], s, c, w);
+          unsafe |= model_unsafe<N, FS, AFFINE>(forms, sm.p[m], a.sim_thresh, gdx, gdy, th, s, c, w, u, sF);
         }
-        unsafe |= model_unsafe(sm.p[0], sn, cs, thd);
+        unsafe |= model_unsafe<N, FS, AFFINE>(forms, sm.p[0], a.sim_thresh, gdx, gdy, th, sn, cs, thd, u, sF);
+        if constexpr (SHIELD) {
+          // The shield: a rejected policy action re-runs this step with the backup action (the state has not moved),
+          // judged by the same code; the real step takes it if it is safe, and a rejected backup freezes.  The code
+          // of the policy's steps is that of SCREEN_ENSEMBLE*, so an environment that never takes the backup
+          // computes what those kernels compute.
+          if (unsafe && !backup_turn) {
+            backup_turn = true;
+            --t;
+            continue;
+          }
+          if (!unsafe && backup_turn) {
+            backup_turn = false;
+            ++ovr;
+          }
+        }
       }
       if (unsafe) {
         // unsafe: nothing advances, and since obs and policy never change it never will again
@@ -551,7 +619,7 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
     } else {
       ret += swimmer_step<N, 1>(P, gdx, gdy, th, thd, u);
     }
-    if (SCREEN == SCREEN_BUILTIN || SCREEN == SCREEN_ENSEMBLE)
+    if (SCREEN == SCREEN_BUILTIN || SCREEN == SCREEN_ENSEMBLE || SCREEN == SCREEN_SHIELD)
       viol += (cost_max_abs_thd<N>(thd) > a.real_thresh) ? 1 : 0;
     if constexpr (AFFINE || STATS) {
       double x[NO];  // the real observation after the step
@@ -595,6 +663,9 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
     if (SCREEN != SCREEN_NONE) {
       if (a.violations) a.violations[e] = viol;
       if (a.frozen_at) a.frozen_at[e] = frozen;
+    }
+    if constexpr (SHIELD) {
+      if (backup_of(forms).overrides) backup_of(forms).overrides[e] = ovr;
     }
   }
 

@@ -1,7 +1,7 @@
 // Host-side template dispatch for one segment count N.  Each rollout_nK.cu translation unit
 // instantiates launch_*_n<K> so the (N x mode) kernel matrix compiles in parallel.  Three rollout
 // families: plain (swm_rollout, with the built-in screen), screened with cost forms and / or an
-// ensemble (swm_rollout_costed / swm_rollout_ensemble) and the model set (swm_rollout_models); all
+// ensemble (swm_rollout_costed / swm_rollout_ensemble / swm_rollout_shielded) and the model set (swm_rollout_models); all
 // take the policy storage from with_policy_storage.
 #pragma once
 #include <type_traits>
@@ -22,9 +22,10 @@ template <int N> int launch_step_n(const Phys& P, int variant, bool acc_only, co
                                    cudaStream_t st);
 template <int N> int launch_rollout_n(const RolloutArgs& a, const RolloutFlags& f, cudaStream_t st);
 // per-step screening with cost forms and / or an ensemble of simulator models: SCREEN_AFFINE without models (forms
-// required), else SCREEN_ENSEMBLE (no forms: the built-in cost) or SCREEN_ENSEMBLE_AFFINE
+// required), else SCREEN_ENSEMBLE (no forms: the built-in cost) or SCREEN_ENSEMBLE_AFFINE; with a backup (models
+// required) SCREEN_SHIELD or SCREEN_SHIELD_AFFINE
 template <int N> int launch_rollout_screened_n(const RolloutArgs& a, const SimModels* models, const CostForms* forms,
-                                               const RolloutFlags& f, cudaStream_t st);
+                                               const Backup* backup, const RolloutFlags& f, cudaStream_t st);
 // model-set mode: cfg->B environments for each of models.M models, one CTA row per model (f as for launch_rollout_n)
 template <int N> int launch_rollout_models_n(const RolloutArgs& a, const SimModels& models, const RolloutFlags& f,
                                              cudaStream_t st);
@@ -83,11 +84,26 @@ static int launch_rollout_one(const RolloutArgs& a, cudaStream_t st) {
 // gym dynamics, linear policies, ARS V1 without statistics.
 template <int N>
 int launch_rollout_screened_n(const RolloutArgs& a, const SimModels* models, const CostForms* forms,
-                              const RolloutFlags& f, cudaStream_t st) {
+                              const Backup* backup, const RolloutFlags& f, cudaStream_t st) {
   if (f.variant != SWM_DYN_GYM || !f.linear || !f.screen || f.norm || f.stats) return SWM_ERR_UNSUPPORTED;
   return with_policy_storage<N>(f.group_w, [&](auto w) {
     constexpr int WMODE = decltype(w)::value;
     const size_t smem = rollout_smem<N, 0, WMODE, false>();
+    if (backup && !forms) {
+      SimModelsBackup mb;
+      mb.models = *models;
+      mb.backup = *backup;
+      return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_SHIELD, false>, smem, a.B, 1, st, a,
+                                 mb);
+    }
+    if (backup) {
+      SimModelsFormsBackup mfb;
+      mfb.models = *models;
+      mfb.forms = *forms;
+      mfb.backup = *backup;
+      return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_SHIELD_AFFINE, false>, smem, a.B, 1,
+                                 st, a, mfb);
+    }
     if (!models)
       return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_AFFINE, false>, smem, a.B, 1, st, a,
                                  *forms);
@@ -172,7 +188,7 @@ template int launch_step_n<SWM_INSTANTIATE_N>(const Phys&, int, bool, const doub
                                               double*, double*, long long, cudaStream_t);
 template int launch_rollout_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const RolloutFlags&, cudaStream_t);
 template int launch_rollout_screened_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const SimModels*, const CostForms*,
-                                                          const RolloutFlags&, cudaStream_t);
+                                                          const Backup*, const RolloutFlags&, cudaStream_t);
 template int launch_rollout_models_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const SimModels&, const RolloutFlags&,
                                                         cudaStream_t);
 

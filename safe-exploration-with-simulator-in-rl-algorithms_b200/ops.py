@@ -8,13 +8,14 @@ swimmer_env.py / environment.py / ars_agent.py / safe_ars.py are thin layers ove
 import ctypes
 import math
 
+import numpy as np
 import torch
 
 from . import _lib
 from ._lib import (ARS_AGENT, ARS_RLGLUE, ARS_TOPB, DELTA_01, DELTA_PM1, GYM, POLICY_DELTAS,
                    POLICY_EXPLICIT, POLICY_FIXED_ACTION, POLICY_PHILOX, RLGLUE)
 
-__all__ = ["step_batched", "step_batched_models", "accelerations_batched", "rollout", "rollout_models", "RolloutResult", "ChunkedRollout", "plan_chunks", "philox_deltas",
+__all__ = ["step_batched", "step_batched_models", "accelerations_batched", "rollout", "rollout_models", "backup_array", "RolloutResult", "ChunkedRollout", "plan_chunks", "philox_deltas",
            "ars_topb", "ars_update", "pack_exchange", "counter_add", "record_nanmean", "stats_finalize", "stats_merge", "reduce_returns", "screen_mask", "policy_actions", "update_args",
            "EstimateData", "prediction_error", "cmaes_default_popsize", "cmaes_state_doubles", "cmaes_view", "cmaes_init",
            "cmaes_sample", "cmaes_update", "cmaes_generation",
@@ -126,7 +127,7 @@ def accelerations_batched(params, states, actions, variant=GYM):
 
 class RolloutResult:
     __slots__ = ("returns", "final_state", "trajectory", "stats_partial", "stats_blocks",
-                 "violations", "frozen_at", "samples")
+                 "violations", "frozen_at", "overrides", "samples")
 
     def __init__(self):
         for s in self.__slots__:
@@ -153,6 +154,10 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
     screens with that cost instead (swm_rollout_costed; one thread per environment, one plain launch).
     screen["sim_params"] = a list or tuple of 1..16 params (the real model's n) screens by the whole ensemble, with
     either cost: a step is taken only if every model judges it safe (swm_rollout_ensemble; same kernel and launch).
+    screen["backup"] = dict(policy=W_b [n-1, 2n+2] or None, action=u_0 [n-1] or None) adds a shield: a step whose
+    action the model(s) reject is taken with the backup action W_b obs + u_0 instead if the same model(s) judge that
+    safe, and freezes only otherwise (swm_rollout_shielded; a single simulator is the ensemble of one).  The result
+    then has `overrides` [B] int32, the number of steps each environment took with the backup.
     stats_pivot[2n+2] enables the V2 moment accumulation.  `out` may carry preallocated
     tensors (returns, final_state, trajectory, stats_partial) to stay allocation-free in loops.
     kernel: _lib.KERNEL_AUTO (chosen from B, n and the SM count) / KERNEL_THREAD (one thread per
@@ -271,12 +276,24 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
     if cost is not None and cost.n != n:
         raise ValueError("the cost is for n=%d segments, the model has n=%d" % (cost.n, n))
     forms = cost.forms if cost is not None else None  # host [J, 2n+3], copied into the launch's arguments
+    backup = screen.get("backup") if screen is not None else None
+    if backup is not None:
+        backup = backup_array(n, backup.get("policy"), backup.get("action"))  # host, copied into the launch's arguments
+        res.overrides = buf("overrides", (B,), torch.int32)
+        if sim_models is None:
+            sim_models = [cfg.screen.sim]
     model_list = _models if _models is not None else sim_models  # the list of the call made below
     if model_list is not None:
         models = (_lib.SwmParams * len(model_list))(*model_list)  # host copies, copied into the launch's arguments
     with torch.cuda.device(dev):
         if _models is not None:
             _lib.check(_lib.lib().swm_rollout_models(models, len(model_list), ctypes.byref(cfg), _lib.stream_ptr()))
+        elif backup is not None:
+            _lib.check(_lib.lib().swm_rollout_shielded(
+                ctypes.byref(params), ctypes.byref(cfg), models, len(model_list),
+                None if forms is None else forms.ctypes.data_as(ctypes.c_void_p),
+                0 if forms is None else forms.shape[0], backup.ctypes.data_as(ctypes.c_void_p),
+                res.overrides.data_ptr(), _lib.stream_ptr()))
         elif model_list is not None:
             _lib.check(_lib.lib().swm_rollout_ensemble(
                 ctypes.byref(params), ctypes.byref(cfg), models, len(model_list),
@@ -289,6 +306,24 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
                                                      forms.ctypes.data_as(ctypes.c_void_p), forms.shape[0],
                                                      _lib.stream_ptr()))
     return res
+
+
+def backup_array(n, policy=None, action=None):
+    """The backup action W_b obs + u_0 of a shield as swm_rollout_shielded takes it: a host float64 array of W_b
+    [n-1, 2n+2] row-major followed by u_0 [n-1] (None: zero).  Raises ValueError for another shape or a non-finite
+    entry."""
+    def host(x, shape, name):
+        if x is None:
+            return np.zeros(shape)
+        x = np.array(x.cpu() if torch.is_tensor(x) else x, dtype=np.float64)
+        if x.shape != shape:
+            raise ValueError("the backup %s must have shape %s for n=%d, got %s" % (name, shape, n, x.shape))
+        if not np.isfinite(x).all():
+            raise ValueError("the backup %s must be finite" % name)
+        return x
+    W = host(policy, (act_dim(n), obs_dim(n)), "policy")
+    u0 = host(action, (act_dim(n),), "action")
+    return np.ascontiguousarray(np.concatenate([W.reshape(-1), u0]))
 
 
 def rollout_models(params_list, H, **kw):

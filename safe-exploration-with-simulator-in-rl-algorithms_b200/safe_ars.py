@@ -135,9 +135,14 @@ class Safe_ARS(Basic_ARS):
     """ARS V1 with per-step safe exploration through a simulator (safe_ars/ars.py:103-153).
 
     `sim_env` may also be a sequence of 1..16 SwimmerEnv (an ensemble of simulator models, e.g. points of the set
-    the real parameters are known to lie in): a step is then taken only if every model judges it safe."""
+    the real parameters are known to lie in): a step is then taken only if every model judges it safe.
 
-    def __init__(self, cost, real_threshold, sim_threshold, sim_env):
+    `backup_policy` W_b [n-1, 2n+2] and / or `backup_action` u_0 [n-1] (declared extension; default: none) add a
+    shield: a step whose action the simulator(s) reject is taken with the backup action W_b obs + u_0 if the same
+    simulator(s) judge that safe (zero torque, a damping controller, a known hand controller), and the rollout freezes
+    only if the backup is unsafe too.  Without them the agent behaves as the reference."""
+
+    def __init__(self, cost, real_threshold, sim_threshold, sim_env, backup_policy=None, backup_action=None):
         if isinstance(sim_env, SwimmerEnv):
             n = sim_env.n
         else:
@@ -159,6 +164,11 @@ class Safe_ARS(Basic_ARS):
         self.real_thresh = real_threshold
         self.sim_thresh = sim_threshold
         self.sim_env = sim_env
+        self.backup = None
+        if backup_policy is not None or backup_action is not None:
+            b = ops.backup_array(n, backup_policy, backup_action)  # ValueError for a wrong shape or non-finite value
+            ws = (n - 1) * (2 * n + 2)
+            self.backup = dict(policy=b[:ws].reshape(n - 1, 2 * n + 2), action=b[ws:])
 
     def _screen(self, real_env):
         if isinstance(self.sim_env, SwimmerEnv):
@@ -172,6 +182,8 @@ class Safe_ARS(Basic_ARS):
         screen = dict(sim_params=sim, sim_thresh=self.sim_thresh, real_thresh=self.real_thresh)
         if isinstance(self.cost, MaxAffineCost):
             screen["cost"] = self.cost
+        if self.backup is not None:
+            screen["backup"] = self.backup
         return screen
 
     def isSafe(self, cost, thresh, env, state, action):
@@ -183,3 +195,14 @@ class Safe_ARS(Basic_ARS):
         env.set_state(state)
         obs, _, _, _ = env.step(action)
         return cost(obs) <= thresh
+
+    def shielded_action(self, cost, thresh, env, state, action):
+        """The action the shielded rollout takes from `state` (host counterpart of the kernel's decision): `action` if
+        isSafe judges it safe, else the backup action W_b state + u_0 if isSafe judges that safe, else None (the
+        rollout freezes).  Without a backup an unsafe action gives None.  Leaves env in its last simulated state."""
+        if self.isSafe(cost, thresh, env, state, action):
+            return action
+        if self.backup is None:
+            return None
+        b = self.backup["policy"] @ np.asarray(state, dtype=np.float64) + self.backup["action"]
+        return b if self.isSafe(cost, thresh, env, state, b) else None
