@@ -437,8 +437,9 @@ SWM_API int swm_rlglue_protocol(const swm_params_t* params, const swm_rlglue_pro
  * candidate x (d = 1..3 physical parameters) over K recorded trajectories of H observations is
  *   err(x) = sum_k sum_{t < H-1} || step_x(s_{k,t}, W_k s_{k,t}) - s_{k,t+1} ||_2
  * with the gym dynamics and the V1 policy product W_k s (as the reference, also for V2-recorded data).
- * A candidate is the base model with fields[i] replaced by x[i]; a candidate with m_i <= 0 or l_i <= 0 is
- * not stepped and gets +inf, and every non-finite sum becomes +inf.  Each err[c] is summed in a fixed order
+ * A candidate is the base model with fields[i] replaced by x[i]; a candidate whose m_i or l_i is not positive
+ * and finite is not stepped and gets +inf, and every non-finite sum becomes +inf.  The recorded data must be
+ * for base->n segments: the struct carries no n, the kernel indexes it with the strides of base->n.  Each err[c] is summed in a fixed order
  * (transitions within a CTA, then CTAs in index order) that depends on neither M nor the candidate's index:
  * results are bit-identical from run to run and permute with the candidates. */
 #define SWM_MAX_CANDIDATES 1024
@@ -467,8 +468,8 @@ SWM_API int swm_prediction_error(const swm_params_t* base, const swm_estimate_da
  *   7+5d+2d^2+L z[lambda, d] (the last generation's standard normal draws)
  * Sampling: z ~ N(0, I) by Box-Muller (r = sqrt(-2 ln(1 - u0)), angle 2 pi u1) from Philox4x32-10, key = seed,
  * counter = (pair j, candidate c, generation, 2), u = the 53-bit uniforms of swm_philox_t; candidate
- * x_c = mean + sigma * B * (D .* z_c).  Update: rank by fitness ascending (+inf and NaN last, ties by lower
- * index), recombination, evolution paths, C and sigma, then C = B diag(D^2) B^T by cyclic Jacobi with a fixed
+ * x_c = mean + sigma * B * (D .* z_c).  Update: rank by fitness ascending (+inf and NaN last, -inf an ordinary
+ * value that ranks first, ties by lower index), recombination, evolution paths, C and sigma, then C = B diag(D^2) B^T by cyclic Jacobi with a fixed
  * sweep count, best-ever tracking, and the stop tests (in this order): tolfun (range of the full best-f history
  * and this generation's fitness < tolfun), tolx (sigma sqrt(C_ii) < tolx and sigma |p_c,i| < tolx for all i),
  * condition (max D^2 / min D^2 > 1e14 or C not positive definite), max generations.  Once status != RUNNING
@@ -491,7 +492,9 @@ SWM_API int swm_cmaes_sample(double* state, int d, int lambda, uint64_t seed, do
 /* one update from the candidates of swm_cmaes_sample and their fitness[lambda]; advances the generation */
 SWM_API int swm_cmaes_update(double* state, int d, int lambda, const double* candidates, const double* fitness,
                              void* stream);
-/* sample + prediction-error objective (data->d == d) + update: one generation, no host round trip */
+/* sample + prediction-error objective (data->d == d) + update: one generation, no host round trip.  The
+ * objective runs with M = lambda, so data->workspace must hold swm_prediction_error_workspace_doubles(K, H,
+ * lambda) doubles; the struct carries no capacity, so this is not checked here. */
 SWM_API int swm_cmaes_generation(double* state, int d, int lambda, uint64_t seed, const swm_params_t* base,
                                  const swm_estimate_data_t* data, double* candidates, double* fitness,
                                  void* stream);

@@ -48,8 +48,12 @@ __host__ __device__ inline swm_params_t candidate_params(const swm_params_t& bas
   return p;
 }
 
-// NaN fails both comparisons: a NaN mass or length is non-physical too
-__host__ __device__ inline bool physical(const swm_params_t& p) { return p.m_i > 0.0 && p.l_i > 0.0; }
+// A mass or length that is not positive and finite is non-physical.  NaN fails every comparison; an infinite
+// mass must be refused explicitly, since it zeroes the torque and friction constants of make_phys and would
+// otherwise step to a finite error.
+__host__ __device__ inline bool physical(double m, double l) {
+  return m > 0.0 && l > 0.0 && isfinite(m) && isfinite(l);
+}
 
 // One thread = one recorded transition (k, t).  The state, its sines/cosines and the V1 action W_k s do not
 // depend on the model, so they are formed once; the loop then steps every candidate model (constants in shared
@@ -94,7 +98,7 @@ __global__ void __launch_bounds__(kEstBlock) prediction_kernel(const EstArgs a) 
   for (int c = 0; c < a.M; ++c) {
     const Phys& P = sP[c];
     double e = 0.0;
-    if (P.m > 0.0 && P.l > 0.0) {  // uniform over the CTA
+    if (physical(P.m, P.l)) {  // uniform over the CTA
       // swimmer_step<N, 0> from the precomputed sines/cosines
       double ut[NA > 0 ? NA : 1], gddx, gddy, thdd[N];
 #pragma unroll
@@ -133,8 +137,8 @@ __global__ void prediction_reduce_kernel(const EstArgs a, long long n_blocks, do
   if (c >= a.M) return;
   double v = 0.0;
   for (long long b = 0; b < n_blocks; ++b) v += a.partial[b * a.M + c];
-  const bool ok = physical(candidate_params(a.base, a.fields, a.d, a.cand + (size_t)c * a.d));
-  err[c] = (ok && isfinite(v)) ? v : __longlong_as_double(0x7ff0000000000000LL);
+  const swm_params_t p = candidate_params(a.base, a.fields, a.d, a.cand + (size_t)c * a.d);
+  err[c] = (physical(p.m_i, p.l_i) && isfinite(v)) ? v : __longlong_as_double(0x7ff0000000000000LL);
 }
 
 // ---- CMA-ES -----------------------------------------------------------------------------------------------
@@ -207,7 +211,7 @@ __global__ void cmaes_sample_kernel(double* __restrict__ S, int d, int lam, uint
   }
 }
 
-// ascending by fitness, NaN / +inf last, ties by lower index
+// ascending by fitness, NaN / +inf last (-inf is an ordinary value and ranks first), ties by lower index
 __device__ __forceinline__ bool fit_less(double a, int ia, double b, int ib) {
   const bool an = !(a < __longlong_as_double(0x7ff0000000000000LL)), bn = !(b < __longlong_as_double(0x7ff0000000000000LL));
   if (an || bn) return (an && bn) ? (ia < ib) : bn;
@@ -246,8 +250,9 @@ __device__ void jacobi_eigen(int d, double* A, double* V) {
   }
 }
 
-// One CTA: every thread ranks one candidate by counting, then thread 0 runs the d <= 3 arithmetic.
-__global__ void cmaes_update_kernel(double* __restrict__ S, int d, int lam, const double* __restrict__ cand,
+// One CTA: every thread ranks one candidate by counting, then thread 0 runs the d <= 3 arithmetic.  The CTA has
+// up to SWM_MAX_CANDIDATES threads: the launch bound keeps the kernel within the register file at that size.
+__global__ void __launch_bounds__(SWM_MAX_CANDIDATES) cmaes_update_kernel(double* __restrict__ S, int d, int lam, const double* __restrict__ cand,
                                     const double* __restrict__ fit) {
   __shared__ int order[SWM_MAX_CANDIDATES];
   if (S[kStatus] != 0.0) return;

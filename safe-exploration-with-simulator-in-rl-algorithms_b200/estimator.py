@@ -31,13 +31,18 @@ class Estimator:
             "cuda", torch.cuda.current_device())
         self._cache = {}
         self._data = None
+        self._data_key = None
 
     def _device_data(self, max_candidates):
-        """The subset's trajectories and policies, uploaded once, with objective scratch for max_candidates."""
-        if self._data is None or self._data.max_candidates < max_candidates:
-            traj = torch.stack([self._traj(int(k))[0] for k in self.subset])
-            pol = torch.stack([self._traj(int(k))[1].reshape(-1) for k in self.subset])
+        """The subset's trajectories and policies, uploaded once per subset, with objective scratch for
+        max_candidates.  Keyed on the subset's indices, so that reassigning or editing `subset` is seen here as
+        it is by `I`."""
+        key = tuple(int(k) for k in self.subset)
+        if self._data is None or self._data_key != key or self._data.max_candidates < max_candidates:
+            traj = torch.stack([self._traj(k)[0] for k in key])
+            pol = torch.stack([self._traj(k)[1].reshape(-1) for k in key])
             self._data = ops.EstimateData(traj, pol, self.unknowns, max_candidates)
+            self._data_key = key
         return self._data
 
     def _base_params(self):

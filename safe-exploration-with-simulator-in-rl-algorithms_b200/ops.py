@@ -655,14 +655,45 @@ class EstimateData:
         return len(self.unknowns)
 
 
+def _est_tensors(device, *checks):
+    """Host-side checks of the tensors an estimation kernel reads or writes, before anything is enqueued.  checks:
+    (name, tensor, shape) with shape a tuple, or an int for "at least that many elements".  First the format of
+    each (float64, shape, contiguous), then that each is a CUDA tensor, on `device` if given."""
+    for name, t, shape in checks:
+        if not isinstance(t, torch.Tensor) or t.dtype != torch.float64:
+            raise ValueError("%s must be a float64 tensor, got %s" % (name, getattr(t, "dtype", type(t).__name__)))
+        if isinstance(shape, int):
+            if t.numel() < shape:
+                raise ValueError("%s must hold at least %d doubles, got %d" % (name, shape, t.numel()))
+        elif tuple(t.shape) != tuple(shape):
+            raise ValueError("%s must have shape %s, got %s" % (name, tuple(shape), tuple(t.shape)))
+        if not t.is_contiguous():
+            raise ValueError("%s must be contiguous" % name)
+    for name, t, _ in checks:
+        if not t.is_cuda:
+            raise ValueError("%s must be a CUDA tensor, got one on %s" % (name, t.device))
+        if device is not None and t.device != device:
+            raise ValueError("%s must be on %s, got %s" % (name, device, t.device))
+
+
+def _est_model(base_params, data):
+    """The objective indexes the recorded data with the strides of base_params.n: they must agree."""
+    if base_params.n != data.n:
+        raise ValueError("the base model has n=%d segments, the recorded data n=%d" % (base_params.n, data.n))
+
+
 def prediction_error(base_params, data, candidates, out=None):
     """err[M] = sum_k sum_t || step_x(s_kt, W_k s_kt) - s_k,t+1 || for candidates[M, d] (Estimator.I of a whole
-    population in one launch; +inf for m_i <= 0 or l_i <= 0 and for non-finite sums).  `data`: EstimateData."""
-    _lib.require_cuda()
+    population in one launch; +inf for m_i or l_i not positive and finite and for non-finite sums).
+    `data`: EstimateData for base_params.n segments."""
+    _est_model(base_params, data)
     candidates = _lib.f64(candidates).contiguous()
     M = candidates.shape[0]
     if tuple(candidates.shape) != (M, data.d) or M > data.max_candidates:
         raise ValueError("candidates must be [M <= %d, %d]" % (data.max_candidates, data.d))
+    checks = [("candidates", candidates, (M, data.d))] + ([("out", out, (M,))] if out is not None else [])
+    _est_tensors(data.trajectories.device, *checks)
+    _lib.require_cuda()
     err = torch.empty(M, dtype=torch.float64, device=candidates.device) if out is None else out
     with torch.cuda.device(candidates.device):
         _lib.check(_lib.lib().swm_prediction_error(ctypes.byref(base_params), ctypes.byref(data.c),
@@ -700,6 +731,7 @@ def cmaes_view(state, d, popsize):
 def cmaes_init(state, x0, popsize, sigma0=1.0, tolfun=1e-11, tolx=1e-11, max_generations=0):
     """Fresh CMA-ES state around x0 (host sequence of d floats); max_generations <= 0: the cma default."""
     d = len(x0)
+    _est_tensors(None, ("state", state, cmaes_state_doubles(d, popsize)))
     x = (ctypes.c_double * d)(*[float(v) for v in x0])
     with torch.cuda.device(state.device):
         _lib.check(_lib.lib().swm_cmaes_init(_lib.ptr(state), d, int(popsize), x, float(sigma0), float(tolfun),
@@ -709,6 +741,8 @@ def cmaes_init(state, x0, popsize, sigma0=1.0, tolfun=1e-11, tolx=1e-11, max_gen
 
 def cmaes_sample(state, d, popsize, seed, candidates):
     """candidates[popsize, d] = mean + sigma B D z of the current generation (z is kept in the state)."""
+    _est_tensors(state.device, ("state", state, cmaes_state_doubles(d, popsize)),
+                 ("candidates", candidates, (popsize, d)))
     with torch.cuda.device(state.device):
         _lib.check(_lib.lib().swm_cmaes_sample(_lib.ptr(state), int(d), int(popsize), int(seed) & (2 ** 64 - 1),
                                                _lib.ptr(candidates), _lib.stream_ptr()))
@@ -717,6 +751,8 @@ def cmaes_sample(state, d, popsize, seed, candidates):
 
 def cmaes_update(state, d, popsize, candidates, fitness):
     """One CMA-ES update from the sampled candidates and their fitness[popsize]."""
+    _est_tensors(state.device, ("state", state, cmaes_state_doubles(d, popsize)),
+                 ("candidates", candidates, (popsize, d)), ("fitness", fitness, (popsize,)))
     with torch.cuda.device(state.device):
         _lib.check(_lib.lib().swm_cmaes_update(_lib.ptr(state), int(d), int(popsize), _lib.ptr(candidates),
                                                _lib.ptr(fitness), _lib.stream_ptr()))
@@ -724,7 +760,13 @@ def cmaes_update(state, d, popsize, candidates, fitness):
 
 
 def cmaes_generation(state, popsize, seed, base_params, data, candidates, fitness):
-    """sample + prediction_error + update of one generation, enqueued without a host round trip (capturable)."""
+    """sample + prediction_error + update of one generation, enqueued without a host round trip (capturable).
+    The objective runs for M = popsize candidates in data's workspace: data.max_candidates must cover it."""
+    _est_model(base_params, data)
+    if int(popsize) > data.max_candidates:
+        raise ValueError("popsize %d exceeds the %d candidates data's workspace holds" % (popsize, data.max_candidates))
+    _est_tensors(data.trajectories.device, ("state", state, cmaes_state_doubles(data.d, popsize)),
+                 ("candidates", candidates, (popsize, data.d)), ("fitness", fitness, (popsize,)))
     with torch.cuda.device(state.device):
         _lib.check(_lib.lib().swm_cmaes_generation(_lib.ptr(state), data.d, int(popsize), int(seed) & (2 ** 64 - 1),
                                                    ctypes.byref(base_params), ctypes.byref(data.c),

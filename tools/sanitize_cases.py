@@ -1,6 +1,7 @@
 """Small invocations of every kernel family (all policy-storage modes, V2 moments in registers and in
 shared memory, screening, trajectories, ragged last block, ARS epilogue, every rollout kernel: per-thread,
-lane-split, lane-split with operator warp; the RL-Glue protocol kernel) for
+lane-split, lane-split with operator warp; the RL-Glue protocol kernel; the estimation objective at n = 2, 8, 10
+and CMA-ES at lambda = 2, 33, 1024) for
 `compute-sanitizer --tool memcheck|racecheck|synccheck python tools/sanitize_cases.py [n ...]`."""
 import os
 import sys
@@ -53,9 +54,34 @@ def main(ns=(2, 3, 4, 5, 6, 7, 8, 9, 10)):
                           distributed=False, sim_params=sim, sim_threshold=-1.0, curve_capacity=4)
         eng.run_iteration()
         eng.run_iteration()
+        if n in (2, 8, 10):
+            estimation(n, rng)
         torch.cuda.synchronize()
         print("n=%d ok" % n, flush=True)
     print("sanitize cases done")
+
+
+def estimation(n, rng):
+    """The prediction-error objective at a ragged transition count (T = 3 * 43 = 129: a second CTA with one
+    transition, CTAs across trajectory boundaries) and M = 129 (a second block of the reduce grid), then CMA-ES
+    generations at lambda = 2, 33 and 1024 (one, two and 32 warps of ranking; 1, 1 and 8 sampling blocks)."""
+    no, K, H = 2 * n + 2, 3, 44
+    trajs = torch.as_tensor(rng.normal(size=(K, H, no)) * 0.5).cuda()
+    pols = torch.as_tensor(rng.uniform(-0.3, 0.3, (K, n - 1, no))).cuda()
+    base = S.make_params(n=n)
+    cand = torch.as_tensor(np.array([1.0, 1.0, 10.0]) * rng.uniform(0.9, 1.1, (129, 3))).cuda()
+    data = S.ops.EstimateData(trajs, pols, ("m_i", "l_i", "k"), max_candidates=1024)
+    assert bool(torch.isfinite(S.ops.prediction_error(base, data, cand)).all())
+    for lam in (2, 33, 1024):
+        state = torch.empty(S.ops.cmaes_state_doubles(3, lam), dtype=torch.float64, device="cuda")
+        S.ops.cmaes_init(state, [1.0, 1.0, 10.0], lam, sigma0=0.05)
+        x = torch.empty(lam, 3, dtype=torch.float64, device="cuda")
+        f = torch.empty(lam, dtype=torch.float64, device="cuda")
+        S.ops.cmaes_sample(state, 3, lam, 1, x)
+        S.ops.prediction_error(base, data, x, out=f)
+        S.ops.cmaes_update(state, 3, lam, x, f)
+        for _ in range(2):
+            S.ops.cmaes_generation(state, lam, 1, base, data, x, f)
 
 
 if __name__ == "__main__":
