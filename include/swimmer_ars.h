@@ -252,6 +252,27 @@ SWM_API int swm_rollout_shielded(const swm_params_t* params, const swm_rollout_t
                                  int n_forms,
                                  const double* backup /* HOST [(n-1)(2n+2) + (n-1)]: W_b row-major, then u_0 */,
                                  int32_t* overrides /* DEVICE [B] or NULL */, void* stream);
+/* swm_rollout_shielded with a lookahead of K = `lookahead` backup steps (model-predictive shielding): an action a is
+ * judged safe from the real state s only if, for EVERY model m,
+ *     x_1 = f_m(s, a),   x_{j+1} = f_m(x_j, backup(x_j)) for j = 1..K,   cost(x_j) <= sim_thresh for j = 1..K+1,
+ * f_m one explicit-Euler step of model m (the step of the one-step judgement) and backup(x) = W_b x + u_0 of the
+ * raw observation x, clipped to +-max_u of the REAL model when clip_actions is set (a NaN cost is unsafe).  The step
+ * is the shield's: the policy's action if it is safe by this rule, else the backup b_0 = backup(s) if it is safe by
+ * the same rule (overrides[e] counts one more), else the environment freezes for good.  Returns, violations,
+ * frozen_at, final_state, trajectory and dir_mask mean what they mean for swm_rollout_shielded.  K = 0 is
+ * swm_rollout_shielded, whose kernels it runs, bit for bit.  One judgement takes up to n_models * (K+1) simulator
+ * steps and stops at the first unsafe cost; a step whose policy action is rejected takes two judgements.  There is
+ * no implicit backup: a zero-torque one is an all-zero `backup` array.
+ * SWM_ERR_BAD_ARG: whatever swm_rollout_shielded rejects, in the same order, then lookahead outside
+ * 0..SWM_MAX_LOOKAHEAD (also for an empty batch).  SWM_ERR_UNSUPPORTED: as swm_rollout_shielded. */
+#define SWM_MAX_LOOKAHEAD 1024
+SWM_API int swm_rollout_lookahead(const swm_params_t* params, const swm_rollout_t* cfg,
+                                  const swm_params_t* sim_models /* HOST [n_models] */, int n_models,
+                                  const double* forms /* HOST [n_forms, 2n+3], or NULL: built-in cost */,
+                                  int n_forms,
+                                  const double* backup /* HOST [(n-1)(2n+2) + (n-1)]: W_b row-major, then u_0 */,
+                                  int lookahead /* 0..SWM_MAX_LOOKAHEAD */,
+                                  int32_t* overrides /* DEVICE [B] or NULL */, void* stream);
 /* Model-set rollouts: the rollouts of swm_rollout under each of n_models models (HOST array, 1..SWM_MAX_SIM_MODELS
  * structs with the same n) in one launch.  Rollout e of model m is exactly what environment e of swm_rollout with
  * params = &models[m] would run (same policy, perturbation, Philox counters, start state and init_perturb); only its

@@ -23,6 +23,7 @@ ABI_VERSION = 3  # include/swimmer_ars.h SWM_ABI_VERSION
 MAX_MODELS_PER_STEP = 24  # SWM_MAX_MODELS_PER_STEP
 MAX_COST_FORMS = 32  # SWM_MAX_COST_FORMS
 MAX_SIM_MODELS = 16  # SWM_MAX_SIM_MODELS
+MAX_LOOKAHEAD = 1024  # SWM_MAX_LOOKAHEAD
 MAX_CANDIDATES = 1024  # SWM_MAX_CANDIDATES
 CMAES_MIN_POPSIZE = 2  # SWM_CMAES_MIN_POPSIZE
 FIELDS = {"m_i": 0, "l_i": 1, "k": 2}  # swm_field
@@ -129,6 +130,7 @@ def lib():
     L.swm_rollout_costed.argtypes = [pp, ctypes.POINTER(SwmRollout), _dp, c_int, _dp]
     L.swm_rollout_ensemble.argtypes = [pp, ctypes.POINTER(SwmRollout), pp, c_int, _dp, c_int, _dp]
     L.swm_rollout_shielded.argtypes = [pp, ctypes.POINTER(SwmRollout), pp, c_int, _dp, c_int, _dp, _dp, _dp]
+    L.swm_rollout_lookahead.argtypes = [pp, ctypes.POINTER(SwmRollout), pp, c_int, _dp, c_int, _dp, c_int, _dp, _dp]
     L.swm_rollout_models.argtypes = [pp, c_int, ctypes.POINTER(SwmRollout), _dp]
     L.swm_rollout_stats_blocks.argtypes = [pp, ctypes.POINTER(SwmRollout), _dp]
     L.swm_rollout_stats_blocks.restype = i64

@@ -537,11 +537,13 @@ int read_backup(int n, const double* backup, int32_t* overrides, Backup& bk) {
 }
 
 // swm_rollout_costed (sim_models == nullptr: the simulator is cfg->screen.sim, the forms are required),
-// swm_rollout_ensemble (the simulators are sim_models; without forms the built-in cost) and swm_rollout_shielded
-// (shield: the ensemble with a backup action, checked after the forms).
+// swm_rollout_ensemble (the simulators are sim_models; without forms the built-in cost), swm_rollout_shielded
+// (shield: the ensemble with a backup action, checked after the forms) and swm_rollout_lookahead (the shield judging
+// by `lookahead` backup steps, checked after everything the shield checks but the buffers of a non-empty batch;
+// 0 is the shield).
 int rollout_screened(const swm_params_t* params, const swm_rollout_t* cfg, const swm_params_t* sim_models,
                      int n_models, const double* forms, int n_forms, void* stream, bool shield = false,
-                     const double* backup = nullptr, int32_t* overrides = nullptr) {
+                     const double* backup = nullptr, int32_t* overrides = nullptr, int lookahead = 0) {
   if (!params_ok(params) || !cfg || !cfg->screen.enabled) return SWM_ERR_BAD_ARG;
   swm_rollout_t c = *cfg;
   SimModels sm;
@@ -567,11 +569,13 @@ int rollout_screened(const swm_params_t* params, const swm_rollout_t* cfg, const
   if (rc != SWM_OK) return rc;
   rc = check_thread_screen(&c, f);
   if (rc != SWM_OK) return rc;
+  if (lookahead < 0 || lookahead > SWM_MAX_LOOKAHEAD) return SWM_ERR_BAD_ARG;
   if (c.B == 0) return SWM_OK;  // empty batch: nothing to do, pointers may be NULL
   rc = check_rollout_buffers(&c, f);
   if (rc != SWM_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-#define CALL(K) launch_rollout_screened_n<K>(a, sim_models ? &sm : nullptr, forms ? &cf : nullptr, shield ? &bk : nullptr, f, st)
+#define CALL(K) launch_rollout_screened_n<K>(a, sim_models ? &sm : nullptr, forms ? &cf : nullptr, shield ? &bk : nullptr, \
+                                             lookahead, f, st)
   SWM_DISPATCH_N(params->n, CALL)
 #undef CALL
 }
@@ -595,6 +599,14 @@ extern "C" int swm_rollout_shielded(const swm_params_t* params, const swm_rollou
                                     const double* backup, int32_t* overrides, void* stream) {
   if (!sim_models) return SWM_ERR_BAD_ARG;
   return rollout_screened(params, cfg, sim_models, n_models, forms, n_forms, stream, true, backup, overrides);
+}
+
+extern "C" int swm_rollout_lookahead(const swm_params_t* params, const swm_rollout_t* cfg,
+                                     const swm_params_t* sim_models, int n_models, const double* forms, int n_forms,
+                                     const double* backup, int lookahead, int32_t* overrides, void* stream) {
+  if (!sim_models) return SWM_ERR_BAD_ARG;
+  return rollout_screened(params, cfg, sim_models, n_models, forms, n_forms, stream, true, backup, overrides,
+                          lookahead);
 }
 
 extern "C" int swm_rollout_models(const swm_params_t* models, int n_models, const swm_rollout_t* cfg, void* stream) {

@@ -196,9 +196,10 @@ __device__ __forceinline__ double cost_max_affine(const CostForms& f, const Obs&
 // Screening modes of the rollout kernel: none, the built-in cost max_i |thd_i|, or max-of-affine forms, judged by
 // the simulator model of RolloutArgs::sim or (ENSEMBLE*) by every model of an ensemble.
 // SHIELD*: the ensemble modes with a backup action that is tried when the policy's action is judged unsafe.
+// LOOKAHEAD*: the shield modes judging an action by K further simulator steps of the backup after it.
 enum ScreenMode {
   SCREEN_NONE = 0, SCREEN_BUILTIN = 1, SCREEN_AFFINE = 2, SCREEN_ENSEMBLE = 3, SCREEN_ENSEMBLE_AFFINE = 4,
-  SCREEN_SHIELD = 5, SCREEN_SHIELD_AFFINE = 6
+  SCREEN_SHIELD = 5, SCREEN_SHIELD_AFFINE = 6, SCREEN_LOOKAHEAD = 7, SCREEN_LOOKAHEAD_AFFINE = 8
 };
 
 // The simulator models of ensemble screening (M = 1..SWM_MAX_SIM_MODELS; entries from M on are not read).
@@ -227,6 +228,18 @@ struct SimModelsFormsBackup {
   CostForms forms;
   Backup backup;
 };
+// The lookahead shield: the shield's arguments and the number K >= 1 of backup steps after a judged action.
+struct SimModelsBackupLookahead {
+  SimModels models;
+  Backup backup;
+  int lookahead;
+};
+struct SimModelsFormsBackupLookahead {
+  SimModels models;
+  CostForms forms;
+  Backup backup;
+  int lookahead;
+};
 
 // Type of the rollout kernel's second argument: the cost forms and / or the simulator models of the screening
 // mode, an empty struct without either.  MODELS (model-set mode, unscreened only): the models whose physics the
@@ -238,6 +251,8 @@ template <> struct ScreenForms<SCREEN_ENSEMBLE> { using type = SimModels; };
 template <> struct ScreenForms<SCREEN_ENSEMBLE_AFFINE> { using type = SimModelsForms; };
 template <> struct ScreenForms<SCREEN_SHIELD> { using type = SimModelsBackup; };
 template <> struct ScreenForms<SCREEN_SHIELD_AFFINE> { using type = SimModelsFormsBackup; };
+template <> struct ScreenForms<SCREEN_LOOKAHEAD> { using type = SimModelsBackupLookahead; };
+template <> struct ScreenForms<SCREEN_LOOKAHEAD_AFFINE> { using type = SimModelsFormsBackupLookahead; };
 template <> struct ScreenForms<SCREEN_NONE, true> { using type = SimModels; };
 
 // The physics of a rollout: RolloutArgs::real, or in the model-set mode model blockIdx.y (warp- and CTA-uniform, read
@@ -261,6 +276,11 @@ __device__ __forceinline__ const SimModels& sim_models_of(const SimModelsBackup&
 __device__ __forceinline__ const SimModels& sim_models_of(const SimModelsFormsBackup& s) { return s.models; }
 __device__ __forceinline__ const Backup& backup_of(const SimModelsBackup& s) { return s.backup; }
 __device__ __forceinline__ const Backup& backup_of(const SimModelsFormsBackup& s) { return s.backup; }
+__device__ __forceinline__ const CostForms& cost_forms_of(const SimModelsFormsBackupLookahead& f) { return f.forms; }
+__device__ __forceinline__ const SimModels& sim_models_of(const SimModelsBackupLookahead& s) { return s.models; }
+__device__ __forceinline__ const SimModels& sim_models_of(const SimModelsFormsBackupLookahead& s) { return s.models; }
+__device__ __forceinline__ const Backup& backup_of(const SimModelsBackupLookahead& s) { return s.backup; }
+__device__ __forceinline__ const Backup& backup_of(const SimModelsFormsBackupLookahead& s) { return s.backup; }
 
 // The judgement of the ensemble modes by one simulator model P: one simulator step with the action `act` from the
 // state (gdx, gdy, th, w) with sines s and cosines c, unsafe unless cost <= sim_thresh (a NaN cost is unsafe).
@@ -291,11 +311,91 @@ __device__ __forceinline__ bool model_unsafe(const F& forms, const Phys& P, doub
   return !(sim_cost <= sim_thresh);
 }
 
+// Sines and cosines of the lookahead's simulated states: 1 tracks them by the rotation of gym_step_tracked, with its
+// exact re-evaluation every 64 lookahead steps; 0 evaluates them with sincos at every lookahead step (DESIGN §3.2).
+#ifndef SWM_LOOKAHEAD_TRACKED_TRIG
+#define SWM_LOOKAHEAD_TRACKED_TRIG 1
+#endif
+
+// The backup action b = W_b . x + u0 of the observation x = (gdx, gdy, th, thd), clipped to +-max_u if `clip`.
+template <int N>
+__device__ __forceinline__ void backup_action(const Backup& bk, double gdx, double gdy, const double (&th)[N],
+                                              const double (&thd)[N], bool clip, double max_u,
+                                              double (&b)[N > 1 ? N - 1 : 1]) {
+  constexpr int NA = N - 1, NO = 2 * N + 2;
+#pragma unroll
+  for (int k = 0; k < NA; ++k) b[k] = 0.0;
+#pragma unroll
+  for (int j = 0; j < NO; ++j) {
+    const double x = (j == 0) ? gdx : (j == 1) ? gdy : ((j & 1) ? thd[(j - 3) / 2] : th[(j - 2) / 2]);
+#pragma unroll
+    for (int k = 0; k < NA; ++k) b[k] = fma(x, bk.W[k][j], b[k]);
+  }
+#pragma unroll
+  for (int k = 0; k < NA; ++k) {
+    b[k] += bk.u0[k];
+    if (clip) b[k] = fmin(fmax(b[k], -max_u), max_u);
+  }
+}
+
+// The judgement of the lookahead modes by one simulator model P: x_1 = f(x_0, act) from the state x_0 = (gdx, gdy, th,
+// w) with sines s and cosines c, then x_{j+1} = f(x_j, backup(x_j)) for j = 1..K; unsafe unless cost(x_j) <=
+// sim_thresh for every j = 1..K+1 (a NaN cost is unsafe), and it stops at the first unsafe cost.  Its first step is
+// model_unsafe's judgement, with the same operations; the K backup steps advance a private copy of the state.  The
+// backup is clipped to the real model's max_u, as in the real step.
+template <int N, int FS, bool AFFINE, typename F>
+__device__ __forceinline__ bool model_unsafe_lookahead(const F& forms, const Phys& P, double sim_thresh, int K,
+                                                       bool clip, double max_u, double gdx, double gdy,
+                                                       const double (&th0)[N], const double (&s0)[N],
+                                                       const double (&c0)[N], const double (&w0)[N],
+                                                       const double (&act)[N > 1 ? N - 1 : 1], double* sF) {
+  constexpr int NA = N - 1, NO = 2 * N + 2;
+  double th[N], w[N], s[N], c[N], ut[NA > 0 ? NA : 1];
+#pragma unroll
+  for (int i = 0; i < N; ++i) { th[i] = th0[i]; w[i] = w0[i]; s[i] = s0[i]; c[i] = c0[i]; }
+#pragma unroll
+  for (int k = 0; k < NA; ++k) ut[k] = act[k] * P.u_scale;
+#pragma unroll 1
+  for (int j = 0;; ++j) {
+    if constexpr (SWM_LOOKAHEAD_TRACKED_TRIG) {
+      gym_step_tracked<N, FS>(P, gdx, gdy, th, w, s, c, ut, (j & 63) == 63, sF);
+    } else {
+      if (j > 0) {
+#pragma unroll
+        for (int i = 0; i < N; ++i) sincos(th[i], &s[i], &c[i]);
+      }
+      double psx, psy, thdd[N];
+      gym_accel<N, FS>(P, s, c, gdx, gdy, w, ut, psx, psy, thdd, sF);
+      gdx = fma(P.h_gdd_c, psx, gdx);
+      gdy = fma(P.h_gdd_c, psy, gdy);
+#pragma unroll
+      for (int i = 0; i < N; ++i) {
+        th[i] = fma(P.h, w[i], th[i]);
+        w[i] = fma(P.h, thdd[i], w[i]);
+      }
+    }
+    double cost;
+    if constexpr (AFFINE)
+      cost = cost_max_affine<NO>(cost_forms_of(forms), [&](int k) {
+        return k == 0 ? gdx : k == 1 ? gdy : (k & 1) ? w[(k - 3) / 2] : th[(k - 2) / 2];
+      });
+    else
+      cost = cost_max_abs_thd<N>(w);
+    if (!(cost <= sim_thresh)) return true;
+    if (j == K) return false;
+    double b[NA > 0 ? NA : 1];
+    backup_action<N>(backup_of(forms), gdx, gdy, th, w, clip, max_u, b);
+#pragma unroll
+    for (int k = 0; k < NA; ++k) ut[k] = b[k] * P.u_scale;
+  }
+}
+
 // LINEAR: 0 fixed actions, 1 linear policy.  NORM: ARS V2 normalisation.  STATS: accumulate
 // shifted first/second moments of every visited state.  SCREEN: per-step simulator screening (ScreenMode).
 // With SCREEN_AFFINE the forms travel as the second kernel argument (5.9 KB of the constant bank), with
 // SCREEN_ENSEMBLE the models (2.3 KB), with SCREEN_ENSEMBLE_AFFINE both (8.2 KB), and the SHIELD modes add the
-// backup (1.7 KB, so at most 9.9 KB); the other kernels' argument block grows by one empty byte only.  MODELS: the
+// backup (1.7 KB, so at most 9.9 KB) and the LOOKAHEAD modes its length K; the other kernels' argument block grows by
+// one empty byte only.  MODELS: the
 // model-set mode (SCREEN_NONE, gym dynamics, no statistics, no trajectory), the models (2.3 KB) as the second
 // argument.
 template <int N, int VARIANT, int WMODE, bool NORM, bool STATS, int SCREEN, bool MODELS>
@@ -304,9 +404,11 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
   static_assert(!MODELS || (SCREEN == SCREEN_NONE && VARIANT == 0 && !STATS), "model set: unscreened gym rollouts");
   constexpr int NO = 2 * N + 2, NA = N - 1, WS = NA * NO;
   constexpr bool LINEAR = (WMODE != W_NONE);
-  constexpr bool SHIELD = SCREEN == SCREEN_SHIELD || SCREEN == SCREEN_SHIELD_AFFINE;
+  constexpr bool LOOKAHEAD = SCREEN == SCREEN_LOOKAHEAD || SCREEN == SCREEN_LOOKAHEAD_AFFINE;
+  constexpr bool SHIELD = SCREEN == SCREEN_SHIELD || SCREEN == SCREEN_SHIELD_AFFINE || LOOKAHEAD;
   constexpr bool ENSEMBLE = SCREEN == SCREEN_ENSEMBLE || SCREEN == SCREEN_ENSEMBLE_AFFINE || SHIELD;
-  constexpr bool AFFINE = SCREEN == SCREEN_AFFINE || SCREEN == SCREEN_ENSEMBLE_AFFINE || SCREEN == SCREEN_SHIELD_AFFINE;
+  constexpr bool AFFINE = SCREEN == SCREEN_AFFINE || SCREEN == SCREEN_ENSEMBLE_AFFINE || SCREEN == SCREEN_SHIELD_AFFINE ||
+                          SCREEN == SCREEN_LOOKAHEAD_AFFINE;
   static_assert(!SHIELD || (VARIANT == 0 && LINEAR && !NORM && !STATS), "shield: gym dynamics, linear V1 policies");
   const Phys& P = rollout_model<MODELS>(a, forms);
   extern __shared__ __align__(16) double smem[];
@@ -570,15 +672,27 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
         // products is hoisted and shared with the code after it (which would keep them live across the loop).
         // The single-model modes keep the judgement inline: called through model_unsafe their kernels compile to the
         // same instructions and spills but other registers and another order.
+        // LOOKAHEAD: each model judges by K backup steps after the action (model_unsafe_lookahead), and the first
+        // unsafe model ends the judgement: the decision is an OR, so skipping the other models cannot change it.
         const SimModels& sm = sim_models_of(forms);
 #pragma unroll 1
-        for (int m = 1; m < sm.M; ++m) {
+        for (int m = 1; m < sm.M && !(LOOKAHEAD && unsafe); ++m) {
           double s[N], c[N], w[N];
 #pragma unroll
           for (int i = 0; i < N; ++i) { s[i] = opaque(sn[i]); c[i] = opaque(cs[i]); w[i] = opaque(thd[i]); }
-          unsafe |= model_unsafe<N, FS, AFFINE>(forms, sm.p[m], a.sim_thresh, gdx, gdy, th, s, c, w, u, sF);
+          if constexpr (LOOKAHEAD)
+            unsafe = model_unsafe_lookahead<N, FS, AFFINE>(forms, sm.p[m], a.sim_thresh, forms.lookahead, a.clip,
+                                                           P.max_u, gdx, gdy, th, s, c, w, u, sF);
+          else
+            unsafe |= model_unsafe<N, FS, AFFINE>(forms, sm.p[m], a.sim_thresh, gdx, gdy, th, s, c, w, u, sF);
         }
-        unsafe |= model_unsafe<N, FS, AFFINE>(forms, sm.p[0], a.sim_thresh, gdx, gdy, th, sn, cs, thd, u, sF);
+        if constexpr (LOOKAHEAD) {
+          if (!unsafe)
+            unsafe = model_unsafe_lookahead<N, FS, AFFINE>(forms, sm.p[0], a.sim_thresh, forms.lookahead, a.clip,
+                                                           P.max_u, gdx, gdy, th, sn, cs, thd, u, sF);
+        } else {
+          unsafe |= model_unsafe<N, FS, AFFINE>(forms, sm.p[0], a.sim_thresh, gdx, gdy, th, sn, cs, thd, u, sF);
+        }
         if constexpr (SHIELD) {
           // The shield: a rejected policy action re-runs this step with the backup action (the state has not moved),
           // judged by the same code; the real step takes it if it is safe, and a rejected backup freezes.  The code
@@ -619,7 +733,7 @@ rollout_kernel(const RolloutArgs a, const __grid_constant__ typename ScreenForms
     } else {
       ret += swimmer_step<N, 1>(P, gdx, gdy, th, thd, u);
     }
-    if (SCREEN == SCREEN_BUILTIN || SCREEN == SCREEN_ENSEMBLE || SCREEN == SCREEN_SHIELD)
+    if (SCREEN == SCREEN_BUILTIN || SCREEN == SCREEN_ENSEMBLE || SCREEN == SCREEN_SHIELD || SCREEN == SCREEN_LOOKAHEAD)
       viol += (cost_max_abs_thd<N>(thd) > a.real_thresh) ? 1 : 0;
     if constexpr (AFFINE || STATS) {
       double x[NO];  // the real observation after the step

@@ -1,7 +1,8 @@
 // Host-side template dispatch for one segment count N.  Each rollout_nK.cu translation unit
 // instantiates launch_*_n<K> so the (N x mode) kernel matrix compiles in parallel.  Three rollout
 // families: plain (swm_rollout, with the built-in screen), screened with cost forms and / or an
-// ensemble (swm_rollout_costed / swm_rollout_ensemble / swm_rollout_shielded) and the model set (swm_rollout_models); all
+// ensemble (swm_rollout_costed / swm_rollout_ensemble / swm_rollout_shielded / swm_rollout_lookahead) and the model
+// set (swm_rollout_models); all
 // take the policy storage from with_policy_storage.
 #pragma once
 #include <type_traits>
@@ -23,9 +24,11 @@ template <int N> int launch_step_n(const Phys& P, int variant, bool acc_only, co
 template <int N> int launch_rollout_n(const RolloutArgs& a, const RolloutFlags& f, cudaStream_t st);
 // per-step screening with cost forms and / or an ensemble of simulator models: SCREEN_AFFINE without models (forms
 // required), else SCREEN_ENSEMBLE (no forms: the built-in cost) or SCREEN_ENSEMBLE_AFFINE; with a backup (models
-// required) SCREEN_SHIELD or SCREEN_SHIELD_AFFINE
+// required) SCREEN_SHIELD or SCREEN_SHIELD_AFFINE, and with a backup and lookahead > 0 SCREEN_LOOKAHEAD or
+// SCREEN_LOOKAHEAD_AFFINE
 template <int N> int launch_rollout_screened_n(const RolloutArgs& a, const SimModels* models, const CostForms* forms,
-                                               const Backup* backup, const RolloutFlags& f, cudaStream_t st);
+                                               const Backup* backup, int lookahead, const RolloutFlags& f,
+                                               cudaStream_t st);
 // model-set mode: cfg->B environments for each of models.M models, one CTA row per model (f as for launch_rollout_n)
 template <int N> int launch_rollout_models_n(const RolloutArgs& a, const SimModels& models, const RolloutFlags& f,
                                              cudaStream_t st);
@@ -84,11 +87,28 @@ static int launch_rollout_one(const RolloutArgs& a, cudaStream_t st) {
 // gym dynamics, linear policies, ARS V1 without statistics.
 template <int N>
 int launch_rollout_screened_n(const RolloutArgs& a, const SimModels* models, const CostForms* forms,
-                              const Backup* backup, const RolloutFlags& f, cudaStream_t st) {
+                              const Backup* backup, int lookahead, const RolloutFlags& f, cudaStream_t st) {
   if (f.variant != SWM_DYN_GYM || !f.linear || !f.screen || f.norm || f.stats) return SWM_ERR_UNSUPPORTED;
   return with_policy_storage<N>(f.group_w, [&](auto w) {
     constexpr int WMODE = decltype(w)::value;
     const size_t smem = rollout_smem<N, 0, WMODE, false>();
+    if (backup && lookahead > 0 && !forms) {
+      SimModelsBackupLookahead mbl;
+      mbl.models = *models;
+      mbl.backup = *backup;
+      mbl.lookahead = lookahead;
+      return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_LOOKAHEAD, false>, smem, a.B, 1, st,
+                                 a, mbl);
+    }
+    if (backup && lookahead > 0) {
+      SimModelsFormsBackupLookahead mfbl;
+      mfbl.models = *models;
+      mfbl.forms = *forms;
+      mfbl.backup = *backup;
+      mfbl.lookahead = lookahead;
+      return launch_rollout_grid(rollout_kernel<N, 0, WMODE, false, false, SCREEN_LOOKAHEAD_AFFINE, false>, smem, a.B,
+                                 1, st, a, mfbl);
+    }
     if (backup && !forms) {
       SimModelsBackup mb;
       mb.models = *models;
@@ -188,7 +208,7 @@ template int launch_step_n<SWM_INSTANTIATE_N>(const Phys&, int, bool, const doub
                                               double*, double*, long long, cudaStream_t);
 template int launch_rollout_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const RolloutFlags&, cudaStream_t);
 template int launch_rollout_screened_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const SimModels*, const CostForms*,
-                                                          const Backup*, const RolloutFlags&, cudaStream_t);
+                                                          const Backup*, int, const RolloutFlags&, cudaStream_t);
 template int launch_rollout_models_n<SWM_INSTANTIATE_N>(const RolloutArgs&, const SimModels&, const RolloutFlags&,
                                                         cudaStream_t);
 

@@ -7,6 +7,7 @@ swimmer_env.py / environment.py / ars_agent.py / safe_ars.py are thin layers ove
 """
 import ctypes
 import math
+import numbers
 
 import numpy as np
 import torch
@@ -15,7 +16,7 @@ from . import _lib
 from ._lib import (ARS_AGENT, ARS_RLGLUE, ARS_TOPB, DELTA_01, DELTA_PM1, GYM, POLICY_DELTAS,
                    POLICY_EXPLICIT, POLICY_FIXED_ACTION, POLICY_PHILOX, RLGLUE)
 
-__all__ = ["step_batched", "step_batched_models", "accelerations_batched", "rollout", "rollout_models", "backup_array", "RolloutResult", "ChunkedRollout", "plan_chunks", "philox_deltas",
+__all__ = ["step_batched", "step_batched_models", "accelerations_batched", "rollout", "rollout_models", "backup_array", "check_lookahead", "RolloutResult", "ChunkedRollout", "plan_chunks", "philox_deltas",
            "ars_topb", "ars_update", "pack_exchange", "counter_add", "record_nanmean", "stats_finalize", "stats_merge", "reduce_returns", "screen_mask", "policy_actions", "update_args",
            "EstimateData", "prediction_error", "cmaes_default_popsize", "cmaes_state_doubles", "cmaes_view", "cmaes_init",
            "cmaes_sample", "cmaes_update", "cmaes_generation",
@@ -158,6 +159,9 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
     action the model(s) reject is taken with the backup action W_b obs + u_0 instead if the same model(s) judge that
     safe, and freezes only otherwise (swm_rollout_shielded; a single simulator is the ensemble of one).  The result
     then has `overrides` [B] int32, the number of steps each environment took with the backup.
+    screen["lookahead"] = K (an int in 0..MAX_LOOKAHEAD; K > 0 needs the backup) makes the shield judge every action by
+    K more simulator steps: an action is safe only if, after it, the backup keeps every model's cost within sim_thresh
+    for K more steps (swm_rollout_lookahead; up to M (K+1) simulator steps per judgement).  K = 0 is the shield above.
     stats_pivot[2n+2] enables the V2 moment accumulation.  `out` may carry preallocated
     tensors (returns, final_state, trajectory, stats_partial) to stay allocation-free in loops.
     kernel: _lib.KERNEL_AUTO (chosen from B, n and the SM count) / KERNEL_THREAD (one thread per
@@ -166,6 +170,8 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
     swm_rollout_t.schedule_sub); "plain" = always one launch; (n_sub, chunk) = forced.
     _models: see rollout_models.
     """
+    lookahead = check_lookahead(screen.get("lookahead", 0) if screen is not None else 0,
+                                screen is not None and screen.get("backup") is not None)
     _lib.require_cuda()
     n = params.n
     no, na, ws = obs_dim(n), act_dim(n), policy_size(n)
@@ -288,6 +294,12 @@ def rollout(params, H, *, B=None, variant=GYM, actions=None, policies=None, base
     with torch.cuda.device(dev):
         if _models is not None:
             _lib.check(_lib.lib().swm_rollout_models(models, len(model_list), ctypes.byref(cfg), _lib.stream_ptr()))
+        elif backup is not None and lookahead > 0:
+            _lib.check(_lib.lib().swm_rollout_lookahead(
+                ctypes.byref(params), ctypes.byref(cfg), models, len(model_list),
+                None if forms is None else forms.ctypes.data_as(ctypes.c_void_p),
+                0 if forms is None else forms.shape[0], backup.ctypes.data_as(ctypes.c_void_p), lookahead,
+                res.overrides.data_ptr(), _lib.stream_ptr()))
         elif backup is not None:
             _lib.check(_lib.lib().swm_rollout_shielded(
                 ctypes.byref(params), ctypes.byref(cfg), models, len(model_list),
@@ -324,6 +336,19 @@ def backup_array(n, policy=None, action=None):
     W = host(policy, (act_dim(n), obs_dim(n)), "policy")
     u0 = host(action, (act_dim(n),), "action")
     return np.ascontiguousarray(np.concatenate([W.reshape(-1), u0]))
+
+
+def check_lookahead(lookahead, has_backup):
+    """The lookahead K of a shield as swm_rollout_lookahead takes it: an int in 0..MAX_LOOKAHEAD, and K > 0 only with
+    a backup.  Raises ValueError otherwise."""
+    if isinstance(lookahead, bool) or not isinstance(lookahead, numbers.Integral):
+        raise ValueError("the lookahead must be an integer, got %r" % (lookahead,))
+    lookahead = int(lookahead)
+    if not 0 <= lookahead <= _lib.MAX_LOOKAHEAD:
+        raise ValueError("the lookahead must be in 0..%d, got %d" % (_lib.MAX_LOOKAHEAD, lookahead))
+    if lookahead > 0 and not has_backup:
+        raise ValueError("a lookahead needs a backup (a zero-torque backup is backup=dict(policy=None, action=None))")
+    return lookahead
 
 
 def rollout_models(params_list, H, **kw):

@@ -140,9 +140,15 @@ class Safe_ARS(Basic_ARS):
     `backup_policy` W_b [n-1, 2n+2] and / or `backup_action` u_0 [n-1] (declared extension; default: none) add a
     shield: a step whose action the simulator(s) reject is taken with the backup action W_b obs + u_0 if the same
     simulator(s) judge that safe (zero torque, a damping controller, a known hand controller), and the rollout freezes
-    only if the backup is unsafe too.  Without them the agent behaves as the reference."""
+    only if the backup is unsafe too.  Without them the agent behaves as the reference.
 
-    def __init__(self, cost, real_threshold, sim_threshold, sim_env, backup_policy=None, backup_action=None):
+    `lookahead` K > 0 (declared extension; needs a backup) makes that shield look ahead: an action, the policy's or
+    the backup's, is safe only if after it the backup keeps every simulator's cost within sim_threshold for K more
+    steps.  That is what lets the shield act on costs of the angles, such as bending limits, which no action changes
+    within one explicit-Euler step.  K = 0 is the one-step shield."""
+
+    def __init__(self, cost, real_threshold, sim_threshold, sim_env, backup_policy=None, backup_action=None,
+                 lookahead=0):
         if isinstance(sim_env, SwimmerEnv):
             n = sim_env.n
         else:
@@ -169,6 +175,7 @@ class Safe_ARS(Basic_ARS):
             b = ops.backup_array(n, backup_policy, backup_action)  # ValueError for a wrong shape or non-finite value
             ws = (n - 1) * (2 * n + 2)
             self.backup = dict(policy=b[:ws].reshape(n - 1, 2 * n + 2), action=b[ws:])
+        self.lookahead = ops.check_lookahead(lookahead, self.backup is not None)  # ValueError without a backup
 
     def _screen(self, real_env):
         if isinstance(self.sim_env, SwimmerEnv):
@@ -184,6 +191,8 @@ class Safe_ARS(Basic_ARS):
             screen["cost"] = self.cost
         if self.backup is not None:
             screen["backup"] = self.backup
+        if self.lookahead > 0:
+            screen["lookahead"] = self.lookahead
         return screen
 
     def isSafe(self, cost, thresh, env, state, action):
@@ -196,13 +205,35 @@ class Safe_ARS(Basic_ARS):
         obs, _, _, _ = env.step(action)
         return cost(obs) <= thresh
 
+    def isRecoverable(self, cost, thresh, env, state, action):
+        """isSafe with the lookahead K: simulate `action` from `state`, then K steps of the backup action, and True only
+        if every one of the K+1 costs is within the threshold (for a sequence of environments: in every one of them).
+        With K = 0 this is isSafe."""
+        if self.lookahead == 0:
+            return self.isSafe(cost, thresh, env, state, action)
+        if not isinstance(env, SwimmerEnv):
+            return all([self.isRecoverable(cost, thresh, e, state, action) for e in env])
+        env.set_state(state)
+        obs, _, _, _ = env.step(action)
+        if not cost(obs) <= thresh:
+            return False
+        for _ in range(self.lookahead):
+            obs, _, _, _ = env.step(self._backup_action(obs))
+            if not cost(obs) <= thresh:
+                return False
+        return True
+
+    def _backup_action(self, obs):
+        return self.backup["policy"] @ np.asarray(obs, dtype=np.float64) + self.backup["action"]
+
     def shielded_action(self, cost, thresh, env, state, action):
         """The action the shielded rollout takes from `state` (host counterpart of the kernel's decision): `action` if
-        isSafe judges it safe, else the backup action W_b state + u_0 if isSafe judges that safe, else None (the
-        rollout freezes).  Without a backup an unsafe action gives None.  Leaves env in its last simulated state."""
-        if self.isSafe(cost, thresh, env, state, action):
+        isRecoverable judges it safe, else the backup action W_b state + u_0 if isRecoverable judges that safe, else
+        None (the rollout freezes).  Without a backup an unsafe action gives None.  Leaves env in its last simulated
+        state."""
+        if self.isRecoverable(cost, thresh, env, state, action):
             return action
         if self.backup is None:
             return None
-        b = self.backup["policy"] @ np.asarray(state, dtype=np.float64) + self.backup["action"]
-        return b if self.isSafe(cost, thresh, env, state, b) else None
+        b = self._backup_action(state)
+        return b if self.isRecoverable(cost, thresh, env, state, b) else None
